@@ -73,6 +73,14 @@ _SIGNATURES = {
     "emia_group_filter_flag": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
     "emia_rle_count": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     "emia_rle_encode": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p]),
+    "emia_rle_line_count": (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),
+    "emia_rle_line_index": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
+    "emia_rle_parse_count": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
+    "emia_rle_parse_fill": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                    c_void_p]),
+    "emia_rle_decode_plan": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
+                                     c_void_p, c_void_p]),
+    "emia_rle_decode": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "emia_moments01": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "emia_moments": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "emia_color_sums": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int, c_int, c_void_p, c_void_p]),

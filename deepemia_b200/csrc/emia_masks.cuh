@@ -26,19 +26,10 @@ __global__ void __launch_bounds__(256) k_mask_bbox(const uint8_t* __restrict__ m
         }
         __syncthreads();
         if (threadIdx.x == 0) {
-            emia_inst_meta mt;
             const int ar = s_red[0];
             area[inst] = ar;
-            if (ar > 0) {
-                ((int4*)bbox)[inst] = make_int4(s_red[1], s_red[2], s_red[3], s_red[4]);
-                mt.ry0 = s_red[1]; mt.ch = s_red[3] - s_red[1] + 1;
-                mt.rx0 = s_red[2]; mt.rx1 = s_red[4] + 1;
-                mt.wc0 = mt.rx0 >> 5; mt.cw = ((mt.rx1 - 1) >> 5) - mt.wc0 + 1;
-            } else {
-                ((int4*)bbox)[inst] = make_int4(-1, -1, -1, -1);
-                mt.ry0 = mt.ch = mt.rx0 = mt.rx1 = mt.wc0 = mt.cw = 0;
-            }
-            mt.valid = 1; mt.reserved = 0;
+            ((int4*)bbox)[inst] = ar > 0 ? make_int4(s_red[1], s_red[2], s_red[3], s_red[4]) : make_int4(-1, -1, -1, -1);
+            const emia_inst_meta mt = emia_meta_from_bbox(ar, s_red[1], s_red[2], s_red[3], s_red[4]);
             meta[inst] = mt;
             crop_words[inst] = (int64_t)mt.ch * mt.cw;
         }

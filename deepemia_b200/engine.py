@@ -1141,6 +1141,121 @@ def rle_encode(iset, idx=None):
     return run_off, runs[:R]
 
 
+RLE_TEXT_CHUNK = 8192        # EMIA_RLE_TEXT_CHUNK
+RLE_HEADER = b"ImageId,EncodedPixels"
+RLE_STATUS = {1: "no comma separates ImageId from EncodedPixels", 2: "EncodedPixels holds a character other than a digit or a blank",
+              3: "odd number of values", 4: "a value of more than 18 digits", 5: "a run with start < 1 or length < 1",
+              6: "a run past pixel H * W", 7: "a run that starts at or before the end of the previous run (unsorted or overlapping)",
+              8: "more than 2^31 - 1 pixels"}
+
+
+def _csv_field(raw):
+    """An ImageId as csv.writer wrote it: a quoted field loses its quotes and doubled inner quotes."""
+    s = raw.decode("utf-8")
+    if len(s) >= 2 and s[0] == '"' and s[-1] == '"':
+        s = s[1:-1].replace('""', '"')
+    return s
+
+
+def _rle_parse(data, device=None):
+    """rle_parse_csv plus the 1-based file line number of every data line (numpy int64)."""
+    lib = _lib.load()
+    dev = _need_cuda(device)
+    data = bytes(data)
+    first = data.split(b"\n", 1)[0].rstrip(b"\r ")
+    if first != RLE_HEADER:
+        raise _lib.EmiaError(f"rle_parse_csv: line 1: header {first[:64]!r} is not {RLE_HEADER!r}")
+    nbytes = len(data)
+    host = torch.empty(nbytes, dtype=torch.uint8, pin_memory=True)
+    host.numpy()[:] = np.frombuffer(data, np.uint8)
+    st = _stream()
+    with _stage("rle_h2d"):
+        text = host.to(dev, non_blocking=True)
+    with _stage("rle_parse"):
+        chunks = (nbytes + RLE_TEXT_CHUNK - 1) // RLE_TEXT_CHUNK
+        chunk_off = torch.zeros(chunks + 1, dtype=torch.int64, device=dev)
+        _lib.check(lib.emia_rle_line_count(_ptr(text), nbytes, _ptr(chunk_off), st), "emia_rle_line_count")
+        exclusive_scan_(chunk_off)
+        L = int(chunk_off[chunks].item()) + (data[-1:] != b"\n")          # lines, the header included
+        line_off = torch.empty(L + 2, dtype=torch.int64, device=dev)
+        _lib.check(lib.emia_rle_line_index(_ptr(text), nbytes, _ptr(chunk_off), _ptr(line_off), st), "emia_rle_line_index")
+        n = L - 1                                                          # lines after the header
+        cnt = torch.zeros((2, n + 1), dtype=torch.int64, device=dev)      # rows: data lines, runs
+        _lib.check(lib.emia_rle_parse_count(_ptr(text), _ptr(line_off[1:]), n, _ptr(cnt[0]), _ptr(cnt[1]), st), "emia_rle_parse_count")
+        exclusive_scan_(cnt[0])
+        exclusive_scan_(cnt[1])
+        D, R = (int(v) for v in cnt[:, n].tolist())
+        run_off = torch.zeros(D + 1, dtype=torch.int64, device=dev)
+        runs = torch.empty((max(R, 1), 2), dtype=torch.int64, device=dev)
+        field = torch.empty((max(D, 1), 2), dtype=torch.int64, device=dev)
+        line_idx = torch.empty(max(D, 1), dtype=torch.int32, device=dev)
+        status = torch.empty(max(D, 1), dtype=torch.int32, device=dev)
+        _lib.check(lib.emia_rle_parse_fill(_ptr(text), _ptr(line_off[1:]), n, _ptr(cnt[0]), _ptr(cnt[1]), _ptr(run_off), _ptr(runs),
+                                           _ptr(field), _ptr(line_idx), _ptr(status), st), "emia_rle_parse_fill")
+    LAUNCHES["count"] += 4
+    status = status[:D].cpu().numpy()
+    line_no = line_idx[:D].cpu().numpy().astype(np.int64) + 2
+    bad = np.nonzero(status)[0]
+    if len(bad):
+        k = int(bad[0])
+        raise _lib.EmiaError(f"rle_parse_csv: line {line_no[k]}: {RLE_STATUS[int(status[k])]}")
+    fld = field[:D].cpu().numpy()
+    ids = [_csv_field(data[a:b]) for a, b in fld.tolist()]
+    return ids, run_off, runs[:R], line_no
+
+
+def rle_parse_csv(data, device=None):
+    """The text of an R50_flip_results.csv file (bytes) -> (image_ids: list[str], run_off int64 [L+1], runs int64 [R, 2]) with the
+    runs of data line k at runs[run_off[k]:run_off[k+1]] (device tensors), one H2D copy of the text and the parse in CUDA.
+    Line 1 must be the header `ImageId,EncodedPixels`; empty lines are skipped; the last comma of a line separates the ImageId
+    (quoted by csv.writer when it holds a comma) from EncodedPixels; an empty EncodedPixels field is an empty mask.
+    Raises EmiaError naming the first malformed line (1-based line number of the file)."""
+    ids, run_off, runs, _ = _rle_parse(data, device)
+    return ids, run_off, runs
+
+
+def _rle_decode(run_off, runs, H, W, rows=None):
+    """(InstanceSet, per-instance status as numpy int32) of the lines `rows` (default: all) of (run_off, runs)."""
+    lib = _lib.load()
+    if not (1 <= H <= 65535 and 1 <= W <= 65535):
+        raise _lib.EmiaError(f"rle_decode: frame {H} x {W} outside 1..65535 (the contour vertex packing limit)")
+    dev = run_off.device
+    assert run_off.dtype == torch.int64 and runs.dtype == torch.int64 and run_off.is_contiguous() and runs.is_contiguous()
+    rows_t = None if rows is None else torch.as_tensor(np.asarray(rows, np.int32), device=dev)
+    n = int(run_off.numel()) - 1 if rows is None else int(rows_t.numel())
+    meta = torch.empty((n, 8), dtype=torch.int32, device=dev)
+    crop_off = torch.empty(n + 1, dtype=torch.int64, device=dev)
+    bbox = torch.empty((n, 4), dtype=torch.int32, device=dev)
+    area = torch.empty(n, dtype=torch.int32, device=dev)
+    status = torch.empty(max(n, 1), dtype=torch.int32, device=dev)
+    st = _stream()
+    rp = _ptr(runs) if runs.numel() else _ptr(run_off)      # no runs at all: never read, but the ABI wants a pointer
+    with _stage("rle_decode"):
+        _lib.check(lib.emia_rle_decode_plan(rp, _ptr(run_off), _ptr(rows_t), n, H, W, _ptr(meta), _ptr(crop_off), _ptr(bbox), _ptr(area),
+                                            _ptr(status), st), "emia_rle_decode_plan")
+        exclusive_scan_(crop_off)
+        total = int(crop_off[n].item()) if n else 0
+        crops = torch.empty(max(total, 1), dtype=torch.int32, device=dev)
+        _lib.check(lib.emia_rle_decode(rp, _ptr(run_off), _ptr(rows_t), n, H, _ptr(meta), _ptr(crop_off), _ptr(crops), st),
+                   "emia_rle_decode")
+    LAUNCHES["count"] += 2
+    iset = InstanceSet(n=n, H=H, W=W, meta=meta, crop_off=crop_off, crops=crops, bbox=bbox, area=area, total_crop_words=total)
+    return iset, status[:n].cpu().numpy()
+
+
+def rle_decode(run_off, runs, H, W):
+    """Inverse of rle_encode: (run_off int64 [n+1], runs int64 [R, 2]) of an H x W frame -> InstanceSet, bit for bit the tables
+    from_masks gives for the same masks (tight bbox crops), so rle_decode(*rle_encode(s), H, W) round-trips.  Runs are column-major
+    and 1-indexed; one may continue from row H-1 of a column into the next columns.  Raises EmiaError naming the first instance
+    with a bad run (start or length < 1, past H * W, unsorted or overlapping) or more than 2^31 - 1 pixels."""
+    iset, status = _rle_decode(run_off, runs, H, W)
+    bad = np.nonzero(status)[0]
+    if len(bad):
+        k = int(bad[0])
+        raise _lib.EmiaError(f"rle_decode: instance {k}: {RLE_STATUS[int(status[k])]}")
+    return iset
+
+
 def gray_hist(iset, image):
     """int32 [n,256] grey-level histograms of the image pixels under every instance (image: H x W x 3 BGR or H x W uint8)."""
     lib = _lib.load()

@@ -616,52 +616,30 @@ def clear_providers():
         _PROVIDERS[k] = None
 
 
-def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw_id=False, dataset_format="json", draw_scalebar=False,
-                  *, images=None, predictors=None, thing_classes=None, small_classes=None, scale_bar_fn=None, **infer_kwargs):
-    """run_inference (src/functions/inference.py:499-1351), same signature and call shape as main.py:480-488:
+def _resolve_images(dataset_name, images):
+    """The (file name, image) pairs of a run: the given ones, else the images provider's, else None."""
+    return images if images is not None else (_PROVIDERS["images"](dataset_name) if _PROVIDERS["images"] else None)
 
-        run_inference(dataset_name, output_dir, visualize=..., threshold=..., draw_id=..., dataset_format=..., draw_scalebar=...)
 
-    with the reference's own subsystems behind registered providers (set_providers) or the keyword-only overrides.  Settings are
-    read from the dataset config exactly as :517-556 does (confidence mode, class-specific settings, tile / ensemble settings,
-    classes_to_infer); small classes come from the mask-size heuristic (:719-723) unless given.  Per image: scale bar ->
-    per-class tile pipeline -> cross-class de-dup -> spatial constraints (:776-905), all on the device; the RLE rows of
-    R50_flip_results.csv and the rows of measurements_results.csv are produced from the SAME device-resident instance set (one
-    K6 and one K5 pass per image, no mask round trip).  Writes R50_flip_results.csv, measurements_results.csv,
-    class_color_legend.txt and, with visualize, <name>_predictions.png (overlay kernel + labels)."""
+def _dataset_config(dataset_name):
     cfg_fn = _PROVIDERS["config"]
-    images = images if images is not None else (_PROVIDERS["images"](dataset_name) if _PROVIDERS["images"] else None)
-    if thing_classes is None and _PROVIDERS["thing_classes"]:
-        thing_classes = _PROVIDERS["thing_classes"](dataset_name)
-    thing_classes = list(thing_classes or [])
-    if predictors is None and _PROVIDERS["predictors"]:
-        predictors = _PROVIDERS["predictors"](dataset_name, threshold, thing_classes)
-    if images is None or not predictors:
-        raise FileNotFoundError(f"No trained models / images registered for dataset '{dataset_name}': call "
-                                "deepemia_b200.functions.inference.set_providers(...) (or pass images= and predictors=)")
-    images = list(images)
-    dataset_config = cfg_fn(dataset_name) if cfg_fn else {}
-    inf_settings = dataset_config.get("inference_overrides", {}) or dataset_config.get("inference_settings", {})
-    tile_cfg = inf_settings.get("tile_settings", {})
-    ens_cfg = inf_settings.get("ensemble_settings", {})
-    kw = dict(class_specific_settings=inf_settings.get("class_specific_settings", {}),
-              confidence_mode=inf_settings.get("confidence_mode", "auto"),
-              tile_size=tile_cfg.get("tile_size", 512), overlap_ratio=tile_cfg.get("overlap_ratio", 0.1),
-              upscale_factor=tile_cfg.get("upscale_factor", 2.0), edge_filter_enabled=tile_cfg.get("edge_filter_enabled", True),
-              ensemble_enabled=ens_cfg.get("enabled", True), ensemble_small_only=ens_cfg.get("small_classes_only", True),
-              classes_to_infer=inf_settings.get("inference_settings", {}).get("classes_to_infer", None))
-    kw.update(infer_kwargs)
-    num_classes = len(thing_classes) if thing_classes else int(kw.pop("num_classes", 1))
-    kw.pop("num_classes", None)
-    if small_classes is None:
-        from ..adapters import calculate_average_mask_sizes, determine_small_classes
-        small_classes = determine_small_classes(calculate_average_mask_sizes(predictors, [im for _, im in images[:5]]), 50)
-    small_classes = set(small_classes)
+    return cfg_fn(dataset_name) if cfg_fn else {}
+
+
+def _stem(name):
+    """The ImageId of an image's rows in R50_flip_results.csv: its file name without the extension."""
+    return name.rsplit(".", 1)[0]
+
+
+def _scale_bars(images, dataset_name, dataset_config, output_dir, scale_bar_fn=None, draw_scalebar=False):
+    """(psum, um_pix) of every image, in order, as run_inference resolves them (inference.py:744-773): scale_bar_fn, else the
+    scale_bar provider, else the package's own detector (batched over all images when there is more than one), else ("0", 1.0).
+    An iterator: an image's own detection (and, with draw_scalebar, its debug overlay) happens when its value is taken."""
+    cfg_fn = _PROVIDERS["config"]
     rois = dataset_config.get("scale_bar_rois", {})
     roi_config = rois.get(dataset_name, rois.get("default", {"x_start_factor": 0.667, "y_start_factor": 0.866, "width_factor": 1.0,
                                                             "height_factor": 0.067}))
     user_fn = scale_bar_fn or ((lambda im: _PROVIDERS["scale_bar"](im, roi_config, dataset_name)) if _PROVIDERS["scale_bar"] else None)
-    os.makedirs(output_dir, exist_ok=True)
     from ..utils import scalebar_ocr as _sb
     if cfg_fn and _sb._state["config"] is None:
         _sb.set_config_provider(cfg_fn)
@@ -678,7 +656,6 @@ def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw
         if draw_scalebar:
             cv2.imwrite(os.path.join(output_dir, f"{name}_scalebar_debug.png"), work)
         return r
-    img_ids, encoded, meas_rows = [], [], []
     # the scale bars of ALL images in one launch per stage (and frame size) when the package's own detector is in use; a failure
     # of the batch falls back to the reference's per-image call with its per-image try / except (inference.py:750-773)
     batch_bars = None
@@ -687,17 +664,74 @@ def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw
             batch_bars = _sb.detect_scale_bars([im for _, im in images], roi_config=roi_config, dataset_name=dataset_name)
         except Exception:
             batch_bars = None
-    for k, (name, image) in enumerate(images):
-        try:
-            psum, um_pix = batch_bars[k] if batch_bars is not None else scale_bar(image, name)
-        except Exception:
-            psum, um_pix = "0", 1.0                                     # inference.py:767-773
+
+    def each():
+        for k, (name, image) in enumerate(images):
+            try:
+                bar = batch_bars[k] if batch_bars is not None else scale_bar(image, name)
+            except Exception:
+                bar = "0", 1.0                                          # inference.py:767-773
+            yield bar
+    return each()
+
+
+def _write_measurements(output_dir, rows):
+    with open(os.path.join(output_dir, "measurements_results.csv"), "w", newline="") as f:
+        w = csv.writer(f)
+        w.writerow(CSV_HEADER)
+        w.writerows(rows)
+
+
+def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw_id=False, dataset_format="json", draw_scalebar=False,
+                  *, images=None, predictors=None, thing_classes=None, small_classes=None, scale_bar_fn=None, **infer_kwargs):
+    """run_inference (src/functions/inference.py:499-1351), same signature and call shape as main.py:480-488:
+
+        run_inference(dataset_name, output_dir, visualize=..., threshold=..., draw_id=..., dataset_format=..., draw_scalebar=...)
+
+    with the reference's own subsystems behind registered providers (set_providers) or the keyword-only overrides.  Settings are
+    read from the dataset config exactly as :517-556 does (confidence mode, class-specific settings, tile / ensemble settings,
+    classes_to_infer); small classes come from the mask-size heuristic (:719-723) unless given.  Per image: scale bar ->
+    per-class tile pipeline -> cross-class de-dup -> spatial constraints (:776-905), all on the device; the RLE rows of
+    R50_flip_results.csv and the rows of measurements_results.csv are produced from the SAME device-resident instance set (one
+    K6 and one K5 pass per image, no mask round trip).  Writes R50_flip_results.csv, measurements_results.csv,
+    class_color_legend.txt and, with visualize, <name>_predictions.png (overlay kernel + labels)."""
+    images = _resolve_images(dataset_name, images)
+    if thing_classes is None and _PROVIDERS["thing_classes"]:
+        thing_classes = _PROVIDERS["thing_classes"](dataset_name)
+    thing_classes = list(thing_classes or [])
+    if predictors is None and _PROVIDERS["predictors"]:
+        predictors = _PROVIDERS["predictors"](dataset_name, threshold, thing_classes)
+    if images is None or not predictors:
+        raise FileNotFoundError(f"No trained models / images registered for dataset '{dataset_name}': call "
+                                "deepemia_b200.functions.inference.set_providers(...) (or pass images= and predictors=)")
+    images = list(images)
+    dataset_config = _dataset_config(dataset_name)
+    inf_settings = dataset_config.get("inference_overrides", {}) or dataset_config.get("inference_settings", {})
+    tile_cfg = inf_settings.get("tile_settings", {})
+    ens_cfg = inf_settings.get("ensemble_settings", {})
+    kw = dict(class_specific_settings=inf_settings.get("class_specific_settings", {}),
+              confidence_mode=inf_settings.get("confidence_mode", "auto"),
+              tile_size=tile_cfg.get("tile_size", 512), overlap_ratio=tile_cfg.get("overlap_ratio", 0.1),
+              upscale_factor=tile_cfg.get("upscale_factor", 2.0), edge_filter_enabled=tile_cfg.get("edge_filter_enabled", True),
+              ensemble_enabled=ens_cfg.get("enabled", True), ensemble_small_only=ens_cfg.get("small_classes_only", True),
+              classes_to_infer=inf_settings.get("inference_settings", {}).get("classes_to_infer", None))
+    kw.update(infer_kwargs)
+    num_classes = len(thing_classes) if thing_classes else int(kw.pop("num_classes", 1))
+    kw.pop("num_classes", None)
+    if small_classes is None:
+        from ..adapters import calculate_average_mask_sizes, determine_small_classes
+        small_classes = determine_small_classes(calculate_average_mask_sizes(predictors, [im for _, im in images[:5]]), 50)
+    small_classes = set(small_classes)
+    os.makedirs(output_dir, exist_ok=True)
+    bars = _scale_bars(images, dataset_name, dataset_config, output_dir, scale_bar_fn, draw_scalebar)
+    img_ids, encoded, meas_rows = [], [], []
+    for (name, image), (psum, um_pix) in zip(images, bars):
         d = _infer_image_dev(predictors, image, num_classes, small_classes, dataset_name=dataset_name, **kw)
         if len(d) == 0:
             continue
         run_off, runs = engine.rle_encode(d.iset)                       # K6 over the final set, once
         ro, rn = run_off.cpu().numpy(), runs.cpu().numpy()
-        stem = name.rsplit(".", 1)[0]
+        stem = _stem(name)
         for i in range(len(d)):
             img_ids.append(stem)
             encoded.append(" ".join(str(int(v)) for v in rn[ro[i]:ro[i + 1]].reshape(-1)))
@@ -709,9 +743,87 @@ def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw
         w = csv.writer(f)
         w.writerow(["ImageId", "EncodedPixels"])
         w.writerows(zip(img_ids, encoded))
-    with open(os.path.join(output_dir, "measurements_results.csv"), "w", newline="") as f:
-        w = csv.writer(f)
-        w.writerow(CSV_HEADER)
-        w.writerows(meas_rows)
+    _write_measurements(output_dir, meas_rows)
     write_class_color_legend(output_dir, thing_classes)
     return None
+
+
+# =================================================================================================================
+# reading saved results back: R50_flip_results.csv -> instances (RLE decode on the device) -> a new measurements_results.csv
+# =================================================================================================================
+def load_rle_results(path, images):
+    """R50_flip_results.csv -> {file name: engine.InstanceSet} for the (file name, image) pairs `images` that run_inference takes.
+    Rows match an image by stem, as run_inference writes them; instance k of an image is the k-th row with its ImageId, in file
+    order; an image without rows maps to an empty set.  The file is parsed once and decoded once per distinct frame size, on the
+    device.  Raises ValueError when two names share a stem, EmiaError naming the line of a malformed row or of an ImageId that
+    matches no image."""
+    images = list(images)
+    by_stem = {}
+    for k, (name, _) in enumerate(images):
+        stem = _stem(name)
+        if stem in by_stem:
+            raise ValueError(f"load_rle_results: {images[by_stem[stem]][0]!r} and {name!r} share the ImageId {stem!r}")
+        by_stem[stem] = k
+    with open(path, "rb") as f:
+        data = f.read()
+    try:
+        ids, run_off, runs, line_no = engine._rle_parse(data)
+    except engine._lib.EmiaError as e:
+        raise engine._lib.EmiaError(f"{path}: {e}") from None
+    rows_of = [[] for _ in images]
+    for r, stem in enumerate(ids):
+        k = by_stem.get(stem)
+        if k is None:
+            raise engine._lib.EmiaError(f"{path}: line {line_no[r]}: ImageId {stem!r} matches no image")
+        rows_of[k].append(r)
+    by_size = {}
+    for k, (_, image) in enumerate(images):
+        by_size.setdefault(tuple(int(s) for s in image.shape[:2]), []).append(k)
+    out, bad = {}, []
+    for (H, W), ks in by_size.items():
+        rows = [r for k in ks for r in rows_of[k]]
+        iset, status = engine._rle_decode(run_off, runs, H, W, rows)
+        bad += [(int(line_no[rows[j]]), int(status[j])) for j in np.nonzero(status)[0][:1]]
+        a = 0
+        for k in ks:
+            m = len(rows_of[k])
+            out[images[k][0]] = iset if len(ks) == 1 else engine.select(iset, list(range(a, a + m)))
+            a += m
+    if bad:
+        line, code = min(bad)
+        raise engine._lib.EmiaError(f"{path}: line {line}: {engine.RLE_STATUS[code]}")
+    return out
+
+
+def remeasure_results(dataset_name, results_dir, output_dir, *, images=None, scale_bar_fn=None):
+    """Measure the masks a run_inference call saved in results_dir again, without the models: writes output_dir/
+    measurements_results.csv as run_inference would with the scale bars (and settings such as measure_contrast_distribution) of
+    now.  Images and scale bars resolve exactly as in run_inference (images= / the images provider; scale_bar_fn / the scale_bar
+    provider / the package's detector).  Class and Class_Name of an instance are those of its rows in results_dir's
+    measurements_results.csv; an instance without rows there has no contour above the area gate (which depends only on the frame
+    size) and gets none here either."""
+    if os.path.realpath(output_dir) == os.path.realpath(results_dir):
+        raise ValueError("remeasure_results: output_dir must differ from results_dir (its measurements_results.csv is an input)")
+    images = _resolve_images(dataset_name, images)
+    if images is None:
+        raise FileNotFoundError(f"No images registered for dataset '{dataset_name}': call "
+                                "deepemia_b200.functions.inference.set_providers(...) (or pass images=)")
+    images = list(images)
+    sets = load_rle_results(os.path.join(results_dir, "R50_flip_results.csv"), images)
+    with open(os.path.join(results_dir, "measurements_results.csv"), newline="") as f:
+        old = list(csv.reader(f))
+    if not old or old[0] != CSV_HEADER:
+        raise ValueError(f"remeasure_results: {results_dir}/measurements_results.csv does not start with the measurements header")
+    class_of = {r[0]: (r[1], r[2]) for r in old[1:]}
+    os.makedirs(output_dir, exist_ok=True)
+    rows = []
+    for (name, image), (psum, um_pix) in zip(images, _scale_bars(images, dataset_name, _dataset_config(dataset_name), output_dir,
+                                                                  scale_bar_fn)):
+        iset = sets[name]
+        got = measure_masks(iset, [0] * iset.n, image.shape, um_pix, name, psum, original_image=image)
+        for r in got:
+            if r[0] not in class_of:
+                raise ValueError(f"remeasure_results: {r[0]} has a measured contour but no row in {results_dir}/measurements_results.csv")
+            r[1], r[2] = class_of[r[0]]
+        rows += got
+    _write_measurements(output_dir, rows)

@@ -1,5 +1,6 @@
 """Mirror of the reference's src/utils/mask_utils.py (functions on the hot path), computing in libemia.so."""
 import numpy as np
+import torch
 
 from .. import engine
 from . import _bridge
@@ -12,6 +13,19 @@ def rle_encoding(x):
     iset = _bridge.upload([np.asarray(x) == 1])
     _, runs = engine.rle_encode(iset)
     return [int(v) for v in runs.cpu().numpy().reshape(-1)]
+
+
+def rle_decoding(rle, shape):
+    """Companion of rle_encoding, not a function of the reference (which only writes the format): [start, length, ...] (a list of
+    ints or the space-separated EncodedPixels string) -> H x W uint8 0/1 mask.  Raises EmiaError on a malformed run list."""
+    H, W = (int(s) for s in shape[:2])
+    vals = np.asarray([int(v) for v in rle.split()] if isinstance(rle, str) else list(rle), np.int64)
+    if vals.size % 2:
+        raise engine._lib.EmiaError(f"rle_decoding: odd number of values ({vals.size})")
+    dev = engine._need_cuda(None)
+    run_off = torch.tensor([0, vals.size // 2], dtype=torch.int64, device=dev)
+    runs = torch.as_tensor(vals.reshape(-1, 2), device=dev).contiguous()
+    return engine.unpack_masks(engine.rle_decode(run_off, runs, H, W))[0].cpu().numpy()
 
 
 def postprocess_masks(ori_mask, ori_score, image, min_crys_size=None):

@@ -284,6 +284,43 @@ int emia_rle_count(const uint32_t* crops, const emia_inst_meta* meta, const int6
                    int64_t n, int H, int64_t* n_runs, void* stream);
 int emia_rle_encode(const uint32_t* crops, const emia_inst_meta* meta, const int64_t* crop_off, const int32_t* bbox,
                     int64_t n, int H, const int64_t* run_off, int64_t* runs, void* stream);
+
+/* ---- K6 read-back: R50_flip_results.csv text -> runs -> instances (csrc/emia_rle_kernels.cuh, core/emia_rle.cuh) ------------------
+ * Text -> runs, each step count / emia_exclusive_scan_i64 / fill:
+ * emia_rle_line_count : chunk_lines[c] = number of '\n' in bytes [c * EMIA_RLE_TEXT_CHUNK, (c + 1) * EMIA_RLE_TEXT_CHUNK) of the
+ *   text (caller scans the ceil(nbytes / EMIA_RLE_TEXT_CHUNK) counts).
+ * emia_rle_line_index : line k of the text is bytes [line_off[k], line_off[k + 1]) (its '\n' included); line_off has
+ *   chunk_off[last] + 2 entries, of which the last is only written (= nbytes) when the text does not end with '\n'.
+ * emia_rle_parse_count: for the n_lines lines [line_off[j], line_off[j + 1]) (the caller skips the header): data_cnt[j] = 1 unless
+ *   the line is empty (only blanks: ' ', '\r', '\n'), run_cnt[j] = runs of a well-formed data line (caller scans both, n_lines + 1).
+ * emia_rle_parse_fill : per data line d (in line order): line_idx[d] = j, field[d] = byte range [begin, end) of its ImageId (the
+ *   text before the LAST comma of the line, quotes included), status[d] = EMIA_RLE_* (0 = OK), run_off[d] (D + 1 entries) and the
+ *   (start, length) values at runs[2 * run_off[d] ..].  An empty EncodedPixels field is an empty mask.
+ * Runs -> instances (the exact inverse of emia_rle_encode; canonical tight-bbox geometry of emia_mask_bbox):
+ * emia_rle_decode_plan: instance i = line rows[i] (rows NULL: i) of run_off / runs, in an H x W frame (1 <= H, W <= 65535): meta,
+ *   crop_words (caller scans), bbox, area and status[i]; a rejected instance (status != 0) gets bbox -1, area 0 and no crop.
+ * emia_rle_decode     : writes every crop word once (no zero pass needed). */
+#define EMIA_RLE_TEXT_CHUNK 8192
+#define EMIA_RLE_OK 0
+#define EMIA_RLE_NO_SEPARATOR 1   /* no comma in a non-empty line */
+#define EMIA_RLE_BAD_CHAR 2       /* EncodedPixels holds a character other than a digit or a blank */
+#define EMIA_RLE_ODD_COUNT 3      /* odd number of values */
+#define EMIA_RLE_LONG_VALUE 4     /* a value of more than 18 digits */
+#define EMIA_RLE_BAD_RUN 5        /* start < 1 or length < 1 */
+#define EMIA_RLE_PAST_END 6       /* a run past pixel H * W */
+#define EMIA_RLE_UNSORTED 7       /* a run that starts at or before the end of the previous run */
+#define EMIA_RLE_AREA 8           /* more than INT32_MAX pixels */
+int emia_rle_line_count(const uint8_t* text, int64_t nbytes, int64_t* chunk_lines, void* stream);
+int emia_rle_line_index(const uint8_t* text, int64_t nbytes, const int64_t* chunk_off, int64_t* line_off, void* stream);
+int emia_rle_parse_count(const uint8_t* text, const int64_t* line_off, int64_t n_lines, int64_t* data_cnt, int64_t* run_cnt,
+                         void* stream);
+int emia_rle_parse_fill(const uint8_t* text, const int64_t* line_off, int64_t n_lines, const int64_t* data_off,
+                        const int64_t* run_scan, int64_t* run_off, int64_t* runs, int64_t* field, int32_t* line_idx,
+                        int32_t* status, void* stream);
+int emia_rle_decode_plan(const int64_t* runs, const int64_t* run_off, const int32_t* rows, int64_t n, int H, int W,
+                         emia_inst_meta* meta, int64_t* crop_words, int32_t* bbox, int32_t* area, int32_t* status, void* stream);
+int emia_rle_decode(const int64_t* runs, const int64_t* run_off, const int32_t* rows, int64_t n, int H,
+                    const emia_inst_meta* meta, const int64_t* crop_off, uint32_t* crops, void* stream);
 /* raw moments (m00, m10, m01) of every instance as exact integers: cv2.moments(mask) of src/functions/inference.py:1101-1104 */
 int emia_moments01(const uint32_t* crops, const emia_inst_meta* meta, const int64_t* crop_off, int64_t n, int64_t* out,
                    void* stream);
