@@ -101,7 +101,6 @@ _SIGNATURES = {
                                   c_void_p, c_void_p]),
     "emia_gather_b32": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "emia_capacity_guard": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_void_p]),
-    "emia_capacity_guard_ranges": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_void_p, c_void_p]),
     "emia_scalebar_edges": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
                                     c_void_p]),
     "emia_hough_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int, c_int]),

@@ -86,8 +86,7 @@ def paste_units(hb, arena, tag):
     """K1 over every unit of the batch (crops only), sync-free."""
     n = hb.n
     meta, crop_off = engine.paste_plan(hb.boxes, hb.H, hb.W, hb.scale_x, hb.scale_y)
-    cap = arena.cap(tag + ".crops", n * 1024 + 65536)
-    arena.guard(tag + ".crops", crop_off[n:], meta, n)
+    cap = engine.buffer_len(crop_off[n:], n, arena, tag + ".crops", n * 1024 + 65536, meta)
     crops = torch.empty(cap, dtype=torch.int32, device=hb.boxes.device)
     return engine.paste(hb.probs, hb.boxes, hb.H, hb.W, scores=hb.scores, classes=hb.classes, scale_x=hb.scale_x, scale_y=hb.scale_y,
                         plan=(meta, crop_off, cap), crops_out=crops, abort=arena.abort)
@@ -232,14 +231,14 @@ def tile_pipeline(full_hb, tile_hb, tile_xy, image_hw, tile_size, overlap_ratio,
         tile_out.idx[:kt.idx.numel()].copy_(kt.idx)
     per_class_in = engine.flatten(final, lists, id_add, cache=tabs.setdefault("f1", {}))
     # ---- per class and image: deduplicate_masks_smart at 0.4 (needs the contour perimeters of the compactness pre-filter)
-    _trace(iset, arena, "k5")
+    engine.trace(iset, arena=arena)
     sp2 = _space_like(tabs, "sp2", per_class_in, dev)
     engine.dedup_smart(iset, per_class_in, 0.4, out=sp2.section(0))
     # ---- all classes of an image: deduplicate_masks_smart at 0.7, spatial constraints, morphometry
     allc = engine.flatten(sp2, cross, cache=tabs.setdefault("f2", {}))
     kept = engine.dedup_smart(iset, allc, cross_class_iou)
     kept = engine.apply_spatial_constraints(iset, kept, rules)
-    meas = _measure(iset, kept, um_pix, min_area, arena, "k5") if measure else None
+    meas = engine.measure_list(iset, kept, um_pix=um_pix, min_area=min_area, arena=arena) if measure else None
     return FlowResult(iset=iset, per_class=sp2.section(0), kept=kept, meas=meas, extra={"combined": comb})
 
 
@@ -250,24 +249,6 @@ def _space_like(tabs, name, groups, dev):
         proto = engine.GroupSpace([np.diff(groups.cap_off_host).astype(np.int64)], dev)
         tabs[name] = proto
     return proto.fresh()
-
-
-def _trace(iset, arena, tag):
-    cap = arena.cap(tag + ".pts", iset.n * 1536 + 65536)
-    iset.extra["pt_cap_total"] = cap
-    engine.trace(iset, single_pass=True, abort=arena.abort)
-    arena._totals.append((tag + ".pts", iset.extra["pt_total"]))
-    arena.caps.setdefault(tag + ".pts", cap)
-
-
-def _measure(iset, groups, um_pix, min_area, arena, tag):
-    L = groups.total_cap
-    rec_cap = arena.cap(tag + ".records", L + L // 8 + 64)
-    scr_cap = arena.cap(tag + ".scratch", L * 4096 + 65536)
-    m = engine.measure_list(iset, groups, um_pix=um_pix, min_area=min_area, capacity=(rec_cap, scr_cap), abort=arena.abort)
-    arena._totals.append((tag + ".records", m.totals[0:1]))
-    arena._totals.append((tag + ".scratch", m.totals[1:2]))
-    return m
 
 
 def ensemble_multiscale(heads, weights, image_hw, params, arena, sorted_iou=0.4, rules=None, um_pix=1.0, measure=True,
@@ -335,7 +316,7 @@ def ensemble_multiscale(heads, weights, image_hw, params, arena, sorted_iou=0.4,
     per_class_in = engine.flatten(final, lists, id_add, cache=tabs.setdefault("f1", {}))
     sp2 = _space_like(tabs, "sp2", per_class_in, dev)
     s_sorted = engine.dedup_sorted(iset, per_class_in, sorted_iou)
-    _trace(iset, arena, "k5")
+    engine.trace(iset, arena=arena)
     # one deduplicate_masks_smart call per class threshold (lists of the other classes pass through empty)
     thr = sorted(set(p.iou_threshold for p in params))
     if len(thr) == 1:
@@ -351,7 +332,7 @@ def ensemble_multiscale(heads, weights, image_hw, params, arena, sorted_iou=0.4,
     allc = engine.flatten(sp2, cross, cache=tabs.setdefault("f2", {}))
     kept = engine.dedup_smart(iset, allc, 0.7)
     kept = engine.apply_spatial_constraints(iset, kept, rules)
-    meas = _measure(iset, kept, um_pix, min_area, arena, "k5") if measure else None
+    meas = engine.measure_list(iset, kept, um_pix=um_pix, min_area=min_area, arena=arena) if measure else None
     return FlowResult(iset=iset, per_class=sp2.section(0), kept=kept, meas=meas, extra={"combined": comb, "posts": posts})
 
 
@@ -376,13 +357,14 @@ def pad_units(probs, boxes, scores, classes, unit_off, cap):
 
 class GraphedFlow:
     """fn(arena) -> FlowResult over STATIC input tensors, captured into a CUDA graph after the eager runs have filled the
-    layout caches and settled the arena's capacities.  replay() enqueues the whole flow as one graph launch; the abort flag
-    and the totals are read by finish() exactly as after an eager run."""
+    layout caches and settled the arena's capacities.  replay() enqueues the whole flow as one graph launch; finish() checks
+    the captured run (abort flag and totals, rewritten by every replay) exactly as after an eager run."""
 
     def __init__(self, fn, arena, pool=None):
         self.fn, self.arena, self.pool = fn, arena, pool
         self.graph = None
         self.res = None
+        self._run = None
         self.launches = 0
 
     def settle(self, max_runs=12):
@@ -399,18 +381,20 @@ class GraphedFlow:
         l0 = engine.LAUNCHES["count"]
         g = torch.cuda.CUDAGraph()
         with torch.cuda.graph(g, pool=self.pool):
-            self.arena.begin()
+            self._run = self.arena.begin()
             self.res = self.fn(self.arena)
-        self.abort = self.arena.abort
-        self.totals = list(self.arena._totals)
         self.graph = g
         self.launches = engine.LAUNCHES["count"] - l0
         return self
+
+    @property
+    def abort(self):
+        """Abort flag of the captured run (device int32, rewritten by every replay)."""
+        return self._run[0]
 
     def replay(self):
         self.graph.replay()
         return self.res
 
     def finish(self):
-        self.arena.abort, self.arena._totals = self.abort, self.totals
-        return self.arena.finish()
+        return self.arena.finish(self._run)

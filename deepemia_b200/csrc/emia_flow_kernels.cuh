@@ -12,7 +12,7 @@
 //   emia_unit_broadcast_i32  : per-unit constants (tile x / y offsets :2411-2414) expanded to instances
 //   emia_scale_f32           : `score * weight` of the ensemble (:1553)
 //   emia_gather_*            : boolean / fancy indexing of instance arrays (replaces per-mask Python list handling)
-//   emia_capacity_guard*     : sync-free execution — variable-size outputs go into caller-sized arenas; a total that exceeds
+//   emia_capacity_guard      : sync-free execution — variable-size outputs go into caller-sized arenas; a total that exceeds
 //                              its arena raises the abort flag AND empties the instance geometry, so that no later kernel
 //                              touches memory outside the arenas; the host looks at the flag once, with the results.
 #pragma once
@@ -39,21 +39,6 @@ extern "C" int emia_capacity_guard(const int64_t* total, int64_t capacity, int32
     // the flag is read by every thread before any thread of the grid may set it only when `over` already holds for all of them
     k_capacity_guard<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(total, capacity, abort_flag, poison_meta, poison_n);
     return emia_check_launch("emia_capacity_guard launch: %s");
-}
-// every range offsets[bounds[b+1]] - offsets[bounds[b]] (b < B) must fit `capacity`
-__global__ void k_capacity_guard_ranges(const int64_t* __restrict__ offsets, const int64_t* __restrict__ bounds, int B,
-                                        int64_t capacity, int32_t* __restrict__ abort_flag) {
-    const int b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (b >= B) return;
-    if (offsets[bounds[b + 1]] - offsets[bounds[b]] > capacity) *abort_flag = 1;
-}
-extern "C" int emia_capacity_guard_ranges(const int64_t* offsets, const int64_t* bounds, int32_t B, int64_t capacity,
-                                          int32_t* abort_flag, void* stream) {
-    if (B < 0 || capacity < 0) return emia_fail(EMIA_ERR_BAD_ARG, "emia_capacity_guard_ranges: %s", "bad argument");
-    if (B == 0) return EMIA_OK;
-    if (!offsets || !bounds || !abort_flag) return emia_fail(EMIA_ERR_BAD_ARG, "emia_capacity_guard_ranges: %s", "null pointer");
-    k_capacity_guard_ranges<<<(unsigned)((B + 127) / 128), 128, 0, (cudaStream_t)stream>>>(offsets, bounds, B, capacity, abort_flag);
-    return emia_check_launch("emia_capacity_guard_ranges launch: %s");
 }
 
 // ---- list filters ---------------------------------------------------------------------------------------------------------

@@ -92,14 +92,18 @@ def exclusive_scan_(t):
 
 
 class Arena:
-    """Capacities of the variable-size device buffers of a flow (crop words, contour vertices, records, ...).
+    """Capacities of the variable-size device buffers of a flow (crop words, contour vertices, records, ...): the one place
+    that decides how such a buffer is sized when its size is known only after a device-side scan (see buffer_len()).
 
-    A flow is enqueued WITHOUT reading any size back: every variable-size output goes into a buffer of the arena's current
-    capacity, a device-side guard (emia_capacity_guard) compares the real total with it, and on overflow raises the abort
-    flag and empties the geometry of the affected instance set, so that no later kernel touches memory outside the buffers.
-    finish() is the one host synchronisation of a run: it reads the flag and the recorded totals, grows the capacities that
-    were too small and tells the caller to run again.  Capacities only grow, in 25 % steps: shards of similar size keep
-    running sync-free whatever their exact instance counts are."""
+    A run is enqueued WITHOUT reading any size back: begin() makes a fresh abort flag, every variable-size output goes into a
+    buffer of the arena's current capacity, and a device-side guard (emia_capacity_guard) compares the real total with it.
+    On overflow the guard raises the abort flag and empties the geometry of the affected instance set, so that no later
+    kernel touches memory outside the buffers.  finish() is the one host synchronisation of a run: it reads the flag and the
+    recorded totals, grows the capacities that were too small (fit()) and tells the caller to run again.
+
+    Capacities only grow, to total * margin + 64, so that shards of similar size keep running sync-free whatever their exact
+    instance counts are.  The batched flows use margin 1.25.  TilePipeline uses its hint_margin, 1.05: it fits its capacities
+    to the totals of an exact-size run, and an overflow there makes the next run exact again."""
 
     def __init__(self, device, margin=1.25):
         self.dev = torch.device(device)
@@ -111,10 +115,12 @@ class Arena:
         self.aborts = 0
 
     def begin(self):
+        """Start a run: a fresh abort flag and no recorded totals.  Returns the run (abort flag, recorded totals), which
+        finish(run) can check after later runs have begun (a run captured in a CUDA graph and replayed)."""
         self.abort = torch.zeros(1, dtype=torch.int32, device=self.dev)
         self._totals = []
         self.runs += 1
-        return self.abort
+        return self.abort, self._totals
 
     def cap(self, name, default):
         c = self.caps.get(name)
@@ -122,6 +128,10 @@ class Arena:
             c = max(int(default), 1)
             self.caps[name] = c
         return c
+
+    def fit(self, name, total):
+        """Raise the capacity of `name` to total * margin + 64 when that is larger."""
+        self.caps[name] = max(self.caps.get(name, 0), int(total * self.margin) + 64)
 
     def guard(self, name, total, poison_meta=None, poison_n=0):
         """total: int64 device tensor view of ONE element (e.g. crop_off[n:]).  Enqueues the device-side check."""
@@ -132,21 +142,35 @@ class Arena:
         LAUNCHES["count"] += 1
         self._totals.append((name, total))
 
-    def finish(self):
-        """One host synchronisation: True when the run is valid; False when a guard tripped (capacities grown: run again)."""
-        vals = torch.cat([self.abort.to(torch.int64)] + [t.reshape(-1)[:1] for _, t in self._totals]).tolist()
+    def finish(self, run=None):
+        """One host synchronisation: True when the run (default: the last one begun) is valid; False when a guard tripped
+        (capacities grown: run again)."""
+        abort, totals = run if run is not None else (self.abort, self._totals)
+        vals = torch.cat([abort.to(torch.int64)] + [t.reshape(-1)[:1] for _, t in totals]).tolist()
         if not vals[0]:
             return True
         self.aborts += 1
         grown = False
-        for (name, _), v in zip(self._totals, vals[1:]):
+        for (name, _), v in zip(totals, vals[1:]):
             if v > self.caps[name]:
-                self.caps[name] = int(v * self.margin) + 64
+                self.fit(name, v)
                 grown = True
         if not grown:       # the flag came from a kernel-side overflow (contour slab): give everything more room
             for k in self.caps:
                 self.caps[k] = int(self.caps[k] * 2)
         return False
+
+
+def buffer_len(total, n, arena=None, name=None, default=0, poison_meta=None):
+    """Elements to allocate for a variable-length buffer of n instances whose size is the device scalar `total` (an int64 view
+    of one element, e.g. crop_off[n:], after the scan).  Without an arena: the total read back (one host synchronisation; 0,
+    without one, when n == 0).  With an arena: its capacity for `name` (`default` on first use), checked on the device by a
+    guard that, on overflow, also empties the geometry poison_meta [n, 8] of the instances."""
+    if arena is None:
+        return int(total.item()) if n else 0
+    c = arena.cap(name, default)
+    arena.guard(name, total, poison_meta, n if poison_meta is not None else 0)
+    return c
 
 
 @dataclass
@@ -217,7 +241,7 @@ def paste(probs, boxes, H, W, scores=None, classes=None, scale_x=1.0, scale_y=1.
     f16 = (1 << 16) if probs.dtype == torch.float16 else 0      # EMIA_PASTE_PROBS_F16: AMP heads, widened exactly in the kernel
     if plan is None:
         meta, crop_off = paste_plan(boxes, H, W, scale_x, scale_y)
-        total = int(crop_off[n].item()) if n else 0
+        total = buffer_len(crop_off[n:], n)
     else:
         meta, crop_off, total = plan
         assert meta.shape[0] == n and crop_off.numel() == n + 1 and meta.is_contiguous() and crop_off.is_contiguous()
@@ -259,7 +283,7 @@ def from_masks(masks, scores=None, classes=None):
     st = _stream()
     _lib.check(lib.emia_mask_bbox(_ptr(masks), n, H, W, _ptr(meta), _ptr(crop_off), _ptr(bbox), _ptr(area), st), "emia_mask_bbox")
     exclusive_scan_(crop_off)
-    total = int(crop_off[n].item()) if n else 0
+    total = buffer_len(crop_off[n:], n)
     crops = torch.empty(max(total, 1), dtype=torch.int32, device=dev)
     _lib.check(lib.emia_mask_pack(_ptr(masks), n, H, W, _ptr(meta), _ptr(crop_off), _ptr(crops), st), "emia_mask_pack")
     LAUNCHES["count"] += 2
@@ -298,11 +322,7 @@ def _pad_plan(iset, arena=None, tag="k2"):
     _lib.check(lib.emia_morph_plan(_ptr(iset.meta), iset.n, _ptr(pad_off), _stream()), "emia_morph_plan")
     exclusive_scan_(pad_off)
     LAUNCHES["count"] += 1
-    if arena is not None:
-        total = arena.cap(tag + ".work", 1 << 18)
-        arena.guard(tag + ".work", pad_off[iset.n:], iset.meta, iset.n)
-    else:
-        total = int(pad_off[iset.n].item()) if iset.n else 0
+    total = buffer_len(pad_off[iset.n:], iset.n, arena, tag + ".work", 1 << 18, iset.meta)
     work = torch.empty(int(lib.emia_morph_scratch_words()) + 3 * total + 1, dtype=torch.int32, device=iset.device)
     iset.extra["pad_plan"] = (pad_off, work)
     return pad_off, work
@@ -350,11 +370,8 @@ def morph(iset, ops, apply=None, arena=None, tag="k2", ops_b=None):
                    "emia_morph_grow_plan")
         exclusive_scan_(crop_off_out)
         LAUNCHES["count"] += 1
-        if arena is not None:
-            total = arena.cap(tag + ".grown", int(iset.total_crop_words * 1.5) + 4 * iset.n + 1024)
-            arena.guard(tag + ".grown", crop_off_out[iset.n:], meta_out, iset.n)
-        else:
-            total = int(crop_off_out[iset.n].item())
+        total = buffer_len(crop_off_out[iset.n:], iset.n, arena, tag + ".grown", int(iset.total_crop_words * 1.5) + 4 * iset.n + 1024,
+                           meta_out)
         geometry = (meta_out, crop_off_out, total)
         crops = torch.empty(max(total, 1), dtype=torch.int32, device=iset.device)
     else:
@@ -470,11 +487,13 @@ def default_min_area(H, W):
     return max(5, H * W * 0.000005 * 0.05)
 
 
-def trace(iset, single_pass=True, marks=None, abort=None):
+def trace(iset, single_pass=True, marks=None, arena=None, tag="k5", pt_cap=None):
     """K5a: external contours of every instance.  Leaves on the device: vertex lists (pts, cstart), the number of contours and
     the hull scratch size per instance, and perim0 = arcLength(contours[0]) (the compactness pre-filter of
-    deduplicate_masks_smart needs it).  single_pass follows every border once into bounded per-instance slabs and does NOT
-    synchronise; an overflow (counter in extra["overflow"]) is detected by the next measure*() call, which re-traces exactly."""
+    deduplicate_masks_smart needs it).  single_pass follows every border once into bounded per-instance slabs; an overflow
+    (counter in extra["overflow"]) is detected by the next measure*() call, which re-traces exactly.  The vertex buffer of
+    the single pass is sized by buffer_len() (capacity tag + ".pts" of the arena), or takes pt_cap when the caller already
+    knows the exact size."""
     lib = _lib.load()
     dev = iset.device
     n = iset.n
@@ -488,21 +507,15 @@ def trace(iset, single_pass=True, marks=None, abort=None):
         with _stage("k5_plan+scan"):
             _lib.check(lib.emia_contour_trace_plan(_ptr(iset.meta), n, _ptr(sizes[1]), st), "emia_contour_trace_plan")
             exclusive_scan_(sizes[1])
-        cap_total = iset.extra.get("pt_cap_total")
-        if cap_total is None:
-            # capacity is a pure function of the crop sizes: 4 * (sum ch + 32 * sum cw) + 32 * n_live
-            cap_total = int(sizes[1, n].item())
-        elif abort is not None:
-            # sync-free: the caller sized the vertex buffer; the device checks it and the trace kernel honours the flag
-            _lib.check(lib.emia_capacity_guard(_ptr(sizes[1, n:]), int(cap_total), _ptr(abort), 0, 0, st), "emia_capacity_guard")
-            LAUNCHES["count"] += 1
-            iset.extra["pt_total"] = sizes[1, n:]
+        # the size is a pure function of the crop sizes: 4 * (sum ch + 32 * sum cw) + 32 * n_live
+        cap_total = pt_cap if pt_cap is not None else buffer_len(sizes[1, n:], n, arena, tag + ".pts", n * 1536 + 65536)
         pts = torch.empty(max(cap_total, 1), dtype=torch.int32, device=dev)
         cstart = torch.empty(n * (CAP_CONTOURS + 1) + 1, dtype=torch.int32, device=dev)
         with _stage("k5_trace"):
             _lib.check(lib.emia_contour_trace_slab(_ptr(iset.crops), _ptr(iset.meta), _ptr(iset.crop_off), n, _ptr(marks), _ptr(sizes[1]),
                                                    CAP_CONTOURS, _ptr(pts), _ptr(cstart), _ptr(sizes[0]), _ptr(sizes[2]), _ptr(flag),
-                                                   _ptr(perim0), _ptr(abort), st), "emia_contour_trace_slab")
+                                                   _ptr(perim0), _ptr(arena.abort) if arena is not None else 0, st),
+                       "emia_contour_trace_slab")
         LAUNCHES["count"] += 2
         iset.cstart_stride = CAP_CONTOURS + 1
         iset.extra["overflow"] = flag
@@ -560,12 +573,12 @@ class Measurements:
                 for g in range(self.groups.G)]
 
 
-def measure_list(iset, groups, um_pix=1.0, min_area=None, capacity=None, abort=None):
+def measure_list(iset, groups, um_pix=1.0, min_area=None, arena=None, tag="k5"):
     """K5b: morphometry of the members of `groups` only (what the reference's measurement loop sees).  Needs trace().
     Returns None when the single-pass trace overflowed (the caller re-traces with single_pass=False).
-    capacity = (records, scratch bytes) + abort (device int32 flag): no host synchronisation — the buffers take the given
-    capacities, the flag is raised on the device when the actual totals (or a slab) overflow, and nothing is written then;
-    the returned Measurements has n_records = None until finalize()."""
+    With an arena there is no host synchronisation: the buffers take the arena's capacities tag + ".records" and
+    tag + ".scratch" (bytes), its abort flag is raised on the device when the actual totals (or a slab) overflow, and nothing
+    is written then; the returned Measurements has n_records = None until finalize()."""
     lib = _lib.load()
     dev = iset.device
     assert iset.pts is not None, "run trace() first"
@@ -583,15 +596,14 @@ def measure_list(iset, groups, um_pix=1.0, min_area=None, capacity=None, abort=N
         exclusive_scan_(offs[1])
     LAUNCHES["count"] += 1
     flag = iset.extra.get("overflow")
-    if capacity is not None:
-        n_rec, n_scr = int(capacity[0]), int(capacity[1])
+    if arena is not None:
         # device-side checks, stream-ordered before the kernels that honour the flag (a slab overflow of the trace counts too)
-        _lib.check(lib.emia_capacity_guard(_ptr(offs[0, L:]), n_rec, _ptr(abort), 0, 0, st), "emia_capacity_guard")
-        _lib.check(lib.emia_capacity_guard(_ptr(offs[1, L:]), n_scr, _ptr(abort), 0, 0, st), "emia_capacity_guard")
-        LAUNCHES["count"] += 2
+        n_rec = buffer_len(offs[0, L:], L, arena, tag + ".records", L + L // 8 + 64)
+        n_scr = buffer_len(offs[1, L:], L, arena, tag + ".scratch", L * 4096 + 65536)
         if flag is not None:
-            abort.logical_or_(flag)
+            arena.abort.logical_or_(flag)
     else:
+        # one read for both totals and the slab overflow flag
         tot = torch.stack([offs[0, L], offs[1, L], flag[0].to(torch.int64) if flag is not None else offs[0, 0]]).tolist()
         n_rec, n_scr, overflow = int(tot[0]), int(tot[1]), int(tot[2])
         if overflow:
@@ -615,10 +627,10 @@ def measure_list(iset, groups, um_pix=1.0, min_area=None, capacity=None, abort=N
             _lib.check(lib.emia_contour_measure_list(L, _ptr(item_inst), _ptr(offs[0]), _ptr(offs[1]), _ptr(iset.cont_off),
                                                      _ptr(iset.pt_off), _ptr(iset.cstart), iset.cstart_stride, float(um_pix),
                                                      float(min_area), _ptr(iset.pts), _ptr(records), _ptr(rec_inst), _ptr(scratch),
-                                                     _ptr(abort) if capacity is not None else 0, _ptr(order) if order is not None else 0, st),
-                       "emia_contour_measure_list")
+                                                     _ptr(arena.abort) if arena is not None else 0, _ptr(order) if order is not None else 0,
+                                                     st), "emia_contour_measure_list")
         LAUNCHES["count"] += 2
-    if capacity is not None:
+    if arena is not None:
         return Measurements(records=records, rec_inst=rec_inst, rec_off=offs[0], n_records=None, groups=groups,
                             totals=torch.stack([offs[0, L], offs[1, L]]))
     return Measurements(records=records[:n_rec], rec_inst=rec_inst[:n_rec], rec_off=offs[0], n_records=n_rec, groups=groups,
@@ -937,7 +949,7 @@ def resize_place(iset, th, tw, Hd, Wd, off_xy=None, tile_size=None, overlap_rati
     _lib.check(lib.emia_resize_place_plan(_ptr(iset.bbox), n, iset.H, iset.W, th, tw, _ptr(off_xy), 0, Hd, Wd, _ptr(meta), _ptr(crop_off), st),
                "emia_resize_place_plan")
     exclusive_scan_(crop_off)
-    total = int(crop_off[n].item()) if n else 0
+    total = buffer_len(crop_off[n:], n)
     crops = torch.empty(max(total, 1), dtype=torch.int32, device=dev)
     bbox = torch.empty((n, 4), dtype=torch.int32, device=dev)
     area = torch.empty(n, dtype=torch.int32, device=dev)
@@ -999,11 +1011,8 @@ class Combined:
         lib = _lib.load()
         n = self.n
         exclusive_scan_(self.crop_off)
-        if arena is not None:
-            total = arena.cap(tag + ".crops", sum(int(part[1].total_crop_words) for part in self._parts) + 64 * n + 1024)
-            arena.guard(tag + ".crops", self.crop_off[n:], self.meta, n)
-        else:
-            total = int(self.crop_off[n].item()) if n else 0
+        total = buffer_len(self.crop_off[n:], n, arena, tag + ".crops",
+                           sum(int(part[1].total_crop_words) for part in self._parts) + 64 * n + 1024, self.meta)
         self.total = total
         self.crops = torch.empty(max(total, 1), dtype=torch.int32, device=self.dev)
         st = _stream()
@@ -1092,7 +1101,7 @@ def select(iset, idx):
     out = _empty_set(k, iset.H, iset.W, dev, iset.scores is not None, iset.classes is not None)
     _gather_into(iset, idx_t, k, out.meta, out.crop_off, 0)
     exclusive_scan_(out.crop_off)
-    total = int(out.crop_off[k].item()) if k else 0
+    total = buffer_len(out.crop_off[k:], k)
     out.crops = torch.empty(max(total, 1), dtype=torch.int32, device=dev)
     out.total_crop_words = total
     _gather_copy(iset, idx_t, k, out, 0)
@@ -1112,7 +1121,7 @@ def concat(isets):
         _gather_into(s_, None, s_.n, out.meta, out.crop_off, a)
         a += s_.n
     exclusive_scan_(out.crop_off)
-    total = int(out.crop_off[n].item()) if n else 0
+    total = buffer_len(out.crop_off[n:], n)
     out.crops = torch.empty(max(total, 1), dtype=torch.int32, device=dev)
     out.total_crop_words = total
     a = 0
@@ -1133,7 +1142,7 @@ def rle_encode(iset, idx=None):
     _lib.check(lib.emia_rle_count(_ptr(iset.crops), _ptr(iset.meta), _ptr(iset.crop_off), _ptr(iset.bbox), n, iset.H, _ptr(run_off), st),
                "emia_rle_count")
     exclusive_scan_(run_off)
-    R = int(run_off[n].item()) if n else 0
+    R = buffer_len(run_off[n:], n)
     runs = torch.empty((max(R, 1), 2), dtype=torch.int64, device=dev)
     _lib.check(lib.emia_rle_encode(_ptr(iset.crops), _ptr(iset.meta), _ptr(iset.crop_off), _ptr(iset.bbox), n, iset.H, _ptr(run_off),
                                    _ptr(runs), st), "emia_rle_encode")
@@ -1234,7 +1243,7 @@ def _rle_decode(run_off, runs, H, W, rows=None):
         _lib.check(lib.emia_rle_decode_plan(rp, _ptr(run_off), _ptr(rows_t), n, H, W, _ptr(meta), _ptr(crop_off), _ptr(bbox), _ptr(area),
                                             _ptr(status), st), "emia_rle_decode_plan")
         exclusive_scan_(crop_off)
-        total = int(crop_off[n].item()) if n else 0
+        total = buffer_len(crop_off[n:], n)
         crops = torch.empty(max(total, 1), dtype=torch.int32, device=dev)
         _lib.check(lib.emia_rle_decode(rp, _ptr(run_off), _ptr(rows_t), n, H, _ptr(meta), _ptr(crop_off), _ptr(crops), st),
                    "emia_rle_decode")
@@ -1470,15 +1479,21 @@ def run_tiles(probs, boxes, scores, classes, tile_offsets, H, W, um_pix=0.5, rul
     Returns (InstanceSet, Groups of kept instances, Measurements of the kept instances)."""
     iset = paste(probs, boxes, H, W, scores=scores, classes=classes, scale_x=scale_x, scale_y=scale_y, frames=frames,
                  variant=variant)
-    groups = groups_from_offsets(tile_offsets, iset.device)
+    kept, meas, _ = _post_paste(iset, groups_from_offsets(tile_offsets, iset.device), um_pix, rules, dedup_iou)
+    return iset, kept, meas
+
+
+def _post_paste(iset, groups, um_pix, rules, dedup_iou, marks=None, pt_cap=None, arena=None):
+    """trace -> deduplicate_masks_smart -> spatial constraints -> morphometry of the survivors.  Without an arena the sizes
+    are read back and a contour slab that overflowed is traced again with exact sizes.  Returns (kept, meas, retraced)."""
     single_pass = True
     while True:
-        trace(iset, single_pass=single_pass)
+        trace(iset, single_pass=single_pass, marks=marks, arena=arena, pt_cap=pt_cap)
         kept = dedup_smart(iset, groups, iou_threshold=dedup_iou)
         kept = apply_spatial_constraints(iset, kept, rules)
-        meas = measure_list(iset, kept, um_pix=um_pix)
+        meas = measure_list(iset, kept, um_pix=um_pix, arena=arena)
         if meas is not None:
-            return iset, kept, meas
+            return kept, meas, not single_pass
         single_pass = False      # a slab overflowed: follow the borders again with exact sizes
 
 
@@ -1490,8 +1505,10 @@ class TilePipeline:
         post  : contours -> de-dup -> spatial constraints -> morphometry of batch b-1 (latency bound) [+ D2H of its results]
 
     so the latency-bound kernels run in the shadow of the bandwidth-bound paste (and, end to end, of the PCIe copy).
-    The plan (crop geometry, vertex capacities) of the WHOLE shard is computed first, with one small device->host read of
-    the per-batch totals; each batch then needs one more read (record/scratch totals) on the post stream only.
+    The first run of a batch count is exact: the plan (crop geometry, vertex capacities) of the WHOLE shard is computed
+    first, with one small device->host read of the per-batch totals; each batch then needs one more read (record/scratch
+    totals) on the post stream only.  Its totals are fitted into an Arena of that batch count (margin hint_margin), and
+    later runs are enqueued sync-free against those capacities (see aborted()).
     Batches see slices of shard-wide arrays; list indices stay shard-global."""
 
     def __init__(self, H, W, um_pix=1.0, rules=None, dedup_iou=0.7, frames=None, variant=2, batches=8, paste_ctas_per_sm=0,
@@ -1506,9 +1523,9 @@ class TilePipeline:
         self._groups_cache = {}
         self._pinned = {}
         self.k1_events = []
-        # sizes of the previous run per shard shape: the next run of that shape is enqueued without reading anything back
+        # capacities per batch count, fitted to an exact run: the next run of that count is enqueued without reading anything back
         self.sync_free, self.hint_margin = sync_free, hint_margin
-        self._hints, self._ib_cache, self._abort, self._last_hkey, self._stale = {}, {}, None, None, None
+        self._arenas, self._ib_cache, self._abort, self._last_batches = {}, {}, None, None
         self.exact_runs = 0      # runs that read sizes back (host synchronisations); the others are enqueued sync-free
 
     def _groups(self, offs):
@@ -1551,13 +1568,12 @@ class TilePipeline:
         # ---- shard-wide plan: crop geometry + vertex capacities, one read of the per-batch totals
         lib = _lib.load()
         meta, crop_off = paste_plan(d_boxes, self.H, self.W)
-        # Sizes: read back once (the first run of this pipeline, or after a guard tripped); afterwards the buffers take the
-        # CAPACITIES remembered from earlier runs (grown in 25 % steps, independent of the exact per-tile instance counts) and the
-        # real totals are only CHECKED on the device: the whole step is enqueued without a single host synchronisation, the
-        # abort flag is looked at when the results are consumed (aborted()).  A tripped guard makes the paste / trace /
-        # measure kernels write nothing; the caller re-runs, which takes the exact-size path again and raises the capacities.
-        hkey = B
-        hints = self._hints.get(hkey) if self.sync_free else None
+        # Sizes: read back once (the first run of this batch count, or after a guard tripped); afterwards the buffers take the
+        # arena's CAPACITIES (fitted to that exact run, independent of the exact per-tile instance counts) and the real totals
+        # are only CHECKED on the device: the whole step is enqueued without a single host synchronisation, the abort flag is
+        # looked at when the results are consumed (aborted()).  A tripped guard makes the paste / trace / measure kernels write
+        # nothing; the caller re-runs, which takes the exact-size path again and fits new capacities.
+        arena = self._arenas.get(B) if self.sync_free else None
         ikey = offs.tobytes()
         ib_t = self._ib_cache.get(ikey)           # batch boundaries as a device array (an upload, not a size read-back)
         if ib_t is None:
@@ -1565,10 +1581,10 @@ class TilePipeline:
                 self._ib_cache.clear()
             ib_t = torch.as_tensor(ib, device=dev)
             self._ib_cache[ikey] = ib_t
-        abort = torch.zeros(1, dtype=torch.int32, device=dev)
         cap_off = None
-        if hints is None:
+        if arena is None:
             self.exact_runs += 1
+            abort = torch.zeros(1, dtype=torch.int32, device=dev)      # never raised: callers OR every run's flag
             cap_off = torch.empty(n + 1, dtype=torch.int64, device=dev)
             _lib.check(lib.emia_contour_trace_plan(_ptr(meta), n, _ptr(cap_off), _stream()), "emia_contour_trace_plan")
             exclusive_scan_(cap_off)
@@ -1576,11 +1592,10 @@ class TilePipeline:
             bounds = torch.stack([crop_off[ib_t], cap_off[ib_t]]).cpu().numpy()
             total_words = int(bounds[0, -1])
             pt_caps = [int(bounds[1, b + 1] - bounds[1, b]) for b in range(B)]
-            meas_caps = [None] * B
         else:
-            total_words, pt_caps, meas_caps = hints["total_words"], [hints["pt_cap"]] * B, [hints["meas_cap"]] * B
-            _lib.check(lib.emia_capacity_guard(_ptr(crop_off[n:]), total_words, _ptr(abort), 0, 0, _stream()), "emia_capacity_guard")
-            LAUNCHES["count"] += 1
+            abort, _ = arena.begin()
+            total_words = buffer_len(crop_off[n:], n, arena, "k1.crops")
+            pt_caps = [None] * B
         crops = torch.empty(max(total_words, 1), dtype=torch.int32, device=dev)
         marks = torch.empty(max(2 * total_words, 1), dtype=torch.int32, device=dev)
         # under CUDA-graph capture with device inputs (one batch: nothing to overlap) everything runs on the caller's stream: the
@@ -1590,7 +1605,7 @@ class TilePipeline:
         s_paste = main if single else self.s_paste
         s_post = main if single else self.s_post
         if capturing:
-            assert hints is not None, "capture needs the sync-free path: run the shard once eagerly first"
+            assert arena is not None, "capture needs the sync-free path: run the shard once eagerly first"
             time_k1 = False
         s_paste.wait_stream(main); s_post.wait_stream(main)
         isets, ev_paste = [], []
@@ -1605,34 +1620,20 @@ class TilePipeline:
                 it = paste(d_probs[i0:i1], d_boxes[i0:i1], self.H, self.W, scores=d_scores[i0:i1], classes=d_classes[i0:i1],
                            frames=self.frames, variant=self.variant, crops_out=crops,
                            plan=(meta[i0:i1], crop_off[i0:i1 + 1], total_words), ctas_per_sm=self.paste_ctas,
-                           abort=abort if hints is not None else None)
+                           abort=arena.abort if arena is not None else None)
                 if time_k1:
                     e1.record(s_paste); self.k1_events.append((e0, e1))
-                it.extra["pt_cap_total"] = pt_caps[b]
                 e = torch.cuda.Event(); e.record(s_paste); ev_paste.append(e)
                 isets.append(it)
-        out = []
+        out, retraced = [], False
         with torch.cuda.stream(s_post):
             for b in range(B):
                 it = isets[b]
                 s_post.wait_event(ev_paste[b])
                 groups = self._groups(offs[tb[b]:tb[b + 1] + 1] - ib[b])
-                if hints is not None:
-                    trace(it, single_pass=True, marks=marks, abort=abort)
-                    kept = dedup_smart(it, groups, iou_threshold=self.dedup_iou)
-                    kept = apply_spatial_constraints(it, kept, self.rules)
-                    meas = measure_list(it, kept, um_pix=self.um_pix, capacity=meas_caps[b], abort=abort)
-                else:
-                    single_pass = True
-                    while True:
-                        trace(it, single_pass=single_pass, marks=marks)
-                        kept = dedup_smart(it, groups, iou_threshold=self.dedup_iou)
-                        kept = apply_spatial_constraints(it, kept, self.rules)
-                        meas = measure_list(it, kept, um_pix=self.um_pix)
-                        if meas is not None:
-                            break
-                        single_pass = False
-                    meas_caps[b] = (int(meas.totals[0]), int(meas.totals[1])) if single_pass else None
+                kept, meas, again = _post_paste(it, groups, self.um_pix, self.rules, self.dedup_iou, marks=marks, pt_cap=pt_caps[b],
+                                                arena=arena)
+                retraced |= again
                 res = {"tiles": (int(tb[b]), int(tb[b + 1])), "inst0": int(ib[b]), "iset": it, "kept": kept, "meas": meas}
                 if to_host:
                     res["host"] = {k: self._pinned_like(b, k, v).copy_(v, non_blocking=True)
@@ -1644,23 +1645,22 @@ class TilePipeline:
             main.wait_stream(self.s_copy)
         self._keep = (crops, marks, meta, crop_off, cap_off, d_probs)
         self._abort = abort
-        if hints is None and self.sync_free and all(c is not None for c in meas_caps):
-            m = self.hint_margin
-            old = self._hints.get(hkey, {"total_words": 0, "pt_cap": 0, "meas_cap": (0, 0)})
-            bucket = lambda v, prev: max(prev, int(v * m) + 64)        # capacities only grow
-            self._hints[hkey] = {"total_words": bucket(total_words, old["total_words"]),
-                                 "pt_cap": bucket(max(pt_caps), old["pt_cap"]),
-                                 "meas_cap": (bucket(max(c[0] for c in meas_caps), old["meas_cap"][0]),
-                                              bucket(max(c[1] for c in meas_caps), old["meas_cap"][1]))}
-        self._last_hkey = hkey
+        if arena is None and self.sync_free and not retraced:
+            arena = Arena(dev, margin=self.hint_margin)
+            arena.fit("k1.crops", total_words)
+            arena.fit("k5.pts", max(pt_caps))
+            arena.fit("k5.records", max(r["meas"].totals[0] for r in out))
+            arena.fit("k5.scratch", max(r["meas"].totals[1] for r in out))
+            self._arenas[B] = arena
+        self._last_batches = B
         return out
 
     def aborted(self):
-        """True when a capacity guard (or a contour slab) tripped in the last sync-free run(): its results are invalid, the hints
-        of that shard shape are dropped and the caller runs again (exact-size path).  One host synchronisation."""
+        """True when a capacity guard (or a contour slab) tripped in the last sync-free run(): its results are invalid, the arena
+        of that batch count is dropped and the caller runs again (exact-size path).  One host synchronisation."""
         if self._abort is None or not bool(self._abort.item()):
             return False
-        self._stale = self._hints.pop(self._last_hkey, None)      # the next run re-measures and raises the capacities
+        self._arenas.pop(self._last_batches, None)      # the next run re-measures and fits new capacities
         return True
 
     def _pinned_like(self, b, name, t):

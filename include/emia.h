@@ -368,8 +368,7 @@ int emia_image_gray_hist(const uint8_t* image, int H, int W, int channels, uint6
  * emia_gather_plan / emia_gather_crops / emia_gather_b32 : dst instance j = src instance idx[j] (idx NULL: identity); crop sizes
  *   for the caller's scan, then crop words + bbox + area; 32-bit payloads (scores, classes).
  * emia_capacity_guard     : if *total > capacity (or *abort_flag already set): *abort_flag = 1 and the ch / cw of poison_meta[0..n)
- *   are zeroed, so that no later kernel reads or writes crops of that set; emia_capacity_guard_ranges: the same test for
- *   every range offsets[bounds[b+1]] - offsets[bounds[b]] (flag only). */
+ *   are zeroed, so that no later kernel reads or writes crops of that set. */
 int emia_group_filter_heads(const int32_t* cap_off, int32_t G, const int32_t* in_len, const int32_t* in_idx,
                             const emia_inst_meta* meta, const int32_t* classes, const float* scores, int32_t target_class,
                             float min_score, int32_t zero_score_empties, int32_t* out_len, int32_t* out_idx, void* stream);
@@ -389,8 +388,6 @@ int emia_gather_crops(const uint32_t* src_crops, const int64_t* src_crop_off, co
 int emia_gather_b32(const void* src, const int32_t* idx, int64_t k, void* dst, void* stream);
 int emia_capacity_guard(const int64_t* total, int64_t capacity, int32_t* abort_flag, emia_inst_meta* poison_meta,
                         int64_t poison_n, void* stream);
-int emia_capacity_guard_ranges(const int64_t* offsets, const int64_t* bounds, int32_t B, int64_t capacity, int32_t* abort_flag,
-                               void* stream);
 
 /* ---- row f3: scale-bar line detection for a batch of micrographs (csrc/emia_scalebar_kernels.cuh, core/emia_scalebar.cuh) -------
  * Replaces the OpenCV calls of detect_scale_bar (src/utils/scalebar_ocr.py:140 cv2.cvtColor(BGR2GRAY), :200 cv2.Canny(gray, 50, 150,
