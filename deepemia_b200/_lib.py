@@ -81,6 +81,11 @@ _SIGNATURES = {
     "emia_rle_decode_plan": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
                                      c_void_p, c_void_p]),
     "emia_rle_decode": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "emia_csv_rle_count": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p]),
+    "emia_csv_rle_write": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
+    "emia_csv_measure_count": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
+    "emia_csv_measure_write": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p,
+                                       c_void_p]),
     "emia_moments01": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "emia_moments": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "emia_color_sums": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int, c_int, c_void_p, c_void_p]),

@@ -18,6 +18,7 @@
 #include "core/emia_nms.cuh"
 #include "core/emia_moments.cuh"
 #include "core/emia_rle.cuh"
+#include "core/emia_text.cuh"
 
 static thread_local char g_err[512] = "";
 static int emia_fail(int code, const char* fmt, const char* detail) {
@@ -825,5 +826,6 @@ extern "C" int emia_paste_threshold_bitpack(const float* probs, const float* box
 #include "emia_morph_kernels.cuh"
 #include "emia_tile_kernels.cuh"
 #include "emia_rle_kernels.cuh"
+#include "emia_text_kernels.cuh"
 #include "emia_flow_kernels.cuh"
 #include "emia_scalebar_kernels.cuh"

@@ -4,6 +4,8 @@ Every computation on the path is a kernel of libemia.so called through the C ABI
 PyTorch provides device memory (torch.empty / zeros), streams, events and CUDA graphs, memcpy-type plumbing (copy_, clone, cat of
 already-computed arrays, the identity index lists of a layout) and — in bench.py / distributed.py — torch.distributed.
 """
+import csv
+import io
 import math
 from dataclasses import dataclass, field
 from typing import Optional
@@ -1263,6 +1265,102 @@ def rle_decode(run_off, runs, H, W):
         k = int(bad[0])
         raise _lib.EmiaError(f"rle_decode: instance {k}: {RLE_STATUS[int(status[k])]}")
     return iset
+
+
+def csv_field(value):
+    """The text csv.writer writes for `value` as one field of a row (QUOTE_MINIMAL: quoted when it holds a comma, a quote or a
+    line break, inner quotes doubled; None is empty; a float is its repr)."""
+    buf = io.StringIO()
+    csv.writer(buf).writerow([value, ""])
+    return buf.getvalue()[:-3]                     # the row ends in ",\r\n"
+
+
+def _text_to_host(text, nbytes):
+    """One D2H copy of text[:nbytes] into pinned memory -> bytes."""
+    if nbytes == 0:
+        return b""
+    host = torch.empty(nbytes, dtype=torch.uint8, pin_memory=True)
+    host.copy_(text[:nbytes], non_blocking=True)
+    torch.cuda.current_stream().synchronize()
+    return host.numpy().tobytes()
+
+
+def _strings_to_device(strings, dev):
+    """(UTF-8 bytes, int64 offsets [k + 1]) of k strings, on the device."""
+    raw = [s.encode("utf-8") for s in strings]
+    off = np.concatenate([[0], np.cumsum([len(b) for b in raw])]).astype(np.int64)
+    data = torch.frombuffer(bytearray(b"".join(raw) or b"\0"), dtype=torch.uint8).to(dev)
+    return data, torch.as_tensor(off, device=dev)
+
+
+def rle_csv_text(run_off, runs, image_id):
+    """The lines of R50_flip_results.csv for the instances of (run_off, runs) (rle_encode's output) of the image `image_id`: byte for
+    byte what csv.writer writes for the rows (image_id, " ".join of the instance's runs), UTF-8, "\\r\\n" line ends; an empty mask
+    gives `<ImageId>,`.  Formatted on the device; one host synchronisation to size the text and one D2H copy of it."""
+    lib = _lib.load()
+    dev = run_off.device
+    assert run_off.dtype == torch.int64 and runs.dtype == torch.int64 and run_off.is_contiguous() and runs.is_contiguous()
+    n = int(run_off.numel()) - 1
+    if n <= 0:
+        return b""
+    prefix = (csv_field(image_id) + ",").encode("utf-8")
+    pre = torch.frombuffer(bytearray(prefix), dtype=torch.uint8).to(dev)
+    line_off = torch.empty(n + 1, dtype=torch.int64, device=dev)
+    st = _stream()
+    rp = _ptr(runs) if runs.numel() else _ptr(run_off)      # no runs at all: never read, but the ABI wants a pointer
+    with _stage("csv_rle_count"):
+        _lib.check(lib.emia_csv_rle_count(rp, _ptr(run_off), n, len(prefix), _ptr(line_off), st), "emia_csv_rle_count")
+    with _stage("csv_rle_scan"):
+        exclusive_scan_(line_off)
+    nbytes = buffer_len(line_off[n:], n)
+    text = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=dev)
+    with _stage("csv_rle_write"):
+        _lib.check(lib.emia_csv_rle_write(rp, _ptr(run_off), n, _ptr(pre), len(prefix), _ptr(line_off), _ptr(text), st),
+                   "emia_csv_rle_write")
+    LAUNCHES["count"] += 2
+    with _stage("csv_rle_d2h"):
+        return _text_to_host(text, nbytes)
+
+
+def measurements_csv_text(iset, file_name, psum, class_idx, class_fields, contrast=None):
+    """The rows of measurements_results.csv for the measured records of `iset` (after measure()), in record order: byte for byte
+    what csv.writer writes for the rows of inference.measure_masks, UTF-8, "\\r\\n" line ends.  Instance i gets Instance_ID
+    `<file_name>_<i + 1>` and the (Class, Class_Name) values class_fields[class_idx[i]]; psum is the Detected scale bar value;
+    contrast: float64 [n, 3] d10 / d50 / d90 per instance (NaN: None), or None for empty contrast fields.  String values are
+    rendered once on the host (csv_field), numbers on the device; one host synchronisation to size the text, one D2H copy."""
+    lib = _lib.load()
+    dev = iset.device
+    assert iset.records is not None, "run measure() first"
+    R, n = int(iset.n_records), iset.n
+    class_idx = np.asarray(class_idx, np.int64).reshape(-1)
+    if len(class_idx) != n or (n and (class_idx.min() < 0 or class_idx.max() >= len(class_fields))):
+        raise ValueError(f"measurements_csv_text: class_idx needs {n} indices into the {len(class_fields)} class_fields")
+    if R == 0:
+        return b""
+    ident = csv_field(f"{file_name}_1")                     # the digits never change the quoting of the whole field
+    pre, suf = (ident[:-2], '"') if ident.endswith('"') else (ident[:-1], "")
+    strs = [pre, suf, csv_field(psum) + "," + csv_field(file_name)]
+    strs += [csv_field(c) + "," + csv_field(name) for c, name in class_fields]
+    sdata, soff = _strings_to_device(strs, dev)
+    cidx = torch.as_tensor(class_idx.astype(np.int32), device=dev)
+    con = None
+    if contrast is not None:
+        con = torch.as_tensor(np.asarray(contrast, np.float64).reshape(n, 3), device=dev).contiguous()
+    records, rec_inst = iset.records.contiguous(), iset.rec_inst.contiguous()
+    row_off = torch.empty(R + 1, dtype=torch.int64, device=dev)
+    st = _stream()
+    args = (_ptr(records), _ptr(rec_inst), R, _ptr(cidx), _ptr(con), _ptr(sdata), _ptr(soff), len(strs))
+    with _stage("csv_measure_count"):
+        _lib.check(lib.emia_csv_measure_count(*args, _ptr(row_off), st), "emia_csv_measure_count")
+    with _stage("csv_measure_scan"):
+        exclusive_scan_(row_off)
+    nbytes = buffer_len(row_off[R:], R)
+    text = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=dev)
+    with _stage("csv_measure_write"):
+        _lib.check(lib.emia_csv_measure_write(*args, _ptr(row_off), _ptr(text), st), "emia_csv_measure_write")
+    LAUNCHES["count"] += 2
+    with _stage("csv_measure_d2h"):
+        return _text_to_host(text, nbytes)
 
 
 def gray_hist(iset, image):

@@ -530,6 +530,36 @@ def measure_masks(masks, classes, image_shape, um_pix, test_img, psum, class_nam
     return rows
 
 
+def _measure_text(iset, classes, image_shape, um_pix, test_img, psum, class_names=None, original_image=None):
+    """measure_masks' rows as the text csv.writer writes for them, formatted on the device (engine.measurements_csv_text)."""
+    if iset.n == 0:
+        return b""
+    engine.measure(iset, um_pix=um_pix, min_area=engine.default_min_area(image_shape[0], image_shape[1]))
+    fields, class_idx = _class_table(classes, class_names)
+    return engine.measurements_csv_text(iset, test_img, psum, class_idx, fields, _contrast(iset, original_image))
+
+
+def _class_table(classes, class_names):
+    """(Class, Class_Name) pairs of the distinct classes as measure_masks names them, and each instance's index among them."""
+    fields, index, class_idx = [], {}, []
+    for cls in classes:
+        cls = int(cls)
+        if cls not in index:
+            index[cls] = len(fields)
+            fields.append((cls, class_names[cls] if class_names is not None and cls < len(class_names) else f"class_{cls}"))
+        class_idx.append(index[cls])
+    return fields, class_idx
+
+
+def _contrast(iset, original_image):
+    """float64 [n, 3] contrast d10 / d50 / d90 per instance (NaN where measure_masks writes None), or None when not measured."""
+    if not (measure_contrast_distribution and original_image is not None):
+        return None
+    from ..utils.contrast import percentiles_from_counts
+    hist = engine.gray_hist(iset, original_image).cpu().numpy()
+    return np.array([[np.nan if v is None else v for v in percentiles_from_counts(h)] for h in hist], np.float64).reshape(-1, 3)
+
+
 def _infer_image_dev(predictors, image, num_classes, small_classes, class_specific_settings=None, confidence_mode='manual',
                      confidence_fn=None, tile_size=512, overlap_ratio=0.1, upscale_factor=2.0, edge_filter_enabled=True,
                      ensemble_enabled=True, ensemble_small_only=True, classes_to_infer=None, spatial_rules=None, dataset_name=None):
@@ -675,11 +705,12 @@ def _scale_bars(images, dataset_name, dataset_config, output_dir, scale_bar_fn=N
     return each()
 
 
-def _write_measurements(output_dir, rows):
-    with open(os.path.join(output_dir, "measurements_results.csv"), "w", newline="") as f:
-        w = csv.writer(f)
-        w.writerow(CSV_HEADER)
-        w.writerows(rows)
+def _write_csv(path, header, texts):
+    """A result file: csv.writer's header line, then the device-formatted rows."""
+    with open(path, "wb") as f:
+        f.write((",".join(engine.csv_field(h) for h in header) + "\r\n").encode("utf-8"))
+        for t in texts:
+            f.write(t)
 
 
 def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw_id=False, dataset_format="json", draw_scalebar=False,
@@ -724,26 +755,20 @@ def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw
     small_classes = set(small_classes)
     os.makedirs(output_dir, exist_ok=True)
     bars = _scale_bars(images, dataset_name, dataset_config, output_dir, scale_bar_fn, draw_scalebar)
-    img_ids, encoded, meas_rows = [], [], []
+    rle_text, meas_text = [], []
     for (name, image), (psum, um_pix) in zip(images, bars):
         d = _infer_image_dev(predictors, image, num_classes, small_classes, dataset_name=dataset_name, **kw)
         if len(d) == 0:
             continue
         run_off, runs = engine.rle_encode(d.iset)                       # K6 over the final set, once
-        ro, rn = run_off.cpu().numpy(), runs.cpu().numpy()
-        stem = _stem(name)
-        for i in range(len(d)):
-            img_ids.append(stem)
-            encoded.append(" ".join(str(int(v)) for v in rn[ro[i]:ro[i + 1]].reshape(-1)))
-        meas_rows += measure_masks(d.iset, d.classes, image.shape, um_pix, name, psum, class_names=thing_classes, original_image=image)
+        rle_text.append(engine.rle_csv_text(run_off, runs, _stem(name)))
+        meas_text.append(_measure_text(d.iset, d.classes, image.shape, um_pix, name, psum, class_names=thing_classes,
+                                       original_image=image))
         if visualize:
             from ..utils.visualize import render_predictions
             cv2.imwrite(os.path.join(output_dir, f"{name}_predictions.png"), render_predictions(image, d.iset, d.classes, thing_classes))
-    with open(os.path.join(output_dir, "R50_flip_results.csv"), "w", newline="") as f:
-        w = csv.writer(f)
-        w.writerow(["ImageId", "EncodedPixels"])
-        w.writerows(zip(img_ids, encoded))
-    _write_measurements(output_dir, meas_rows)
+    _write_csv(os.path.join(output_dir, "R50_flip_results.csv"), ["ImageId", "EncodedPixels"], rle_text)
+    _write_csv(os.path.join(output_dir, "measurements_results.csv"), CSV_HEADER, meas_text)
     write_class_color_legend(output_dir, thing_classes)
     return None
 
@@ -816,14 +841,21 @@ def remeasure_results(dataset_name, results_dir, output_dir, *, images=None, sca
         raise ValueError(f"remeasure_results: {results_dir}/measurements_results.csv does not start with the measurements header")
     class_of = {r[0]: (r[1], r[2]) for r in old[1:]}
     os.makedirs(output_dir, exist_ok=True)
-    rows = []
+    texts = []
     for (name, image), (psum, um_pix) in zip(images, _scale_bars(images, dataset_name, _dataset_config(dataset_name), output_dir,
                                                                   scale_bar_fn)):
         iset = sets[name]
-        got = measure_masks(iset, [0] * iset.n, image.shape, um_pix, name, psum, original_image=image)
-        for r in got:
-            if r[0] not in class_of:
-                raise ValueError(f"remeasure_results: {r[0]} has a measured contour but no row in {results_dir}/measurements_results.csv")
-            r[1], r[2] = class_of[r[0]]
-        rows += got
-    _write_measurements(output_dir, rows)
+        if iset.n == 0:
+            continue
+        engine.measure(iset, um_pix=um_pix, min_area=engine.default_min_area(image.shape[0], image.shape[1]))
+        measured = np.unique(iset.rec_inst[iset.records[:, engine.REC_MEASURED] == 1.0].cpu().numpy())
+        if len(measured) == 0:
+            continue
+        index, class_idx = {}, [0] * iset.n         # (Class, Class_Name) of the old rows -> index; unmeasured instances: unused
+        for k in measured.tolist():
+            key = f"{name}_{k + 1}"
+            if key not in class_of:
+                raise ValueError(f"remeasure_results: {key} has a measured contour but no row in {results_dir}/measurements_results.csv")
+            class_idx[k] = index.setdefault(class_of[key], len(index))
+        texts.append(engine.measurements_csv_text(iset, name, psum, class_idx, list(index), _contrast(iset, image)))
+    _write_csv(os.path.join(output_dir, "measurements_results.csv"), CSV_HEADER, texts)

@@ -321,6 +321,26 @@ int emia_rle_decode_plan(const int64_t* runs, const int64_t* run_off, const int3
                          emia_inst_meta* meta, int64_t* crop_words, int32_t* bbox, int32_t* area, int32_t* status, void* stream);
 int emia_rle_decode(const int64_t* runs, const int64_t* run_off, const int32_t* rows, int64_t n, int H,
                     const emia_inst_meta* meta, const int64_t* crop_off, uint32_t* crops, void* stream);
+/* ---- Result CSV text (csrc/emia_text_kernels.cuh, core/emia_text.cuh): byte for byte what csv.writer writes ----------------
+ * Count -> exclusive scan of the n + 1 lengths (caller) -> write at the scanned offsets; the host renders every string field once
+ * (csv.writer's QUOTE_MINIMAL rule) and the kernels only copy its bytes.
+ * emia_csv_rle_count / _write: line i of R50_flip_results.csv for instance i of (run_off, runs) (emia_rle_encode's layout):
+ *   prefix (the ImageId field and its comma, prefix_len bytes), the runs as "s1 l1 s2 l2 ...", "\r\n".
+ * emia_csv_measure_count / _write: a measurements_results.csv row for every record r with records[r][15] (measured) == 1, none
+ *   (length 0) for the others.  Fields: strs[0] instance + 1 strs[1] (Instance_ID), strs[3 + class_idx[rec_inst[r]]] (Class,
+ *   Class_Name; class_idx[i] in [0, n_str - 3)), the 12 measurements (Python float / np.float64 repr, np.float32 str for C. Length,
+ *   C. Width, Aspect ratio, Ferret diameter and Roundness, int 0 for the axes and the eccentricity below 5 contour points), the
+ *   contrast d10 / d50 / d90 from contrast[inst][3] (NULL or NaN: empty), strs[2] (Detected scale bar,File name), "\r\n".
+ *   String k is strs[str_off[k], str_off[k + 1]). */
+int emia_csv_rle_count(const int64_t* runs, const int64_t* run_off, int64_t n, int64_t prefix_len, int64_t* line_len, void* stream);
+int emia_csv_rle_write(const int64_t* runs, const int64_t* run_off, int64_t n, const uint8_t* prefix, int64_t prefix_len,
+                       const int64_t* line_off, uint8_t* text, void* stream);
+int emia_csv_measure_count(const double* records, const int32_t* rec_inst, int64_t n_rec, const int32_t* class_idx,
+                           const double* contrast, const uint8_t* strs, const int64_t* str_off, int n_str, int64_t* row_len,
+                           void* stream);
+int emia_csv_measure_write(const double* records, const int32_t* rec_inst, int64_t n_rec, const int32_t* class_idx,
+                           const double* contrast, const uint8_t* strs, const int64_t* str_off, int n_str, const int64_t* row_off,
+                           uint8_t* text, void* stream);
 /* raw moments (m00, m10, m01) of every instance as exact integers: cv2.moments(mask) of src/functions/inference.py:1101-1104 */
 int emia_moments01(const uint32_t* crops, const emia_inst_meta* meta, const int64_t* crop_off, int64_t n, int64_t* out,
                    void* stream);
