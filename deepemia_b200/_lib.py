@@ -38,6 +38,8 @@ _SIGNATURES = {
     "emia_contour_measure_list": (c_int, [c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_double, c_double,
                                           c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "emia_list_measure_order": (c_int, [c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
+    "emia_contour_shape_list": (c_int, [c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_double, c_void_p,
+                                        c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "emia_contour_measure_stored": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_double, c_double,
                                             c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "emia_group_workspace_bytes": (c_size_t, [c_void_p, c_int]),
@@ -86,6 +88,10 @@ _SIGNATURES = {
     "emia_csv_measure_count": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
     "emia_csv_measure_write": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p,
                                        c_void_p]),
+    "emia_csv_measure_shape_count": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
+                                             c_void_p, c_void_p]),
+    "emia_csv_measure_shape_write": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
+                                             c_void_p, c_void_p, c_void_p]),
     "emia_moments01": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "emia_moments": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "emia_color_sums": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int, c_int, c_void_p, c_void_p]),

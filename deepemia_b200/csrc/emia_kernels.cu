@@ -19,6 +19,7 @@
 #include "core/emia_moments.cuh"
 #include "core/emia_rle.cuh"
 #include "core/emia_text.cuh"
+#include "core/emia_shape.cuh"
 
 static thread_local char g_err[512] = "";
 static int emia_fail(int code, const char* fmt, const char* detail) {

@@ -812,3 +812,56 @@ extern "C" int emia_contour_measure_list(int64_t n_items, const int32_t* item_in
                                                                                         EMIA_PRESORT_MAX, records, rec_inst, nullptr, scratch, abort_flag, order);
     return emia_check_launch("emia_contour_measure_list launch: %s");
 }
+
+// ---- shape descriptors of the records of emia_contour_measure_list: one THREAD per list slot, as k_contour_measure ------------
+// Contour k of a slot reuses the k-th sub-block of the slot's scratch (dead once the records are written); rows of records below
+// the area gate are NaN.
+__global__ void __launch_bounds__(EMIA_MEASURE_THREADS) k_contour_shape(int64_t n, const int32_t* __restrict__ item_inst,
+                                                                        const int64_t* __restrict__ rec_off,
+                                                                        const int64_t* __restrict__ inst_cont_off,
+                                                                        const int64_t* __restrict__ pt_off,
+                                                                        const int64_t* __restrict__ scratch_off, double um_pix,
+                                                                        const uint32_t* __restrict__ pts, const int32_t* __restrict__ cstart,
+                                                                        int cstart_stride, const double* __restrict__ records,
+                                                                        uint8_t* __restrict__ scratch, const int32_t* __restrict__ order,
+                                                                        double* __restrict__ shape) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n) return;
+    const int64_t it = order ? (int64_t)order[t] : t;
+    if (it < 0 || it >= n) return;
+    const int64_t i = item_inst ? (int64_t)item_inst[it] : it;
+    if (i < 0) return;
+    const int64_t c0 = rec_off[it];
+    const int nc = (int)(rec_off[it + 1] - c0);
+    if (nc == 0) return;
+    const int32_t* cs = cstart_stride > 0 ? cstart + (size_t)i * cstart_stride : cstart + inst_cont_off[i] + i;
+    const uint32_t* p = pts + pt_off[i];
+    uint8_t* sc0 = scratch + scratch_off[it];
+    size_t sub_end = 0;
+    for (int k = 0; k < nc; ++k) sub_end += emia_measure_sub_bytes(cs[k + 1] - cs[k]);
+    for (int j = 0; j < nc; ++j) {
+        const int k = nc - 1 - j;                     // records are in OpenCV order: reverse discovery order
+        const int len = cs[k + 1] - cs[k];
+        sub_end -= emia_measure_sub_bytes(len);
+        double* out = shape + (size_t)(c0 + j) * EMIA_S_COUNT;
+        if (records[(size_t)(c0 + j) * EMIA_REC_FIELDS + EMIA_REC_MEASURED] != 1.0) {
+            for (int f = 0; f < EMIA_S_COUNT; ++f) out[f] = __longlong_as_double(0x7ff8000000000000ll);
+        } else {
+            emia_shape_contour(p + cs[k], len, um_pix, sc0 + sub_end, out);
+        }
+    }
+}
+
+extern "C" int emia_contour_shape_list(int64_t n_items, const int32_t* item_inst, const int64_t* rec_off, const int64_t* scr_off,
+                                       const int64_t* inst_cont_off, const int64_t* pt_off, const int32_t* cstart, int32_t cstart_stride,
+                                       double um_pix, const uint32_t* pts, const double* records, uint8_t* scratch, const int32_t* order,
+                                       double* shape, void* stream) {
+    if (n_items < 0 || cstart_stride < 0) return emia_fail(EMIA_ERR_BAD_ARG, "emia_contour_shape_list: %s", "bad argument");
+    if (n_items == 0) return EMIA_OK;
+    if (!item_inst || !rec_off || !scr_off || !pt_off || !cstart || !pts || !records || !scratch || !shape ||
+        (cstart_stride == 0 && !inst_cont_off))
+        return emia_fail(EMIA_ERR_BAD_ARG, "emia_contour_shape_list: %s", "null pointer");
+    k_contour_shape<<<EMIA_MEASURE_GRID(n_items), EMIA_MEASURE_THREADS, 0, (cudaStream_t)stream>>>(
+        n_items, item_inst, rec_off, inst_cont_off, pt_off, scr_off, um_pix, pts, cstart, cstart_stride, records, scratch, order, shape);
+    return emia_check_launch("emia_contour_shape_list launch: %s");
+}

@@ -81,8 +81,13 @@ extern "C" int emia_csv_rle_write(const int64_t* runs, const int64_t* run_off, i
 
 // ---- measurements_results.csv: one row per measured record ------------------------------------------------------------------
 // Lane f writes field f: 0 Instance_ID (strs[0] + instance + 1 + strs[1]), 1 Class,Class_Name (strs[3 + class_idx]), 2..13 the
-// measurements, 14..16 the contrast percentiles, 17 "Detected scale bar,File name" (strs[2]) and the line end.
-__device__ __forceinline__ int emia_csv_measure_field(int lane, const double* rec, const double* contrast, uint8_t* num) {
+// measurements, 14..16 the contrast percentiles, 17 "Detected scale bar,File name" (strs[2]) and the line end — or, with the shape
+// columns, a ',' and lanes 18..27 the ten shape values (repr of a Python float), the last one ending the row.
+#define EMIA_CSV_SHAPE_LANE0 (EMIA_CSV_SEP_LANES + 1)
+__device__ __forceinline__ int emia_csv_measure_field(int lane, const double* rec, const double* contrast, const double* shape,
+                                                      uint8_t* num) {
+    if (shape && lane >= EMIA_CSV_SHAPE_LANE0 && lane < EMIA_CSV_SHAPE_LANE0 + EMIA_S_COUNT)
+        return emia_format_f64(num, shape[lane - EMIA_CSV_SHAPE_LANE0]);
     if (lane >= 2 && lane < 14) {
         const int c = lane - 2;                     // REC_MAJOR .. REC_SPHER
         if (c <= 2 && rec[14] < 5.0) { num[0] = '0'; return 1; }            // no ellipse below 5 contour points: int 0
@@ -99,7 +104,8 @@ __device__ __forceinline__ int emia_csv_measure_field(int lane, const double* re
 template <bool kWrite>
 __global__ void __launch_bounds__(EMIA_CSV_THREADS) k_csv_measure(const double* __restrict__ records, const int32_t* __restrict__ rec_inst,
                                                                   int64_t n_rec, const int32_t* __restrict__ class_idx,
-                                                                  const double* __restrict__ contrast, const uint8_t* __restrict__ strs,
+                                                                  const double* __restrict__ contrast, const double* __restrict__ shape,
+                                                                  const uint8_t* __restrict__ strs,
                                                                   const int64_t* __restrict__ str_off, int64_t* __restrict__ row_len,
                                                                   const int64_t* __restrict__ row_off, uint8_t* __restrict__ text) {
     const unsigned FULL = 0xffffffffu;
@@ -113,14 +119,16 @@ __global__ void __launch_bounds__(EMIA_CSV_THREADS) k_csv_measure(const double* 
     }
     const int inst = rec_inst[r];
     uint8_t num[EMIA_TEXT_NUM_MAX];
-    int nlen = emia_csv_measure_field(lane, rec, contrast ? contrast + 3 * (int64_t)inst : nullptr, num);
+    int nlen = emia_csv_measure_field(lane, rec, contrast ? contrast + 3 * (int64_t)inst : nullptr,
+                                      shape ? shape + r * EMIA_S_COUNT : nullptr, num);
     int s0 = -1, s1 = -1;                           // strings before / after the number
     if (lane == 0) { s0 = 0; s1 = 1; nlen = emia_write_i64(num, (int64_t)inst + 1); }
     else if (lane == 1) s0 = 3 + class_idx[inst];
     else if (lane == EMIA_CSV_SEP_LANES) s0 = 2;
     const int64_t a0 = s0 >= 0 ? str_off[s0] : 0, l0 = s0 >= 0 ? str_off[s0 + 1] - a0 : 0;
     const int64_t a1 = s1 >= 0 ? str_off[s1] : 0, l1 = s1 >= 0 ? str_off[s1 + 1] - a1 : 0;
-    const int term = lane < EMIA_CSV_SEP_LANES ? 1 : lane == EMIA_CSV_SEP_LANES ? 2 : 0;
+    const int last = shape ? EMIA_CSV_SHAPE_LANE0 + EMIA_S_COUNT - 1 : EMIA_CSV_SEP_LANES;
+    const int term = lane < last ? 1 : lane == last ? 2 : 0;
     const int64_t len = l0 + nlen + l1 + term;
     int64_t inc = len;
     for (int d = 1; d < 32; d <<= 1) {
@@ -147,26 +155,46 @@ static int emia_csv_measure_args(const char* what, const double* records, const 
     return EMIA_OK;
 }
 
+// shape: NULL, or float64 [n_rec][EMIA_S_COUNT] (emia_contour_shape_list) for the ten shape columns after "File name"
+static int emia_csv_measure_launch(const char* what, bool write, const double* records, const int32_t* rec_inst, int64_t n_rec,
+                                   const int32_t* class_idx, const double* contrast, const double* shape, const uint8_t* strs,
+                                   const int64_t* str_off, int n_str, int64_t* row_len, const int64_t* row_off, uint8_t* text,
+                                   void* stream) {
+    if (int rc = emia_csv_measure_args(what, records, rec_inst, n_rec, class_idx, strs, str_off, n_str, write ? (const void*)text : row_len))
+        return rc;
+    if (n_rec == 0) return EMIA_OK;
+    if (write && !row_off) return emia_fail(EMIA_ERR_BAD_ARG, "%s: null pointer", what);
+    const unsigned grid = (unsigned)((n_rec * 32 + EMIA_CSV_THREADS - 1) / EMIA_CSV_THREADS);
+    if (write)
+        k_csv_measure<true><<<grid, EMIA_CSV_THREADS, 0, (cudaStream_t)stream>>>(records, rec_inst, n_rec, class_idx, contrast, shape, strs,
+                                                                                 str_off, nullptr, row_off, text);
+    else
+        k_csv_measure<false><<<grid, EMIA_CSV_THREADS, 0, (cudaStream_t)stream>>>(records, rec_inst, n_rec, class_idx, contrast, shape, strs,
+                                                                                  str_off, row_len, nullptr, nullptr);
+    return emia_check_launch(write ? "emia_csv_measure_write launch: %s" : "emia_csv_measure_count launch: %s");
+}
+
 extern "C" int emia_csv_measure_count(const double* records, const int32_t* rec_inst, int64_t n_rec, const int32_t* class_idx,
                                       const double* contrast, const uint8_t* strs, const int64_t* str_off, int n_str, int64_t* row_len,
                                       void* stream) {
-    if (int rc = emia_csv_measure_args("emia_csv_measure_count", records, rec_inst, n_rec, class_idx, strs, str_off, n_str, row_len))
-        return rc;
-    if (n_rec == 0) return EMIA_OK;
-    k_csv_measure<false><<<(unsigned)((n_rec * 32 + EMIA_CSV_THREADS - 1) / EMIA_CSV_THREADS), EMIA_CSV_THREADS, 0,
-                           (cudaStream_t)stream>>>(records, rec_inst, n_rec, class_idx, contrast, strs, str_off, row_len, nullptr,
-                                                   nullptr);
-    return emia_check_launch("emia_csv_measure_count launch: %s");
+    return emia_csv_measure_launch("emia_csv_measure_count", false, records, rec_inst, n_rec, class_idx, contrast, nullptr, strs,
+                                   str_off, n_str, row_len, nullptr, nullptr, stream);
 }
 extern "C" int emia_csv_measure_write(const double* records, const int32_t* rec_inst, int64_t n_rec, const int32_t* class_idx,
                                       const double* contrast, const uint8_t* strs, const int64_t* str_off, int n_str,
                                       const int64_t* row_off, uint8_t* text, void* stream) {
-    if (int rc = emia_csv_measure_args("emia_csv_measure_write", records, rec_inst, n_rec, class_idx, strs, str_off, n_str, text))
-        return rc;
-    if (n_rec == 0) return EMIA_OK;
-    if (!row_off) return emia_fail(EMIA_ERR_BAD_ARG, "emia_csv_measure_write: %s", "null pointer");
-    k_csv_measure<true><<<(unsigned)((n_rec * 32 + EMIA_CSV_THREADS - 1) / EMIA_CSV_THREADS), EMIA_CSV_THREADS, 0,
-                          (cudaStream_t)stream>>>(records, rec_inst, n_rec, class_idx, contrast, strs, str_off, nullptr, row_off,
-                                                  text);
-    return emia_check_launch("emia_csv_measure_write launch: %s");
+    return emia_csv_measure_launch("emia_csv_measure_write", true, records, rec_inst, n_rec, class_idx, contrast, nullptr, strs,
+                                   str_off, n_str, nullptr, row_off, text, stream);
+}
+extern "C" int emia_csv_measure_shape_count(const double* records, const int32_t* rec_inst, int64_t n_rec, const int32_t* class_idx,
+                                            const double* contrast, const double* shape, const uint8_t* strs, const int64_t* str_off,
+                                            int n_str, int64_t* row_len, void* stream) {
+    return emia_csv_measure_launch("emia_csv_measure_shape_count", false, records, rec_inst, n_rec, class_idx, contrast, shape, strs,
+                                   str_off, n_str, row_len, nullptr, nullptr, stream);
+}
+extern "C" int emia_csv_measure_shape_write(const double* records, const int32_t* rec_inst, int64_t n_rec, const int32_t* class_idx,
+                                            const double* contrast, const double* shape, const uint8_t* strs, const int64_t* str_off,
+                                            int n_str, const int64_t* row_off, uint8_t* text, void* stream) {
+    return emia_csv_measure_launch("emia_csv_measure_shape_write", true, records, rec_inst, n_rec, class_idx, contrast, shape, strs,
+                                   str_off, n_str, nullptr, row_off, text, stream);
 }

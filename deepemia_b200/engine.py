@@ -575,6 +575,24 @@ class Measurements:
                 for g in range(self.groups.G)]
 
 
+def _measure_order(iset, item_inst, rec_off, L):
+    """The K5 work order of a list of L slots, or None below MEASURE_ORDER_MIN_SLOTS."""
+    if not (MEASURE_ORDER and L >= MEASURE_ORDER_MIN_SLOTS):
+        return None
+    # work order: slots sorted by vertex count (a warp of the morphometry kernel is as slow as its longest contour).  Measured:
+    # 1 M slots -0.80 ms, 128 K slots -0.04 ms, 8 K - 44 K slots (the batched flows) +0.06 ... +0.17 ms (three more graph
+    # nodes and a scattered hull pass for a stage that is only 0.1 ms there) - hence the threshold
+    lib = _lib.load()
+    dev = iset.device
+    order = torch.empty(L, dtype=torch.int32, device=dev)
+    bins = torch.empty(128, dtype=torch.int32, device=dev)
+    with _stage("k5_order"):
+        _lib.check(lib.emia_list_measure_order(L, _ptr(item_inst), _ptr(rec_off), _ptr(iset.cont_off), _ptr(iset.cstart),
+                                               iset.cstart_stride, _ptr(order), _ptr(bins), _stream()), "emia_list_measure_order")
+    LAUNCHES["count"] += 2
+    return order
+
+
 def measure_list(iset, groups, um_pix=1.0, min_area=None, arena=None, tag="k5"):
     """K5b: morphometry of the members of `groups` only (what the reference's measurement loop sees).  Needs trace().
     Returns None when the single-pass trace overflowed (the caller re-traces with single_pass=False).
@@ -614,17 +632,7 @@ def measure_list(iset, groups, um_pix=1.0, min_area=None, arena=None, tag="k5"):
     rec_inst = torch.empty(max(n_rec, 1), dtype=torch.int32, device=dev)
     scratch = torch.empty(max(n_scr, 16), dtype=torch.uint8, device=dev)
     if L:
-        order = None
-        if MEASURE_ORDER and L >= MEASURE_ORDER_MIN_SLOTS:
-            # work order: slots sorted by vertex count (a warp of the morphometry kernel is as slow as its longest contour).  Measured:
-            # 1 M slots -0.80 ms, 128 K slots -0.04 ms, 8 K - 44 K slots (the batched flows) +0.06 ... +0.17 ms (three more graph
-            # nodes and a scattered hull pass for a stage that is only 0.1 ms there) - hence the threshold
-            order = torch.empty(L, dtype=torch.int32, device=dev)
-            bins = torch.empty(128, dtype=torch.int32, device=dev)
-            with _stage("k5_order"):
-                _lib.check(lib.emia_list_measure_order(L, _ptr(item_inst), _ptr(offs[0]), _ptr(iset.cont_off), _ptr(iset.cstart),
-                                                       iset.cstart_stride, _ptr(order), _ptr(bins), st), "emia_list_measure_order")
-            LAUNCHES["count"] += 2
+        order = _measure_order(iset, item_inst, offs[0], L)
         with _stage("k5_measure"):
             _lib.check(lib.emia_contour_measure_list(L, _ptr(item_inst), _ptr(offs[0]), _ptr(offs[1]), _ptr(iset.cont_off),
                                                      _ptr(iset.pt_off), _ptr(iset.cstart), iset.cstart_stride, float(um_pix),
@@ -637,6 +645,55 @@ def measure_list(iset, groups, um_pix=1.0, min_area=None, arena=None, tag="k5"):
                             totals=torch.stack([offs[0, L], offs[1, L]]))
     return Measurements(records=records[:n_rec], rec_inst=rec_inst[:n_rec], rec_off=offs[0], n_records=n_rec, groups=groups,
                         totals=(n_rec, n_scr))
+
+
+SHAPE_FIELDS = 10   # EMIA_S_COUNT: area, convex area, solidity, convex perimeter, convexity, max / min Feret, Feret angle, centroid x / y
+
+
+def shape_list(iset, meas, um_pix=1.0):
+    """Shape descriptors float64 [R, SHAPE_FIELDS] of the records of `meas`, an exact measure_list result on `iset` (row r belongs to
+    meas.records[r]; NaN rows for records below the area gate): area, convex hull area, solidity, convex hull perimeter, convexity,
+    max / min Feret diameter, max-Feret angle in degrees [0, 180) with y up (areas and lengths scaled by um_pix), and the centroid in
+    frame pixels (core/emia_shape.cuh, oracle/shape.py).  The hull scratch of measure_list is sized again (one host
+    synchronisation); the slots take the K5 work order from MEASURE_ORDER_MIN_SLOTS on."""
+    lib = _lib.load()
+    dev = iset.device
+    if meas.n_records is None:
+        raise ValueError("shape_list needs an exact measure_list result: call finalize() first")
+    R = int(meas.n_records)
+    shape = torch.empty((max(R, 1), SHAPE_FIELDS), dtype=torch.float64, device=dev)
+    groups = meas.groups
+    L = groups.total_cap
+    if R == 0 or L == 0:
+        return shape[:0]
+    st = _stream()
+    item_inst = torch.empty(L, dtype=torch.int32, device=dev)
+    offs = torch.zeros((2, L + 1), dtype=torch.int64, device=dev)
+    with _stage("shape_plan+scan"):
+        _lib.check(lib.emia_list_measure_plan(_ptr(groups.cap_off), groups.G, L, _ptr(groups.length), _ptr(groups.idx),
+                                              _ptr(iset.extra["n_contours"]), _ptr(iset.extra["scratch_bytes"]), _ptr(item_inst),
+                                              _ptr(offs[0]), _ptr(offs[1]), st), "emia_list_measure_plan")
+        exclusive_scan_(offs[1])
+    LAUNCHES["count"] += 1
+    scratch = torch.empty(max(buffer_len(offs[1, L:], L), 16), dtype=torch.uint8, device=dev)
+    order = _measure_order(iset, item_inst, meas.rec_off, L)
+    records = meas.records.contiguous()
+    with _stage("shape"):
+        _lib.check(lib.emia_contour_shape_list(L, _ptr(item_inst), _ptr(meas.rec_off), _ptr(offs[1]), _ptr(iset.cont_off), _ptr(iset.pt_off),
+                                               _ptr(iset.cstart), iset.cstart_stride, float(um_pix), _ptr(iset.pts), _ptr(records),
+                                               _ptr(scratch), _ptr(order) if order is not None else 0, _ptr(shape), st),
+                   "emia_contour_shape_list")
+    LAUNCHES["count"] += 1
+    return shape[:R]
+
+
+def shape_descriptors(iset):
+    """shape_list over every record of a set after measure(): float64 [n_records, SHAPE_FIELDS], row for row with iset.records, at
+    the um_pix of that measure() call."""
+    assert iset.records is not None, "run measure() first"
+    ident = groups_from_offsets([0, iset.n], iset.device)
+    meas = Measurements(records=iset.records, rec_inst=iset.rec_inst, rec_off=iset.cont_off, n_records=iset.n_records, groups=ident)
+    return shape_list(iset, meas, iset.extra["um_pix"])
 
 
 def measure(iset, um_pix=1.0, min_area=None, single_pass=True):
@@ -661,6 +718,27 @@ def measure(iset, um_pix=1.0, min_area=None, single_pass=True):
 def measure_contours(contours, um_pix=1.0, device=None):
     """Morphometry records [n,16] (float64, device) of n explicit contours (each an int array [K,2] or OpenCV's [K,1,2]):
     the kernel behind calculate_measurements (src/utils/measurements.py:114-233) for callers that hold contours."""
+    return _measure_contours(contours, um_pix, device)[0]
+
+
+def shape_contours(contours, um_pix=1.0, device=None):
+    """Shape descriptors [n, SHAPE_FIELDS] (float64, device; shape_list's columns) of n explicit contours, measured without an area
+    gate."""
+    lib = _lib.load()
+    records, n, d_cont, d_pt, d_cs, d_scr, d_pts, scratch = _measure_contours(contours, um_pix, device)
+    dev = records.device
+    shape = torch.empty((max(n, 1), SHAPE_FIELDS), dtype=torch.float64, device=dev)
+    item_inst = torch.arange(max(n, 1), dtype=torch.int32, device=dev)
+    _lib.check(lib.emia_contour_shape_list(n, _ptr(item_inst), _ptr(d_cont), _ptr(d_scr), _ptr(d_cont), _ptr(d_pt), _ptr(d_cs), 0,
+                                           float(um_pix), _ptr(d_pts), _ptr(records), _ptr(scratch), 0, _ptr(shape), _stream()),
+               "emia_contour_shape_list")
+    LAUNCHES["count"] += 1
+    return shape[:n]
+
+
+def _measure_contours(contours, um_pix, device):
+    """measure_contours: (records [n, 16], n, and the device list it measured: cont_off, pt_off, cstart, scratch offsets, points,
+    scratch)."""
     lib = _lib.load()
     dev = _need_cuda(device)
     n = len(contours)
@@ -687,7 +765,7 @@ def measure_contours(contours, um_pix=1.0, device=None):
                                                _ptr(d_pts), _ptr(records), _ptr(rec_inst), _ptr(perim0), _ptr(scratch), _stream()),
                "emia_contour_measure_stored")
     LAUNCHES["count"] += 2
-    return records[:n]
+    return records[:n], n, d_cont, d_pt, d_cs, d_scr, d_pts, scratch
 
 
 def contours_to_host(iset):
@@ -1322,12 +1400,14 @@ def rle_csv_text(run_off, runs, image_id):
         return _text_to_host(text, nbytes)
 
 
-def measurements_csv_text(iset, file_name, psum, class_idx, class_fields, contrast=None):
+def measurements_csv_text(iset, file_name, psum, class_idx, class_fields, contrast=None, shape=None):
     """The rows of measurements_results.csv for the measured records of `iset` (after measure()), in record order: byte for byte
     what csv.writer writes for the rows of inference.measure_masks, UTF-8, "\\r\\n" line ends.  Instance i gets Instance_ID
     `<file_name>_<i + 1>` and the (Class, Class_Name) values class_fields[class_idx[i]]; psum is the Detected scale bar value;
-    contrast: float64 [n, 3] d10 / d50 / d90 per instance (NaN: None), or None for empty contrast fields.  String values are
-    rendered once on the host (csv_field), numbers on the device; one host synchronisation to size the text, one D2H copy."""
+    contrast: float64 [n, 3] d10 / d50 / d90 per instance (NaN: None), or None for empty contrast fields; shape: None, or the
+    float64 [n_records, SHAPE_FIELDS] device tensor of shape_descriptors(iset), whose values follow "File name" as Python floats.
+    String values are rendered once on the host (csv_field), numbers on the device; one host synchronisation to size the text,
+    one D2H copy."""
     lib = _lib.load()
     dev = iset.device
     assert iset.records is not None, "run measure() first"
@@ -1346,18 +1426,23 @@ def measurements_csv_text(iset, file_name, psum, class_idx, class_fields, contra
     con = None
     if contrast is not None:
         con = torch.as_tensor(np.asarray(contrast, np.float64).reshape(n, 3), device=dev).contiguous()
+    if shape is not None:
+        if not (isinstance(shape, torch.Tensor) and shape.device == iset.records.device and shape.dtype == torch.float64 and
+                tuple(shape.shape) == (R, SHAPE_FIELDS)):
+            raise ValueError(f"measurements_csv_text: shape must be a float64 [{R}, {SHAPE_FIELDS}] tensor beside the records")
+        shape = shape.contiguous()
     records, rec_inst = iset.records.contiguous(), iset.rec_inst.contiguous()
     row_off = torch.empty(R + 1, dtype=torch.int64, device=dev)
     st = _stream()
-    args = (_ptr(records), _ptr(rec_inst), R, _ptr(cidx), _ptr(con), _ptr(sdata), _ptr(soff), len(strs))
+    args = (_ptr(records), _ptr(rec_inst), R, _ptr(cidx), _ptr(con), _ptr(shape), _ptr(sdata), _ptr(soff), len(strs))
     with _stage("csv_measure_count"):
-        _lib.check(lib.emia_csv_measure_count(*args, _ptr(row_off), st), "emia_csv_measure_count")
+        _lib.check(lib.emia_csv_measure_shape_count(*args, _ptr(row_off), st), "emia_csv_measure_shape_count")
     with _stage("csv_measure_scan"):
         exclusive_scan_(row_off)
     nbytes = buffer_len(row_off[R:], R)
     text = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=dev)
     with _stage("csv_measure_write"):
-        _lib.check(lib.emia_csv_measure_write(*args, _ptr(row_off), _ptr(text), st), "emia_csv_measure_write")
+        _lib.check(lib.emia_csv_measure_shape_write(*args, _ptr(row_off), _ptr(text), st), "emia_csv_measure_shape_write")
     LAUNCHES["count"] += 2
     with _stage("csv_measure_d2h"):
         return _text_to_host(text, nbytes)

@@ -25,7 +25,7 @@ from .. import engine
 from ..utils import _bridge
 from ..utils.mask_utils import rle_encoding  # noqa: F401  (re-exported like the reference's import)
 from ..utils import spatial_constraints as _sc
-from ..utils.measurements import record_to_dict, KEY_ORDER
+from ..utils.measurements import record_to_dict, KEY_ORDER, SHAPE_HEADER
 
 # ---- module-level settings (reference: config.yaml via inference.py:55-93) ---------------------------------------------------
 PARALLEL_MASK_PROCESSING = True            # l4_performance_optimizations.enable_parallel_mask_processing
@@ -504,14 +504,17 @@ def tile_based_inference_pipeline(predictor, image, target_class, small_classes,
 # =================================================================================================================
 # measurement loop + CSV (inference.py:987-1010, :1148-1253) and the per-image part of run_inference (:776-905)
 # =================================================================================================================
-def measure_masks(masks, classes, image_shape, um_pix, test_img, psum, class_names=None, original_image=None):
-    """Rows of measurements_results.csv for one image: one row per external contour whose contourArea reaches the gate (Q12)."""
+def measure_masks(masks, classes, image_shape, um_pix, test_img, psum, class_names=None, original_image=None, shape_columns=False):
+    """Rows of measurements_results.csv for one image: one row per external contour whose contourArea reaches the gate (Q12).
+    shape_columns: the row continues after "File name" with the ten SHAPE_HEADER values (engine.shape_descriptors) as Python
+    floats."""
     if (masks.n if isinstance(masks, engine.InstanceSet) else len(masks)) == 0:
         return []
     iset = masks if isinstance(masks, engine.InstanceSet) else _bridge.upload(masks)
     engine.measure(iset, um_pix=um_pix, min_area=engine.default_min_area(image_shape[0], image_shape[1]))
     rec = iset.records.cpu().numpy()
     cont_off = iset.cont_off.cpu().numpy()
+    shape = engine.shape_descriptors(iset).cpu().numpy() if shape_columns else None
     hist = None
     if measure_contrast_distribution and original_image is not None:
         from ..utils.contrast import percentiles_from_counts
@@ -526,17 +529,19 @@ def measure_masks(masks, classes, image_shape, um_pix, test_img, psum, class_nam
             m = record_to_dict(rec[j])
             if hist is not None:
                 m["contrast_d10"], m["contrast_d50"], m["contrast_d90"] = percentiles_from_counts(hist[k])
-            rows.append([f"{test_img}_{k + 1}", cls, name] + [m[key] for key in KEY_ORDER] + [psum, test_img])
+            rows.append([f"{test_img}_{k + 1}", cls, name] + [m[key] for key in KEY_ORDER] + [psum, test_img] +
+                        ([float(v) for v in shape[j]] if shape is not None else []))
     return rows
 
 
-def _measure_text(iset, classes, image_shape, um_pix, test_img, psum, class_names=None, original_image=None):
+def _measure_text(iset, classes, image_shape, um_pix, test_img, psum, class_names=None, original_image=None, shape_columns=False):
     """measure_masks' rows as the text csv.writer writes for them, formatted on the device (engine.measurements_csv_text)."""
     if iset.n == 0:
         return b""
     engine.measure(iset, um_pix=um_pix, min_area=engine.default_min_area(image_shape[0], image_shape[1]))
     fields, class_idx = _class_table(classes, class_names)
-    return engine.measurements_csv_text(iset, test_img, psum, class_idx, fields, _contrast(iset, original_image))
+    return engine.measurements_csv_text(iset, test_img, psum, class_idx, fields, _contrast(iset, original_image),
+                                        engine.shape_descriptors(iset) if shape_columns else None)
 
 
 def _class_table(classes, class_names):
@@ -714,7 +719,8 @@ def _write_csv(path, header, texts):
 
 
 def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw_id=False, dataset_format="json", draw_scalebar=False,
-                  *, images=None, predictors=None, thing_classes=None, small_classes=None, scale_bar_fn=None, **infer_kwargs):
+                  *, images=None, predictors=None, thing_classes=None, small_classes=None, scale_bar_fn=None, shape_columns=False,
+                  **infer_kwargs):
     """run_inference (src/functions/inference.py:499-1351), same signature and call shape as main.py:480-488:
 
         run_inference(dataset_name, output_dir, visualize=..., threshold=..., draw_id=..., dataset_format=..., draw_scalebar=...)
@@ -725,7 +731,9 @@ def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw
     per-class tile pipeline -> cross-class de-dup -> spatial constraints (:776-905), all on the device; the RLE rows of
     R50_flip_results.csv and the rows of measurements_results.csv are produced from the SAME device-resident instance set (one
     K6 and one K5 pass per image, no mask round trip).  Writes R50_flip_results.csv, measurements_results.csv,
-    class_color_legend.txt and, with visualize, <name>_predictions.png (overlay kernel + labels)."""
+    class_color_legend.txt and, with visualize, <name>_predictions.png (overlay kernel + labels).  shape_columns: each row of
+    measurements_results.csv continues after "File name" with the ten SHAPE_HEADER columns (area, convex hull, Feret diameters,
+    centroid: engine.shape_descriptors)."""
     images = _resolve_images(dataset_name, images)
     if thing_classes is None and _PROVIDERS["thing_classes"]:
         thing_classes = _PROVIDERS["thing_classes"](dataset_name)
@@ -756,6 +764,7 @@ def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw
     os.makedirs(output_dir, exist_ok=True)
     bars = _scale_bars(images, dataset_name, dataset_config, output_dir, scale_bar_fn, draw_scalebar)
     rle_text, meas_text = [], []
+    shape_kw = {"shape_columns": True} if shape_columns else {}      # without the option, _measure_text is called as it always was
     for (name, image), (psum, um_pix) in zip(images, bars):
         d = _infer_image_dev(predictors, image, num_classes, small_classes, dataset_name=dataset_name, **kw)
         if len(d) == 0:
@@ -763,12 +772,12 @@ def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw
         run_off, runs = engine.rle_encode(d.iset)                       # K6 over the final set, once
         rle_text.append(engine.rle_csv_text(run_off, runs, _stem(name)))
         meas_text.append(_measure_text(d.iset, d.classes, image.shape, um_pix, name, psum, class_names=thing_classes,
-                                       original_image=image))
+                                       original_image=image, **shape_kw))
         if visualize:
             from ..utils.visualize import render_predictions
             cv2.imwrite(os.path.join(output_dir, f"{name}_predictions.png"), render_predictions(image, d.iset, d.classes, thing_classes))
     _write_csv(os.path.join(output_dir, "R50_flip_results.csv"), ["ImageId", "EncodedPixels"], rle_text)
-    _write_csv(os.path.join(output_dir, "measurements_results.csv"), CSV_HEADER, meas_text)
+    _write_csv(os.path.join(output_dir, "measurements_results.csv"), CSV_HEADER + (SHAPE_HEADER if shape_columns else []), meas_text)
     write_class_color_legend(output_dir, thing_classes)
     return None
 
@@ -820,13 +829,13 @@ def load_rle_results(path, images):
     return out
 
 
-def remeasure_results(dataset_name, results_dir, output_dir, *, images=None, scale_bar_fn=None):
+def remeasure_results(dataset_name, results_dir, output_dir, *, images=None, scale_bar_fn=None, shape_columns=False):
     """Measure the masks a run_inference call saved in results_dir again, without the models: writes output_dir/
     measurements_results.csv as run_inference would with the scale bars (and settings such as measure_contrast_distribution) of
     now.  Images and scale bars resolve exactly as in run_inference (images= / the images provider; scale_bar_fn / the scale_bar
     provider / the package's detector).  Class and Class_Name of an instance are those of its rows in results_dir's
     measurements_results.csv; an instance without rows there has no contour above the area gate (which depends only on the frame
-    size) and gets none here either."""
+    size) and gets none here either.  shape_columns: as in run_inference, whether or not the old file has them."""
     if os.path.realpath(output_dir) == os.path.realpath(results_dir):
         raise ValueError("remeasure_results: output_dir must differ from results_dir (its measurements_results.csv is an input)")
     images = _resolve_images(dataset_name, images)
@@ -837,7 +846,7 @@ def remeasure_results(dataset_name, results_dir, output_dir, *, images=None, sca
     sets = load_rle_results(os.path.join(results_dir, "R50_flip_results.csv"), images)
     with open(os.path.join(results_dir, "measurements_results.csv"), newline="") as f:
         old = list(csv.reader(f))
-    if not old or old[0] != CSV_HEADER:
+    if not old or old[0] not in (CSV_HEADER, CSV_HEADER + SHAPE_HEADER):
         raise ValueError(f"remeasure_results: {results_dir}/measurements_results.csv does not start with the measurements header")
     class_of = {r[0]: (r[1], r[2]) for r in old[1:]}
     os.makedirs(output_dir, exist_ok=True)
@@ -857,5 +866,6 @@ def remeasure_results(dataset_name, results_dir, output_dir, *, images=None, sca
             if key not in class_of:
                 raise ValueError(f"remeasure_results: {key} has a measured contour but no row in {results_dir}/measurements_results.csv")
             class_idx[k] = index.setdefault(class_of[key], len(index))
-        texts.append(engine.measurements_csv_text(iset, name, psum, class_idx, list(index), _contrast(iset, image)))
-    _write_csv(os.path.join(output_dir, "measurements_results.csv"), CSV_HEADER, texts)
+        texts.append(engine.measurements_csv_text(iset, name, psum, class_idx, list(index), _contrast(iset, image),
+                                                  engine.shape_descriptors(iset) if shape_columns else None))
+    _write_csv(os.path.join(output_dir, "measurements_results.csv"), CSV_HEADER + (SHAPE_HEADER if shape_columns else []), texts)

@@ -12,6 +12,9 @@ _FIELDS = {"major_axis_length": engine.REC_MAJOR, "minor_axis_length": engine.RE
            "Length": engine.REC_LENGTH, "Width": engine.REC_WIDTH, "CircularED": engine.REC_CED, "Aspect_Ratio": engine.REC_ASPECT,
            "Circularity": engine.REC_CIRC, "Chords": engine.REC_CHORDS, "Feret_diam": engine.REC_FERET, "Roundness": engine.REC_ROUND,
            "Sphericity": engine.REC_SPHER}
+# the opt-in columns after "File name" (no reference counterpart): engine.shape_descriptors / core/emia_shape.cuh
+SHAPE_HEADER = ["Area", "Convex area", "Solidity", "Convex perimeter", "Convexity", "Max Feret diameter", "Min Feret diameter",
+                "Feret angle", "Centroid X", "Centroid Y"]
 KEY_ORDER = ["major_axis_length", "minor_axis_length", "eccentricity", "Length", "Width", "CircularED", "Aspect_Ratio", "Circularity",
              "Chords", "Feret_diam", "Roundness", "Sphericity", "contrast_d10", "contrast_d50", "contrast_d90"]
 
@@ -45,6 +48,14 @@ def calculate_measurements(c, single_im_mask, um_pix=1.0, pixelsPerMetric=1.0, o
         from .contrast import contrast_percentiles
         out["contrast_d10"], out["contrast_d50"], out["contrast_d90"] = contrast_percentiles(original_image, single_im_mask)
     return out
+
+
+def shape_descriptors(c, um_pix=1.0):
+    """The SHAPE_HEADER values of one OpenCV contour `c` ([K,1,2] or [K,2] int), as {column: float}: area, convex hull area and
+    perimeter, solidity, convexity, max / min Feret diameter and the max-Feret angle (degrees in [0, 180), y up), centroid in pixels.
+    Computed in libemia.so without an area gate; lengths and areas are scaled by um_pix."""
+    vals = engine.shape_contours([np.asarray(c).reshape(-1, 2)], um_pix=um_pix)[0].cpu().numpy()
+    return {k: float(v) for k, v in zip(SHAPE_HEADER, vals)}
 
 
 # ---- colour -> wavelength helpers (src/utils/measurements.py:32-111; no caller in the reference, kept for API completeness) --------

@@ -156,7 +156,10 @@ int emia_contour_measure_stored(const emia_inst_meta* meta, int64_t n, const int
  *   entries from emia_list_measure_order; NULL = list order): the order in which the slots are WORKED ON — the results do not depend
  *   on it.
  * emia_list_measure_order: order[] = the slots sorted by vertex count, longest first, dead slots last (a warp is as slow as its
- *   longest contour); bins = 128 int32 of workspace (cleared inside). */
+ *   longest contour); bins = 128 int32 of workspace (cleared inside).
+ * emia_contour_shape_list: after emia_contour_measure_list on the same list (same arguments, its records and its scratch, whose
+ *   contents it overwrites), shape[r][10] = the shape descriptors of record r (core/emia_shape.cuh: area, convex area, solidity,
+ *   convex perimeter, convexity, max / min Feret diameter, Feret angle, centroid x / y); NaN for records below the area gate. */
 int emia_list_measure_plan(const int32_t* cap_off, int32_t G, int32_t total_cap, const int32_t* in_len,
                            const int32_t* in_idx, const int64_t* n_contours, const int64_t* scratch_bytes,
                            int32_t* item_inst, int64_t* rec_cnt, int64_t* scr_cnt, void* stream);
@@ -166,6 +169,10 @@ int emia_contour_measure_list(int64_t n_items, const int32_t* item_inst, const i
                               int32_t* rec_inst, uint8_t* scratch, const int32_t* abort_flag, const int32_t* order, void* stream);
 int emia_list_measure_order(int64_t n_items, const int32_t* item_inst, const int64_t* rec_off, const int64_t* inst_cont_off,
                             const int32_t* cstart, int32_t cstart_stride, int32_t* order, int32_t* bins, void* stream);
+int emia_contour_shape_list(int64_t n_items, const int32_t* item_inst, const int64_t* rec_off, const int64_t* scr_off,
+                            const int64_t* inst_cont_off, const int64_t* pt_off, const int32_t* cstart, int32_t cstart_stride,
+                            double um_pix, const uint32_t* pts, const double* records, uint8_t* scratch, const int32_t* order,
+                            double* shape, void* stream);
 
 /* ---- K4: mask-IoU de-duplication and spatial constraints ----------------------------------------------------
  * All operate on G groups at once; see "Instance layout".  total_cap = cap_off[G] (the host knows it).
@@ -331,7 +338,10 @@ int emia_rle_decode(const int64_t* runs, const int64_t* run_off, const int32_t* 
  *   Class_Name; class_idx[i] in [0, n_str - 3)), the 12 measurements (Python float / np.float64 repr, np.float32 str for C. Length,
  *   C. Width, Aspect ratio, Ferret diameter and Roundness, int 0 for the axes and the eccentricity below 5 contour points), the
  *   contrast d10 / d50 / d90 from contrast[inst][3] (NULL or NaN: empty), strs[2] (Detected scale bar,File name), "\r\n".
- *   String k is strs[str_off[k], str_off[k + 1]). */
+ *   String k is strs[str_off[k], str_off[k + 1]).
+ * emia_csv_measure_shape_count / _write: the same rows with shape = NULL; otherwise strs[2] ends with ',' and the ten shape values
+ *   shape[r][10] (emia_contour_shape_list) follow as Python float repr, the last one ending the row.  The two entry points above
+ *   keep their signature for existing callers. */
 int emia_csv_rle_count(const int64_t* runs, const int64_t* run_off, int64_t n, int64_t prefix_len, int64_t* line_len, void* stream);
 int emia_csv_rle_write(const int64_t* runs, const int64_t* run_off, int64_t n, const uint8_t* prefix, int64_t prefix_len,
                        const int64_t* line_off, uint8_t* text, void* stream);
@@ -341,6 +351,12 @@ int emia_csv_measure_count(const double* records, const int32_t* rec_inst, int64
 int emia_csv_measure_write(const double* records, const int32_t* rec_inst, int64_t n_rec, const int32_t* class_idx,
                            const double* contrast, const uint8_t* strs, const int64_t* str_off, int n_str, const int64_t* row_off,
                            uint8_t* text, void* stream);
+int emia_csv_measure_shape_count(const double* records, const int32_t* rec_inst, int64_t n_rec, const int32_t* class_idx,
+                                 const double* contrast, const double* shape, const uint8_t* strs, const int64_t* str_off, int n_str,
+                                 int64_t* row_len, void* stream);
+int emia_csv_measure_shape_write(const double* records, const int32_t* rec_inst, int64_t n_rec, const int32_t* class_idx,
+                                 const double* contrast, const double* shape, const uint8_t* strs, const int64_t* str_off, int n_str,
+                                 const int64_t* row_off, uint8_t* text, void* stream);
 /* raw moments (m00, m10, m01) of every instance as exact integers: cv2.moments(mask) of src/functions/inference.py:1101-1104 */
 int emia_moments01(const uint32_t* crops, const emia_inst_meta* meta, const int64_t* crop_off, int64_t n, int64_t* out,
                    void* stream);
