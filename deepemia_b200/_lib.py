@@ -92,6 +92,13 @@ _SIGNATURES = {
                                              c_void_p, c_void_p]),
     "emia_csv_measure_shape_write": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
                                              c_void_p, c_void_p, c_void_p]),
+    "emia_neighbour_plan": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_int,
+                                    c_void_p, c_void_p, c_void_p, c_void_p]),
+    "emia_neighbour_search": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_int,
+                                      c_void_p, c_void_p, c_double, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "emia_csv_neighbour_count": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
+    "emia_csv_neighbour_write": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p,
+                                         c_void_p]),
     "emia_moments01": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "emia_moments": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "emia_color_sums": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int, c_int, c_void_p, c_void_p]),

@@ -20,6 +20,7 @@
 #include "core/emia_rle.cuh"
 #include "core/emia_text.cuh"
 #include "core/emia_shape.cuh"
+#include "core/emia_neighbour.cuh"
 
 static thread_local char g_err[512] = "";
 static int emia_fail(int code, const char* fmt, const char* detail) {
@@ -828,5 +829,6 @@ extern "C" int emia_paste_threshold_bitpack(const float* probs, const float* box
 #include "emia_tile_kernels.cuh"
 #include "emia_rle_kernels.cuh"
 #include "emia_text_kernels.cuh"
+#include "emia_neighbour_kernels.cuh"
 #include "emia_flow_kernels.cuh"
 #include "emia_scalebar_kernels.cuh"

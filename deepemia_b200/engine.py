@@ -1371,6 +1371,15 @@ def _strings_to_device(strings, dev):
     return data, torch.as_tensor(off, device=dev)
 
 
+def _row_strings(file_name, psum, class_fields):
+    """The string fields of a result row, rendered by csv_field: the Instance_ID text before and after the number, "Detected scale
+    bar,File name", and "Class,Class_Name" per class-table entry."""
+    ident = csv_field(f"{file_name}_1")                     # the digits never change the quoting of the whole field
+    pre, suf = (ident[:-2], '"') if ident.endswith('"') else (ident[:-1], "")
+    strs = [pre, suf, csv_field(psum) + "," + csv_field(file_name)]
+    return strs + [csv_field(c) + "," + csv_field(name) for c, name in class_fields]
+
+
 def rle_csv_text(run_off, runs, image_id):
     """The lines of R50_flip_results.csv for the instances of (run_off, runs) (rle_encode's output) of the image `image_id`: byte for
     byte what csv.writer writes for the rows (image_id, " ".join of the instance's runs), UTF-8, "\\r\\n" line ends; an empty mask
@@ -1417,10 +1426,7 @@ def measurements_csv_text(iset, file_name, psum, class_idx, class_fields, contra
         raise ValueError(f"measurements_csv_text: class_idx needs {n} indices into the {len(class_fields)} class_fields")
     if R == 0:
         return b""
-    ident = csv_field(f"{file_name}_1")                     # the digits never change the quoting of the whole field
-    pre, suf = (ident[:-2], '"') if ident.endswith('"') else (ident[:-1], "")
-    strs = [pre, suf, csv_field(psum) + "," + csv_field(file_name)]
-    strs += [csv_field(c) + "," + csv_field(name) for c, name in class_fields]
+    strs = _row_strings(file_name, psum, class_fields)
     sdata, soff = _strings_to_device(strs, dev)
     cidx = torch.as_tensor(class_idx.astype(np.int32), device=dev)
     con = None
@@ -1481,6 +1487,105 @@ def moments01(iset):
     _lib.check(lib.emia_moments01(_ptr(iset.crops), _ptr(iset.meta), _ptr(iset.crop_off), iset.n, _ptr(out), _stream()), "emia_moments01")
     LAUNCHES["count"] += 1
     return out[:iset.n]
+
+
+NB_VALUES = 4      # EMIA_NB_F: centroid x, centroid y, nearest-neighbour distance, edge distance
+NB_INTS = 6        # EMIA_NB_I: listed, nearest neighbour, closest neighbour, touching, agglomerate, agglomerate size
+
+
+@dataclass
+class NeighbourResult:
+    """Relations of the instances of one image (neighbours()): values float64 [n, NB_VALUES] (centroid x / y in frame pixels, the
+    nearest-neighbour and edge distances scaled by um_pix; NaN without a candidate) and ints int32 [n, NB_INTS] (listed, nearest and
+    closest neighbour index or -1, touching count, agglomerate index (-1: not listed), agglomerate size), device tensors."""
+    values: torch.Tensor
+    ints: torch.Tensor
+
+    @property
+    def listed(self):
+        return self.ints[:, 0] != 0
+
+
+def neighbour_cell_size(H, W, n):
+    """Grid cell side of neighbours(): about one instance per cell (frame area over instance count), at least 16 pixels."""
+    return max(16, int(math.ceil(math.sqrt(H * W / max(n, 1)))))
+
+
+def neighbours(iset, class_idx, um_pix=1.0):
+    """Nearest neighbour, closest neighbour, edge distance, touching count and agglomerate of every instance of one image after
+    measure() (definitions: oracle/neighbours.py).  Listed instances are those with a measured record; candidates are listed
+    instances with the same class_idx (an index per instance into the class table of measurements_csv_text).  One host
+    synchronisation sizes the grid's cell lists (buffer_len)."""
+    lib = _lib.load()
+    dev = iset.device
+    assert iset.records is not None, "run measure() first"
+    n = iset.n
+    cidx = np.asarray(class_idx, np.int64).reshape(-1)
+    if len(cidx) != n or (n and cidx.min() < 0):
+        raise ValueError(f"neighbours: class_idx needs {n} non-negative class-table indices")
+    values = torch.empty((max(n, 1), NB_VALUES), dtype=torch.float64, device=dev)
+    ints = torch.empty((max(n, 1), NB_INTS), dtype=torch.int32, device=dev)
+    if n == 0:
+        return NeighbourResult(values[:0], ints[:0])
+    n_class = int(cidx.max()) + 1
+    cs = neighbour_cell_size(iset.H, iset.W, n)
+    ncells = n_class * ((iset.W + cs - 1) // cs) * ((iset.H + cs - 1) // cs)
+    cls = torch.as_tensor(cidx.astype(np.int32), device=dev)
+    with _stage("nb_moments"):
+        mom = moments01(iset)
+    cell_off = torch.empty(ncells + 1, dtype=torch.int64, device=dev)
+    bbox = iset.bbox.contiguous()
+    st = _stream()
+    with _stage("nb_plan"):
+        _lib.check(lib.emia_neighbour_plan(_ptr(iset.records.contiguous()), _ptr(iset.cont_off), _ptr(bbox), _ptr(mom), _ptr(cls), n,
+                                           n_class, iset.H, iset.W, cs, _ptr(values), _ptr(ints), _ptr(cell_off), st),
+                   "emia_neighbour_plan")
+    with _stage("nb_scan"):
+        exclusive_scan_(cell_off)
+    n_ent = buffer_len(cell_off[ncells:], ncells)
+    ent = torch.empty(max(n_ent, 1), dtype=torch.int32, device=dev)
+    work = torch.empty(n + ncells, dtype=torch.int32, device=dev)
+    with _stage("nb_search"):
+        _lib.check(lib.emia_neighbour_search(_ptr(iset.crops), _ptr(iset.meta), _ptr(iset.crop_off), _ptr(bbox), _ptr(cls), n, n_class,
+                                             iset.H, iset.W, cs, _ptr(cell_off), _ptr(ent), float(um_pix), _ptr(values), _ptr(ints),
+                                             _ptr(work), st), "emia_neighbour_search")
+    LAUNCHES["count"] += 5
+    return NeighbourResult(values[:n], ints[:n])
+
+
+def neighbours_csv_text(iset, nb, file_name, psum, class_idx, class_fields):
+    """The rows of neighbours_results.csv for the listed instances of `iset` (nb = neighbours(iset, class_idx, ...)), in instance
+    order: byte for byte what csv.writer writes for inference.neighbour_rows, UTF-8, "\\r\\n" line ends.  Instance_ID, Class,
+    Class_Name, Detected scale bar and File name as in measurements_csv_text.  One host synchronisation to size the text, one D2H
+    copy."""
+    lib = _lib.load()
+    dev = iset.device
+    n = iset.n
+    class_idx = np.asarray(class_idx, np.int64).reshape(-1)
+    if len(class_idx) != n or (n and (class_idx.min() < 0 or class_idx.max() >= len(class_fields))):
+        raise ValueError(f"neighbours_csv_text: class_idx needs {n} indices into the {len(class_fields)} class_fields")
+    if tuple(nb.values.shape) != (n, NB_VALUES) or tuple(nb.ints.shape) != (n, NB_INTS):
+        raise ValueError(f"neighbours_csv_text: nb must be the neighbours() result of this {n}-instance set")
+    if n == 0:
+        return b""
+    strs = _row_strings(file_name, psum, class_fields)
+    sdata, soff = _strings_to_device(strs, dev)
+    cidx = torch.as_tensor(class_idx.astype(np.int32), device=dev)
+    values, ints = nb.values.contiguous(), nb.ints.contiguous()
+    row_off = torch.empty(n + 1, dtype=torch.int64, device=dev)
+    st = _stream()
+    args = (_ptr(values), _ptr(ints), n, _ptr(cidx), _ptr(sdata), _ptr(soff), len(strs))
+    with _stage("csv_nb_count"):
+        _lib.check(lib.emia_csv_neighbour_count(*args, _ptr(row_off), st), "emia_csv_neighbour_count")
+    with _stage("csv_nb_scan"):
+        exclusive_scan_(row_off)
+    nbytes = buffer_len(row_off[n:], n)
+    text = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=dev)
+    with _stage("csv_nb_write"):
+        _lib.check(lib.emia_csv_neighbour_write(*args, _ptr(row_off), _ptr(text), st), "emia_csv_neighbour_write")
+    LAUNCHES["count"] += 2
+    with _stage("csv_nb_d2h"):
+        return _text_to_host(text, nbytes)
 
 
 MOMENT_NAMES = ("m00", "m10", "m01", "m20", "m11", "m02", "m30", "m21", "m12", "m03", "mu20", "mu11", "mu02", "mu30", "mu21", "mu12",

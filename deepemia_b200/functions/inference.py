@@ -25,7 +25,7 @@ from .. import engine
 from ..utils import _bridge
 from ..utils.mask_utils import rle_encoding  # noqa: F401  (re-exported like the reference's import)
 from ..utils import spatial_constraints as _sc
-from ..utils.measurements import record_to_dict, KEY_ORDER, SHAPE_HEADER
+from ..utils.measurements import record_to_dict, KEY_ORDER, SHAPE_HEADER, NEIGHBOUR_HEADER
 
 # ---- module-level settings (reference: config.yaml via inference.py:55-93) ---------------------------------------------------
 PARALLEL_MASK_PROCESSING = True            # l4_performance_optimizations.enable_parallel_mask_processing
@@ -544,6 +544,26 @@ def _measure_text(iset, classes, image_shape, um_pix, test_img, psum, class_name
                                         engine.shape_descriptors(iset) if shape_columns else None)
 
 
+def neighbour_rows(iset, nb, file_name, psum, class_idx, class_fields):
+    """Rows of neighbours_results.csv for one image from the device values of nb = engine.neighbours(iset, class_idx, ...): one per
+    listed instance, in instance order, as Python values (None for an empty field).  The reference for the device text of
+    engine.neighbours_csv_text, as measure_masks is for the measurement rows."""
+    vals = nb.values.cpu().numpy()
+    ints = nb.ints.cpu().numpy()
+    ident = lambda k: f"{file_name}_{int(k) + 1}"                                   # noqa: E731
+    rows = []
+    for k in range(iset.n):
+        listed, nn, closest, touching, agg, size = (int(v) for v in ints[k])
+        if not listed:
+            continue
+        cls, name = class_fields[int(class_idx[k])]
+        has = nn >= 0
+        rows.append([ident(k), cls, name, float(vals[k, 0]), float(vals[k, 1]), ident(nn) if has else None,
+                     float(vals[k, 2]) if has else None, ident(closest) if has else None, float(vals[k, 3]) if has else None, touching,
+                     ident(agg), size, psum, file_name])
+    return rows
+
+
 def _class_table(classes, class_names):
     """(Class, Class_Name) pairs of the distinct classes as measure_masks names them, and each instance's index among them."""
     fields, index, class_idx = [], {}, []
@@ -720,7 +740,7 @@ def _write_csv(path, header, texts):
 
 def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw_id=False, dataset_format="json", draw_scalebar=False,
                   *, images=None, predictors=None, thing_classes=None, small_classes=None, scale_bar_fn=None, shape_columns=False,
-                  **infer_kwargs):
+                  neighbours=False, **infer_kwargs):
     """run_inference (src/functions/inference.py:499-1351), same signature and call shape as main.py:480-488:
 
         run_inference(dataset_name, output_dir, visualize=..., threshold=..., draw_id=..., dataset_format=..., draw_scalebar=...)
@@ -733,7 +753,8 @@ def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw
     K6 and one K5 pass per image, no mask round trip).  Writes R50_flip_results.csv, measurements_results.csv,
     class_color_legend.txt and, with visualize, <name>_predictions.png (overlay kernel + labels).  shape_columns: each row of
     measurements_results.csv continues after "File name" with the ten SHAPE_HEADER columns (area, convex hull, Feret diameters,
-    centroid: engine.shape_descriptors)."""
+    centroid: engine.shape_descriptors).  neighbours: also writes neighbours_results.csv (NEIGHBOUR_HEADER: nearest neighbour, edge
+    distance, touching neighbours and agglomerate of every instance with rows in measurements_results.csv; engine.neighbours)."""
     images = _resolve_images(dataset_name, images)
     if thing_classes is None and _PROVIDERS["thing_classes"]:
         thing_classes = _PROVIDERS["thing_classes"](dataset_name)
@@ -763,7 +784,7 @@ def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw
     small_classes = set(small_classes)
     os.makedirs(output_dir, exist_ok=True)
     bars = _scale_bars(images, dataset_name, dataset_config, output_dir, scale_bar_fn, draw_scalebar)
-    rle_text, meas_text = [], []
+    rle_text, meas_text, nb_text = [], [], []
     shape_kw = {"shape_columns": True} if shape_columns else {}      # without the option, _measure_text is called as it always was
     for (name, image), (psum, um_pix) in zip(images, bars):
         d = _infer_image_dev(predictors, image, num_classes, small_classes, dataset_name=dataset_name, **kw)
@@ -773,11 +794,17 @@ def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw
         rle_text.append(engine.rle_csv_text(run_off, runs, _stem(name)))
         meas_text.append(_measure_text(d.iset, d.classes, image.shape, um_pix, name, psum, class_names=thing_classes,
                                        original_image=image, **shape_kw))
+        if neighbours:
+            fields, class_idx = _class_table(d.classes, thing_classes)
+            nb = engine.neighbours(d.iset, class_idx, um_pix)
+            nb_text.append(engine.neighbours_csv_text(d.iset, nb, name, psum, class_idx, fields))
         if visualize:
             from ..utils.visualize import render_predictions
             cv2.imwrite(os.path.join(output_dir, f"{name}_predictions.png"), render_predictions(image, d.iset, d.classes, thing_classes))
     _write_csv(os.path.join(output_dir, "R50_flip_results.csv"), ["ImageId", "EncodedPixels"], rle_text)
     _write_csv(os.path.join(output_dir, "measurements_results.csv"), CSV_HEADER + (SHAPE_HEADER if shape_columns else []), meas_text)
+    if neighbours:
+        _write_csv(os.path.join(output_dir, "neighbours_results.csv"), NEIGHBOUR_HEADER, nb_text)
     write_class_color_legend(output_dir, thing_classes)
     return None
 
@@ -829,13 +856,14 @@ def load_rle_results(path, images):
     return out
 
 
-def remeasure_results(dataset_name, results_dir, output_dir, *, images=None, scale_bar_fn=None, shape_columns=False):
+def remeasure_results(dataset_name, results_dir, output_dir, *, images=None, scale_bar_fn=None, shape_columns=False, neighbours=False):
     """Measure the masks a run_inference call saved in results_dir again, without the models: writes output_dir/
     measurements_results.csv as run_inference would with the scale bars (and settings such as measure_contrast_distribution) of
     now.  Images and scale bars resolve exactly as in run_inference (images= / the images provider; scale_bar_fn / the scale_bar
     provider / the package's detector).  Class and Class_Name of an instance are those of its rows in results_dir's
     measurements_results.csv; an instance without rows there has no contour above the area gate (which depends only on the frame
-    size) and gets none here either.  shape_columns: as in run_inference, whether or not the old file has them."""
+    size) and gets none here either.  shape_columns: as in run_inference, whether or not the old file has them.  neighbours: also
+    writes output_dir/neighbours_results.csv as run_inference does, with the classes of the old rows."""
     if os.path.realpath(output_dir) == os.path.realpath(results_dir):
         raise ValueError("remeasure_results: output_dir must differ from results_dir (its measurements_results.csv is an input)")
     images = _resolve_images(dataset_name, images)
@@ -850,7 +878,7 @@ def remeasure_results(dataset_name, results_dir, output_dir, *, images=None, sca
         raise ValueError(f"remeasure_results: {results_dir}/measurements_results.csv does not start with the measurements header")
     class_of = {r[0]: (r[1], r[2]) for r in old[1:]}
     os.makedirs(output_dir, exist_ok=True)
-    texts = []
+    texts, nb_text = [], []
     for (name, image), (psum, um_pix) in zip(images, _scale_bars(images, dataset_name, _dataset_config(dataset_name), output_dir,
                                                                   scale_bar_fn)):
         iset = sets[name]
@@ -868,4 +896,9 @@ def remeasure_results(dataset_name, results_dir, output_dir, *, images=None, sca
             class_idx[k] = index.setdefault(class_of[key], len(index))
         texts.append(engine.measurements_csv_text(iset, name, psum, class_idx, list(index), _contrast(iset, image),
                                                   engine.shape_descriptors(iset) if shape_columns else None))
+        if neighbours:
+            nb = engine.neighbours(iset, class_idx, um_pix)
+            nb_text.append(engine.neighbours_csv_text(iset, nb, name, psum, class_idx, list(index)))
     _write_csv(os.path.join(output_dir, "measurements_results.csv"), CSV_HEADER + (SHAPE_HEADER if shape_columns else []), texts)
+    if neighbours:
+        _write_csv(os.path.join(output_dir, "neighbours_results.csv"), NEIGHBOUR_HEADER, nb_text)

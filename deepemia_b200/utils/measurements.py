@@ -15,6 +15,10 @@ _FIELDS = {"major_axis_length": engine.REC_MAJOR, "minor_axis_length": engine.RE
 # the opt-in columns after "File name" (no reference counterpart): engine.shape_descriptors / core/emia_shape.cuh
 SHAPE_HEADER = ["Area", "Convex area", "Solidity", "Convex perimeter", "Convexity", "Max Feret diameter", "Min Feret diameter",
                 "Feret angle", "Centroid X", "Centroid Y"]
+# the columns of the opt-in neighbours_results.csv (no reference counterpart): engine.neighbours / core/emia_neighbour.cuh
+NEIGHBOUR_HEADER = ["Instance_ID", "Class", "Class_Name", "Centroid X", "Centroid Y", "Nearest neighbour", "Nearest neighbour distance",
+                    "Closest neighbour", "Edge distance", "Touching neighbours", "Agglomerate", "Agglomerate size", "Detected scale bar",
+                    "File name"]
 KEY_ORDER = ["major_axis_length", "minor_axis_length", "eccentricity", "Length", "Width", "CircularED", "Aspect_Ratio", "Circularity",
              "Chords", "Feret_diam", "Roundness", "Sphericity", "contrast_d10", "contrast_d50", "contrast_d90"]
 

@@ -357,6 +357,34 @@ int emia_csv_measure_shape_count(const double* records, const int32_t* rec_inst,
 int emia_csv_measure_shape_write(const double* records, const int32_t* rec_inst, int64_t n_rec, const int32_t* class_idx,
                                  const double* contrast, const double* shape, const uint8_t* strs, const int64_t* str_off, int n_str,
                                  const int64_t* row_off, uint8_t* text, void* stream);
+/* ---- neighbours_results.csv: relations between the particles of one image (no reference counterpart; definitions in
+ * oracle/neighbours.py).  LISTED instances are those with a record whose EMIA_REC_MEASURED is 1; CANDIDATES are two listed
+ * instances of the same class key class_idx[i] in [0, n_class).  Outputs per instance:
+ *   nbf[i][4] (double): centroid x = m10 / m00, y = m01 / m00 (frame pixels), sqrt(d2) * um_pix of the centroid nearest neighbour,
+ *     sqrt(D2) * um_pix of the closest mask (D2 = least integer squared pixel distance between the masks); NaN when none;
+ *   nbi[i][6] (int32): listed, nearest neighbour, closest neighbour (-1: no candidate; ties to the lowest index), the number of
+ *     candidates with D2 <= 2, the agglomerate (lowest member of the component of D2 <= 2 edges; -1 when not listed), its size.
+ * Grid: cells of cell_size pixels, gx = ceil(W / cell_size), gy = ceil(H / cell_size), ncells = n_class * gx * gy.  bbox[i] (y_min,
+ * x_min, y_max, x_max) must contain the instance's pixels.
+ * emia_neighbour_plan: records / inst_cont_off as emia_contour_measure writes them, moments01 from emia_moments01; fills nbf / nbi
+ *   for the listed flag and centroid, and cell_cnt[ncells + 1] (cleared inside) with the cells each listed bbox covers.  The caller
+ *   scans cell_cnt (emia_exclusive_scan_i64) into cell_off; cell_off[ncells] entries of ent.
+ * emia_neighbour_search: fills ent and the rest of nbf / nbi; work = n + ncells int32 of workspace.  The results do not depend on
+ *   the order of the entries inside a cell. */
+int emia_neighbour_plan(const double* records, const int64_t* inst_cont_off, const int32_t* bbox, const int64_t* moments01,
+                        const int32_t* class_idx, int64_t n, int32_t n_class, int32_t H, int32_t W, int32_t cell_size, double* nbf,
+                        int32_t* nbi, int64_t* cell_cnt, void* stream);
+int emia_neighbour_search(const uint32_t* crops, const emia_inst_meta* meta, const int64_t* crop_off, const int32_t* bbox,
+                          const int32_t* class_idx, int64_t n, int32_t n_class, int32_t H, int32_t W, int32_t cell_size,
+                          const int64_t* cell_off, int32_t* ent, double um_pix, double* nbf, int32_t* nbi, int32_t* work, void* stream);
+/* emia_csv_neighbour_count / _write: one row per listed instance of neighbours_results.csv, count -> scan -> write as the measurement
+ *   rows: Instance_ID (strs[0] + index + 1 + strs[1], also for the three neighbour fields), Class,Class_Name (strs[3 + class_idx]),
+ *   the values of nbf / nbi (Python float repr, decimal integers; empty without a candidate), strs[2] (Detected scale bar,File name),
+ *   "\r\n".  Rows of instances that are not listed are empty. */
+int emia_csv_neighbour_count(const double* nbf, const int32_t* nbi, int64_t n, const int32_t* class_idx, const uint8_t* strs,
+                             const int64_t* str_off, int n_str, int64_t* row_len, void* stream);
+int emia_csv_neighbour_write(const double* nbf, const int32_t* nbi, int64_t n, const int32_t* class_idx, const uint8_t* strs,
+                             const int64_t* str_off, int n_str, const int64_t* row_off, uint8_t* text, void* stream);
 /* raw moments (m00, m10, m01) of every instance as exact integers: cv2.moments(mask) of src/functions/inference.py:1101-1104 */
 int emia_moments01(const uint32_t* crops, const emia_inst_meta* meta, const int64_t* crop_off, int64_t n, int64_t* out,
                    void* stream);
