@@ -105,7 +105,11 @@ struct EmiaTraceState {
     uint32_t* mk;
     uint32_t* ng;
     EmiaContourOut o;
-    int y, c;                 // scan position (row, word)
+    // scan position (row, word).  A trace without marks never scans: while it follows the seeded contour, the row holds wleft,
+    // the border-start candidates (foreground pixels whose west neighbour is background) not yet accounted for; every step
+    // whose examined-empty arc contains W takes one off (see emia_trace_begin_seeded)
+    union { int y; int wleft; };
+    int c;
     uint32_t done_mask;       // bits of the current word already examined
     int x0, y0, x1, y1, x3, y3, s, prev_s;
     // 3 x 64-pixel window of the crop around the border pixel being followed: rows wy-1, wy, wy+1, word columns wc, wc+1
@@ -121,6 +125,18 @@ struct EmiaTraceState {
 #define EMIA_TRACE_SCAN 0
 #define EMIA_TRACE_FOLLOW 1
 #define EMIA_TRACE_DONE 2
+#define EMIA_TRACE_START 3    // a border starts at (x0, y0): emia_trace_start
+
+// Seed of a crop (emia_trace_seed): the first foreground pixel in raster order and the crop's candidate count, packed into one
+// int64; negative values are the two cases without a seeded start
+#define EMIA_SEED_PACK(x, y, ncand) ((int64_t)(x) | ((int64_t)(y) << 16) | ((int64_t)(ncand) << 32))
+#define EMIA_SEED_X(s) ((int)((s) & 0xFFFF))
+#define EMIA_SEED_Y(s) ((int)(((s) >> 16) & 0xFFFF))
+#define EMIA_SEED_NCAND(s) ((int)((s) >> 32))
+#define EMIA_SEED_EMPTY ((int64_t)-1)      // no foreground pixel: no contour
+#define EMIA_SEED_CLASSIC ((int64_t)-2)    // the crop's extent does not fit the packing: trace with the full scan
+// x < 2^16 and y < 2^16; the candidate count (at most half the pixels) then stays below 2^31
+#define EMIA_SEED_FITS(ch, cw) ((ch) <= 0xFFFF && (cw) <= 0x7FF)
 
 EMIA_HD void emia_trace_begin(EmiaTraceState& T) {
     T.o.n_contours = 0; T.o.n_pts = 0; T.o.overflow = 0;
@@ -196,7 +212,44 @@ EMIA_HD void emia_mark_or(uint32_t* word, uint32_t bit) {
 #endif
 }
 
-// One scan step: walks the rest of the current row for a start candidate.  Returns the next phase.
+// Mark-plane update of a followed border pixel; a trace without marks (mk == nullptr, the seeded first contour) skips it.
+EMIA_HD void emia_trace_mark(const EmiaTraceState& T, int x, int y, int negative) {
+    if (!T.mk) return;
+    const int wi = y * T.v.wwords + (x >> 5);
+    const uint32_t bit = 1u << (x & 31);
+    emia_mark_or(&T.mk[wi], bit);
+    if (negative) emia_mark_or(&T.ng[wi], bit);
+}
+
+// Start following the outer border whose start pixel is (x0, y0) (local).  Returns the next phase.
+EMIA_HD int emia_trace_start(EmiaTraceState& T) {
+    const EmiaBitView& v = T.v;
+    EmiaContourOut& o = T.o;
+    const int x = T.x0, y = T.y0;
+    if (o.store && o.n_contours >= o.cap_contours) { o.overflow = 1; return EMIA_TRACE_DONE; }
+    emia_win_move(T, x, y);
+    const uint32_t N8 = emia_win_nbr8(T, x);
+    // first neighbour clockwise from W: directions 3,2,1,0,7,6,5 -> bit k of M
+    const uint32_t M = ((N8 >> 3) & 1u) | (((N8 >> 2) & 1u) << 1) | (((N8 >> 1) & 1u) << 2) | ((N8 & 1u) << 3) |
+                       (((N8 >> 7) & 1u) << 4) | (((N8 >> 6) & 1u) << 5) | (((N8 >> 5) & 1u) << 6);
+    if (M == 0u) {   // isolated pixel: its W neighbour is examined and found empty once
+        emia_trace_mark(T, x, y, 1);
+        if (!T.mk) T.wleft--;
+        emia_contour_emit(o, v.x_origin + x, v.y_origin + y);
+        emia_contour_close(o);
+        o.n_contours++;
+        if (o.store) o.cstart[o.n_contours] = o.n_pts;
+        return o.overflow ? EMIA_TRACE_DONE : EMIA_TRACE_SCAN;
+    }
+    T.s = (3 - emia_ctz(M)) & 7;
+    T.x1 = x + EMIA_DX(T.s); T.y1 = y + EMIA_DY(T.s);
+    T.x3 = x; T.y3 = y;
+    T.prev_s = T.s ^ 4;
+    return EMIA_TRACE_FOLLOW;
+}
+
+// One scan step: walks the rest of the current row for a start candidate.  Returns the next phase (EMIA_TRACE_START with the
+// candidate in (x0, y0) when a border starts there).
 EMIA_HD int emia_trace_scan_step(EmiaTraceState& T) {
     const EmiaBitView& v = T.v;
     const int ww = v.wwords;
@@ -244,44 +297,23 @@ EMIA_HD int emia_trace_scan_step(EmiaTraceState& T) {
             if (!((T.ng[y * ww + cc] >> hb) & 1u)) return EMIA_TRACE_SCAN;   // inside an already-followed outer border
         }
     }
-    EmiaContourOut& o = T.o;
-    if (o.store && o.n_contours >= o.cap_contours) { o.overflow = 1; return EMIA_TRACE_DONE; }
-    emia_win_move(T, x, y);
-    const uint32_t N8 = emia_win_nbr8(T, x);
-    // first neighbour clockwise from W: directions 3,2,1,0,7,6,5 -> bit k of M
-    const uint32_t M = ((N8 >> 3) & 1u) | (((N8 >> 2) & 1u) << 1) | (((N8 >> 1) & 1u) << 2) | ((N8 & 1u) << 3) |
-                       (((N8 >> 7) & 1u) << 4) | (((N8 >> 6) & 1u) << 5) | (((N8 >> 5) & 1u) << 6);
-    const int wi = y * ww + (x >> 5);
-    const uint32_t bit = 1u << (x & 31);
-    if (M == 0u) {   // isolated pixel
-        emia_mark_or(&T.mk[wi], bit); emia_mark_or(&T.ng[wi], bit);
-        emia_contour_emit(o, v.x_origin + x, v.y_origin + y);
-        emia_contour_close(o);
-        o.n_contours++;
-        if (o.store) o.cstart[o.n_contours] = o.n_pts;
-        return o.overflow ? EMIA_TRACE_DONE : EMIA_TRACE_SCAN;
-    }
-    T.s = (3 - emia_ctz(M)) & 7;
-    T.x0 = x; T.y0 = y; T.x1 = x + EMIA_DX(T.s); T.y1 = y + EMIA_DY(T.s);
-    T.x3 = x; T.y3 = y;
-    T.prev_s = T.s ^ 4;
-    return EMIA_TRACE_FOLLOW;
+    T.x0 = x; T.y0 = y;
+    return EMIA_TRACE_START;
 }
 
 // One border-following step.  Returns the next phase.
 EMIA_HD int emia_trace_follow_step(EmiaTraceState& T) {
     const EmiaBitView& v = T.v;
-    const int ww = v.wwords;
     EmiaContourOut& o = T.o;
     const uint32_t N8 = emia_win_nbr8(T, T.x3);                    // the window was centred on (x3, y3) by the previous step
     const int s_end = T.s;
     const int r = (s_end + 1) & 7;
     const uint32_t rot = ((N8 >> r) | (N8 << (8 - r))) & 0xFFu;
-    const int s = (s_end + 1 + emia_ctz(rot)) & 7;                 // next foreground neighbour counter-clockwise
-    const int wi = T.y3 * ww + (T.x3 >> 5);
-    const uint32_t bit = 1u << (T.x3 & 31);
-    emia_mark_or(&T.mk[wi], bit);                                   // label +2 ...
-    if ((unsigned)(s - 1) < (unsigned)s_end) emia_mark_or(&T.ng[wi], bit);   // ... or -126 when the east neighbour was examined empty
+    const int e = emia_ctz(rot);                                    // neighbours examined and found empty: s_end+1 .. s_end+e
+    const int s = (s_end + 1 + e) & 7;                              // next foreground neighbour counter-clockwise
+    // label +2, or -126 when the east neighbour was examined empty
+    emia_trace_mark(T, T.x3, T.y3, (unsigned)(s - 1) < (unsigned)s_end);
+    if (!T.mk) T.wleft -= ((3 - s_end) & 7) < e;                    // the west neighbour was examined empty
     if (s != T.prev_s) {
         emia_contour_emit(o, v.x_origin + T.x3, v.y_origin + T.y3);
         T.prev_s = s;
@@ -300,6 +332,10 @@ EMIA_HD int emia_trace_follow_step(EmiaTraceState& T) {
     return EMIA_TRACE_FOLLOW;
 }
 
+EMIA_HD int emia_trace_step(EmiaTraceState& T, int phase) {
+    return phase == EMIA_TRACE_SCAN ? emia_trace_scan_step(T) : phase == EMIA_TRACE_START ? emia_trace_start(T) : emia_trace_follow_step(T);
+}
+
 // marks_zeroed != 0: the caller cleared both planes already (the kernels clear the whole buffer with coalesced stores).
 EMIA_HD_NOINLINE void emia_find_external_contours(const EmiaBitView& v, uint32_t* mk, uint32_t* ng, EmiaContourOut& o, int marks_zeroed = 0) {
     const int nw = v.h * v.wwords;
@@ -308,7 +344,71 @@ EMIA_HD_NOINLINE void emia_find_external_contours(const EmiaBitView& v, uint32_t
     T.v = v; T.mk = mk; T.ng = ng; T.o = o;
     emia_trace_begin(T);
     int phase = EMIA_TRACE_SCAN;
-    while (phase != EMIA_TRACE_DONE) phase = (phase == EMIA_TRACE_SCAN) ? emia_trace_scan_step(T) : emia_trace_follow_step(T);
+    while (phase != EMIA_TRACE_DONE) phase = emia_trace_step(T, phase);
+    o = T.o;
+}
+
+// ---- seeded trace: the first contour without the row scan ------------------------------------------------------------
+// In RETR_EXTERNAL mode a border can start only at a candidate (a foreground pixel whose west neighbour is background), and a
+// marked candidate starts nothing.  So:
+//  - the first border starts at the first foreground pixel in raster order (nothing is marked yet, nothing lies to its left);
+//  - following a border examines the west neighbour of each of its candidates, once per candidate (T.wleft counts these
+//    examinations down from the crop's candidate count).  When the first border closes with wleft == 0, every candidate is
+//    marked, the scan would start nothing more, and the crop has exactly one external contour.  The border is then followed
+//    without reading or writing the mark planes at all.
+// Otherwise (a hole, a second component) the crop is traced again from row 0 with marks (emia_trace_restart).
+
+// Seed of a crop (the serial form of k_trace_seed).
+EMIA_HD int64_t emia_trace_seed(const EmiaBitView& v) {
+    if (!EMIA_SEED_FITS(v.h, v.wwords)) return EMIA_SEED_CLASSIC;
+    int64_t first = -1, ncand = 0;
+    for (int y = 0; y < v.h; ++y) {
+        const uint32_t* row = v.bits + (size_t)y * v.pitch_words;
+        for (int c = 0; c < v.wwords; ++c) {
+            const uint32_t F = row[c];
+            const uint32_t left = (F << 1) | (c > 0 ? (row[c - 1] >> 31) : 0u);
+            ncand += emia_popc(F & ~left);
+            if (F && first < 0) first = EMIA_SEED_PACK(c * 32 + emia_ctz(F), y, 0);
+        }
+    }
+    return first < 0 ? EMIA_SEED_EMPTY : first | EMIA_SEED_PACK(0, 0, ncand);
+}
+
+// Begin a trace from its seed without marks (T.mk == nullptr).  Returns the next phase; EMIA_TRACE_SCAN with T.mk == nullptr
+// means the seeded part is over: the crop is done when T.wleft == 0, and is traced again with emia_trace_restart otherwise.
+EMIA_HD int emia_trace_begin_seeded(EmiaTraceState& T, int64_t seed) {
+    T.mk = nullptr; T.ng = nullptr;
+    emia_trace_begin(T);
+    if (seed < 0) { T.wleft = (seed == EMIA_SEED_EMPTY) ? 0 : -1; return EMIA_TRACE_SCAN; }
+    T.wleft = EMIA_SEED_NCAND(seed);
+    T.x0 = EMIA_SEED_X(seed); T.y0 = EMIA_SEED_Y(seed);
+    return EMIA_TRACE_START;
+}
+
+// The classic trace from row 0 with marks: clears the two planes (h * wwords words each) and resets the output.
+EMIA_HD void emia_trace_restart(EmiaTraceState& T, uint32_t* mk, uint32_t* ng) {
+    const int nw = T.v.h * T.v.wwords;
+    for (int i = 0; i < nw; ++i) { mk[i] = 0u; ng[i] = 0u; }
+    T.mk = mk; T.ng = ng;
+    emia_trace_begin(T);
+}
+
+// Plain driver of the seeded trace; same result as emia_find_external_contours.  *fast = 1 when the seeded contour was the
+// only one (no restart).
+EMIA_HD_NOINLINE void emia_find_external_contours_seeded(const EmiaBitView& v, int64_t seed, uint32_t* mk, uint32_t* ng,
+                                                          EmiaContourOut& o, int* fast) {
+    EmiaTraceState T;
+    T.v = v; T.o = o;
+    int phase = emia_trace_begin_seeded(T, seed);
+    *fast = 1;
+    while (phase != EMIA_TRACE_DONE) {
+        if (phase == EMIA_TRACE_SCAN && !T.mk) {
+            if (T.wleft == 0) break;
+            emia_trace_restart(T, mk, ng);
+            *fast = 0;
+        }
+        phase = emia_trace_step(T, phase);
+    }
     o = T.o;
 }
 

@@ -592,6 +592,46 @@ __global__ void k_trace_caps(const emia_inst_meta* __restrict__ meta, int64_t n,
     cap[i] = (m.ch > 0 && m.cw > 0) ? (int64_t)(4 * (m.ch + 32 * m.cw) + 32) : 0;
 }
 
+// Seed of every crop for k_contour_trace_slab (emia_trace_seed, one warp per instance, coalesced over the crop words): the first
+// foreground pixel in raster order and the number of border-start candidates, written to seed[i].
+__global__ void __launch_bounds__(256) k_trace_seed(const uint32_t* __restrict__ crops, const emia_inst_meta* __restrict__ meta,
+                                                    const int64_t* __restrict__ crop_off, int64_t n, int64_t* __restrict__ seed,
+                                                    const int32_t* __restrict__ abort_flag) {
+    if (abort_flag && *abort_flag) return;
+    const int lane = threadIdx.x & 31;
+    const int64_t warps = (int64_t)gridDim.x * (blockDim.x >> 5);
+    for (int64_t i = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); i < n; i += warps) {
+        const emia_inst_meta m = meta[i];
+        const int cw = m.cw, words = m.ch * m.cw;
+        if (words <= 0 || !EMIA_SEED_FITS(m.ch, m.cw)) {
+            if (lane == 0) seed[i] = words <= 0 ? EMIA_SEED_EMPTY : EMIA_SEED_CLASSIC;
+            continue;
+        }
+        const uint32_t* bits = crops + crop_off[i];
+        unsigned first = 0xFFFFFFFFu, ncand = 0u;
+        // word j of the crop is column c = j % cw of its row; 32 % cw < cw steps c from one word of this lane to the next
+        const int step = 32 % cw;
+        int c = lane % cw;
+        for (int j = lane; j < words; j += 32) {
+            const uint32_t F = bits[j];
+            const uint32_t left = (F << 1) | (c > 0 ? (bits[j - 1] >> 31) : 0u);
+            ncand += __popc(F & ~left);
+            if (F != 0u && first == 0xFFFFFFFFu) first = (unsigned)j;
+            c += step;
+            if (c >= cw) c -= cw;
+        }
+        first = __reduce_min_sync(0xFFFFFFFFu, first);
+        ncand = __reduce_add_sync(0xFFFFFFFFu, ncand);
+        if (lane == 0) {
+            if (first == 0xFFFFFFFFu) seed[i] = EMIA_SEED_EMPTY;
+            else {
+                const int y = (int)first / cw;
+                seed[i] = EMIA_SEED_PACK(((int)first - y * cw) * 32 + __ffs(bits[first]) - 1, y, ncand);
+            }
+        }
+    }
+}
+
 // Lanes are PERSISTENT inside a CTA-owned chunk of instances: a lane that finishes its instance takes the next one from a
 // shared-memory counter INSIDE the same flat loop (phase "next"), so the warp keeps executing one instruction stream with
 // most lanes busy — border lengths differ 4x between instances and one-instance-per-thread left 8 of 32 lanes active (ncu).
@@ -642,15 +682,20 @@ __global__ void __launch_bounds__(EMIA_TRACE_THREADS, EMIA_TRACE_MIN_CTAS) k_con
             if (m.ch * m.cw <= 0) { cs[0] = 0; n_contours[i] = 0; scratch_bytes[i] = 0; i = -1; continue; }
             const int64_t off = crop_off[i];
             T.v = emia_make_view(crops, m, off);
-            T.mk = marks + 2 * off;
-            T.ng = T.mk + m.ch * m.cw;
             T.o.pts = pts + pt_cap_off[i]; T.o.cap_pts = (int)(pt_cap_off[i + 1] - pt_cap_off[i]);
             T.o.cstart = cs; T.o.cap_contours = capc; T.o.store = 1;
             T.o.track = perim0 != nullptr; T.o.diag = s_diag;
-            emia_trace_begin(T);
-            phase = EMIA_TRACE_SCAN;
+            phase = emia_trace_begin_seeded(T, n_contours[i]);   // the seed k_trace_seed left in n_contours[i]
         } else if (phase == EMIA_TRACE_SCAN) {
+            if (!T.mk) {
+                // the seeded contour is closed: it was the only one, or the crop is traced again with marks
+                if (T.wleft == 0) { phase = EMIA_TRACE_DONE; continue; }
+                uint32_t* mk = marks + 2 * crop_off[i];
+                emia_trace_restart(T, mk, mk + T.v.h * T.v.wwords);
+            }
             phase = emia_trace_scan_step(T);
+        } else if (phase == EMIA_TRACE_START) {
+            phase = emia_trace_start(T);
         } else {
             phase = emia_trace_follow_step(T);
         }
@@ -679,7 +724,7 @@ extern "C" int emia_contour_trace_slab(const uint32_t* crops, const emia_inst_me
     if (chunk < EMIA_TRACE_THREADS) chunk = EMIA_TRACE_THREADS;
     if (chunk > EMIA_TRACE_CHUNK) chunk = EMIA_TRACE_CHUNK;
     const unsigned grid = (unsigned)((n + chunk - 1) / chunk);
-    emia_launch_clear_marks(marks, crop_off, n, (cudaStream_t)stream);
+    k_trace_seed<<<emia_num_sms() * 8, 256, 0, (cudaStream_t)stream>>>(crops, meta, crop_off, n, n_contours, abort_flag);
     k_contour_trace_slab<<<grid, EMIA_TRACE_THREADS, 0, (cudaStream_t)stream>>>(crops, meta, crop_off, n, marks, pt_cap_off, cap_contours, pts,
                                                                              cstart_slab, n_contours, scratch_bytes, overflow, perim0, (int)chunk, abort_flag);
     return emia_check_launch("emia_contour_trace_slab launch: %s");

@@ -135,7 +135,10 @@ int emia_contour_store(const uint32_t* crops, const emia_inst_meta* meta, const 
  * (caller scans them into pt_cap_off), emia_contour_trace_slab follows the borders once into those slabs
  * (cstart_slab: cap_contours + 1 ints per instance) and raises *overflow (caller-zeroed counter) when a capacity is
  * exceeded — the caller then falls back to emia_contour_count / emia_contour_measure; emia_contour_measure_stored
- * computes the records from stored vertices (cstart_stride = cap_contours + 1 for slabs, 0 for the packed layout). */
+ * computes the records from stored vertices (cstart_stride = cap_contours + 1 for slabs, 0 for the packed layout).
+ * emia_contour_trace_slab first writes a per-crop seed (first foreground pixel, candidate count) into n_contours and then
+ * overwrites it with the contour count of every instance; crops with exactly one external contour are followed without
+ * the mark planes, so `marks` (2 words per crop word) needs no initial contents and is left undefined. */
 int emia_contour_trace_plan(const emia_inst_meta* meta, int64_t n, int64_t* pt_cap, void* stream);
 int emia_contour_trace_slab(const uint32_t* crops, const emia_inst_meta* meta, const int64_t* crop_off, int64_t n,
                             uint32_t* marks, const int64_t* pt_cap_off, int32_t cap_contours, uint32_t* pts,
