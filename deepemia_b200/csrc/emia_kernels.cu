@@ -21,6 +21,7 @@
 #include "core/emia_text.cuh"
 #include "core/emia_shape.cuh"
 #include "core/emia_neighbour.cuh"
+#include "core/emia_coco.cuh"
 
 static thread_local char g_err[512] = "";
 static int emia_fail(int code, const char* fmt, const char* detail) {
@@ -829,6 +830,7 @@ extern "C" int emia_paste_threshold_bitpack(const float* probs, const float* box
 #include "emia_tile_kernels.cuh"
 #include "emia_rle_kernels.cuh"
 #include "emia_text_kernels.cuh"
+#include "emia_coco_kernels.cuh"
 #include "emia_neighbour_kernels.cuh"
 #include "emia_flow_kernels.cuh"
 #include "emia_scalebar_kernels.cuh"

@@ -1409,6 +1409,94 @@ def rle_csv_text(run_off, runs, image_id):
         return _text_to_host(text, nbytes)
 
 
+def coco_annotations_text(iset, run_off, runs, image_id, category_ids, scores, first_id):
+    """The "annotations" entries of coco_instances.json for the n instances of `iset` (with (run_off, runs) = rle_encode(iset)), joined
+    by ", ": byte for byte json.dumps of the dicts oracle/coco.py defines.  Instance i gets id first_id + i, image_id, category_id
+    category_ids[i], segmentation {"size": [H, W], "counts": pycocotools' compressed RLE string}, the popcount as area, the tight bbox
+    [x, y, w, h] as floats and float(scores[i]) as score.  Formatted on the device; one host synchronisation to size the text and
+    one D2H copy of it."""
+    lib = _lib.load()
+    dev = iset.device
+    n = iset.n
+    if n <= 0:
+        return b""
+    assert run_off.dtype == torch.int64 and runs.dtype == torch.int64 and run_off.is_contiguous() and runs.is_contiguous()
+    assert int(run_off.numel()) == n + 1
+    cat = torch.as_tensor(np.asarray([int(c) for c in category_ids], np.int32), device=dev)
+    sc = torch.as_tensor(np.asarray([float(s) for s in scores], np.float64), device=dev)
+    assert cat.numel() == n and sc.numel() == n
+    bbox, area = iset.bbox.contiguous(), iset.area.contiguous()
+    ann_off = torch.empty(n + 1, dtype=torch.int64, device=dev)
+    st = _stream()
+    rp = _ptr(runs) if runs.numel() else _ptr(run_off)      # no runs at all: never read, but the ABI wants a pointer
+    args = (rp, _ptr(run_off), n, _ptr(bbox), _ptr(area), _ptr(sc), _ptr(cat), iset.H, iset.W, int(image_id), int(first_id))
+    with _stage("coco_ann_count"):
+        _lib.check(lib.emia_coco_ann_count(*args, _ptr(ann_off), st), "emia_coco_ann_count")
+    with _stage("coco_ann_scan"):
+        exclusive_scan_(ann_off)
+    nbytes = buffer_len(ann_off[n:], n)
+    text = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=dev)
+    with _stage("coco_ann_write"):
+        _lib.check(lib.emia_coco_ann_write(*args, _ptr(ann_off), _ptr(text), st), "emia_coco_ann_write")
+    LAUNCHES["count"] += 2
+    with _stage("coco_ann_d2h"):
+        return _text_to_host(text, nbytes)
+
+
+COCO_STATUS = {1: "counts hold a character outside '0'..'o'", 2: "counts end inside a value",
+               3: "a count below 0 or above 2^31 - 1 (or a value of more than 7 characters)", 4: "counts do not add up to H * W",
+               5: "more than 2^31 - 1 pixels"}
+
+
+def _coco_decode(data, str_off, H, W):
+    """n compressed-RLE counts strings of H x W masks (bytes `data`, string j at data[str_off[j]:str_off[j + 1]]) -> (InstanceSet of
+    the n masks, per-string status as numpy int32: 0 or a COCO_STATUS key).  A rejected string gives an empty mask.  One H2D copy;
+    counts -> runs on the device, then the RLE decode (tight bbox crops, as rle_decode)."""
+    lib = _lib.load()
+    if not (1 <= H <= 65535 and 1 <= W <= 65535):
+        raise _lib.EmiaError(f"coco_decode: frame {H} x {W} outside 1..65535 (the contour vertex packing limit)")
+    dev = _need_cuda(None)
+    off = np.asarray(str_off, np.int64)
+    n = len(off) - 1
+    nbytes = len(data)
+    a = (nbytes + 7) // 8 * 8                                      # the offsets follow the text, 8-byte aligned
+    host = torch.zeros(a + 8 * (n + 1), dtype=torch.uint8, pin_memory=True)
+    hv = host.numpy()
+    hv[:nbytes] = np.frombuffer(bytes(data), np.uint8)
+    hv[a:] = off.view(np.uint8)
+    st = _stream()
+    with _stage("coco_h2d"):
+        both = host.to(dev, non_blocking=True)                    # one H2D copy of text and offsets
+    text = both[:max(a, 1)]
+    s_off = both[a:].view(torch.int64)
+    with _stage("coco_counts"):
+        run_off = torch.zeros(n + 1, dtype=torch.int64, device=dev)
+        status = torch.empty(max(n, 1), dtype=torch.int32, device=dev)
+        _lib.check(lib.emia_coco_counts_count(_ptr(text), _ptr(s_off), n, H, W, _ptr(run_off), _ptr(status), st), "emia_coco_counts_count")
+        exclusive_scan_(run_off)
+        R = buffer_len(run_off[n:], n)
+        runs = torch.empty((max(R, 1), 2), dtype=torch.int64, device=dev)
+        _lib.check(lib.emia_coco_counts_fill(_ptr(text), _ptr(s_off), n, H, W, _ptr(run_off), _ptr(runs), st), "emia_coco_counts_fill")
+    LAUNCHES["count"] += 2
+    iset, plan = _rle_decode(run_off, runs[:R], H, W)
+    code = status[:n].cpu().numpy()
+    code = np.where((code == 0) & (plan != 0), 5, code).astype(np.int32)     # valid counts: only the area limit remains
+    return iset, code
+
+
+def coco_decode(strings, H, W):
+    """The compressed-RLE "counts" strings (str or bytes) of n H x W masks -> InstanceSet, bit for bit the tables rle_decode gives for
+    the same masks (tight bbox crops).  Raises EmiaError naming the first rejected string (0-based) and why."""
+    raw = [s.encode("utf-8") if isinstance(s, str) else bytes(s) for s in strings]
+    off = np.concatenate([[0], np.cumsum([len(b) for b in raw])]).astype(np.int64)
+    iset, status = _coco_decode(b"".join(raw), off, H, W)
+    bad = np.nonzero(status)[0]
+    if len(bad):
+        k = int(bad[0])
+        raise _lib.EmiaError(f"coco_decode: string {k}: {COCO_STATUS[int(status[k])]}")
+    return iset
+
+
 def measurements_csv_text(iset, file_name, psum, class_idx, class_fields, contrast=None, shape=None):
     """The rows of measurements_results.csv for the measured records of `iset` (after measure()), in record order: byte for byte
     what csv.writer writes for the rows of inference.measure_masks, UTF-8, "\\r\\n" line ends.  Instance i gets Instance_ID

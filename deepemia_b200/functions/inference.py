@@ -14,6 +14,7 @@ adapter).  detector_postprocess + paste_masks_in_image then happen in K1.  A lis
 Module-level settings mirror the reference's module globals (inference.py:55-93) and can be overridden by the host application.
 """
 import csv
+import json
 import os
 from dataclasses import dataclass
 
@@ -565,13 +566,18 @@ def neighbour_rows(iset, nb, file_name, psum, class_idx, class_fields):
 
 
 def _class_table(classes, class_names):
-    """(Class, Class_Name) pairs of the distinct classes as measure_masks names them, and each instance's index among them."""
+    """(Class, Class_Name) pairs of the distinct classes as measure_masks names them, and each instance's index among them.
+    class_names: a list indexed by class, or a dict {class: name}; a class it does not name is class_<class>."""
     fields, index, class_idx = [], {}, []
     for cls in classes:
         cls = int(cls)
         if cls not in index:
             index[cls] = len(fields)
-            fields.append((cls, class_names[cls] if class_names is not None and cls < len(class_names) else f"class_{cls}"))
+            if isinstance(class_names, dict):
+                name = class_names.get(cls, f"class_{cls}")
+            else:
+                name = class_names[cls] if class_names is not None and cls < len(class_names) else f"class_{cls}"
+            fields.append((cls, name))
         class_idx.append(index[cls])
     return fields, class_idx
 
@@ -738,9 +744,19 @@ def _write_csv(path, header, texts):
             f.write(t)
 
 
+def _write_coco(path, images, ann_texts, thing_classes, classes):
+    """coco_instances.json: json.dumps of {"images", "annotations", "categories"}, the annotations being the device texts."""
+    cats = [{"id": k, "name": n} for k, n in enumerate(thing_classes)]
+    cats += [{"id": c, "name": f"class_{c}"} for c in sorted(classes) if c >= len(thing_classes)]
+    with open(path, "wb") as f:
+        f.write((json.dumps({"images": images})[:-1] + ', "annotations": [').encode())
+        f.write(b", ".join(t for t in ann_texts if t))
+        f.write(('], "categories": ' + json.dumps(cats) + "}").encode())
+
+
 def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw_id=False, dataset_format="json", draw_scalebar=False,
                   *, images=None, predictors=None, thing_classes=None, small_classes=None, scale_bar_fn=None, shape_columns=False,
-                  neighbours=False, **infer_kwargs):
+                  neighbours=False, coco_json=False, **infer_kwargs):
     """run_inference (src/functions/inference.py:499-1351), same signature and call shape as main.py:480-488:
 
         run_inference(dataset_name, output_dir, visualize=..., threshold=..., draw_id=..., dataset_format=..., draw_scalebar=...)
@@ -754,7 +770,10 @@ def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw
     class_color_legend.txt and, with visualize, <name>_predictions.png (overlay kernel + labels).  shape_columns: each row of
     measurements_results.csv continues after "File name" with the ten SHAPE_HEADER columns (area, convex hull, Feret diameters,
     centroid: engine.shape_descriptors).  neighbours: also writes neighbours_results.csv (NEIGHBOUR_HEADER: nearest neighbour, edge
-    distance, touching neighbours and agglomerate of every instance with rows in measurements_results.csv; engine.neighbours)."""
+    distance, touching neighbours and agglomerate of every instance with rows in measurements_results.csv; engine.neighbours).
+    coco_json: also writes coco_instances.json, COCO instance JSON with compressed RLE (oracle/coco.py defines it): every image, one
+    annotation per line of R50_flip_results.csv (category_id = Class, the score of the final set), formatted on the device
+    (engine.coco_annotations_text) from the same K6 runs."""
     images = _resolve_images(dataset_name, images)
     if thing_classes is None and _PROVIDERS["thing_classes"]:
         thing_classes = _PROVIDERS["thing_classes"](dataset_name)
@@ -785,13 +804,21 @@ def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw
     os.makedirs(output_dir, exist_ok=True)
     bars = _scale_bars(images, dataset_name, dataset_config, output_dir, scale_bar_fn, draw_scalebar)
     rle_text, meas_text, nb_text = [], [], []
+    coco_images, coco_ann, coco_classes, n_ann = [], [], set(), 0
     shape_kw = {"shape_columns": True} if shape_columns else {}      # without the option, _measure_text is called as it always was
     for (name, image), (psum, um_pix) in zip(images, bars):
         d = _infer_image_dev(predictors, image, num_classes, small_classes, dataset_name=dataset_name, **kw)
+        if coco_json:
+            coco_images.append({"id": len(coco_images) + 1, "file_name": name, "height": int(image.shape[0]),
+                                "width": int(image.shape[1])})
         if len(d) == 0:
             continue
         run_off, runs = engine.rle_encode(d.iset)                       # K6 over the final set, once
         rle_text.append(engine.rle_csv_text(run_off, runs, _stem(name)))
+        if coco_json:
+            coco_ann.append(engine.coco_annotations_text(d.iset, run_off, runs, len(coco_images), d.classes, d.scores, n_ann + 1))
+            coco_classes.update(int(c) for c in d.classes)
+            n_ann += len(d)
         meas_text.append(_measure_text(d.iset, d.classes, image.shape, um_pix, name, psum, class_names=thing_classes,
                                        original_image=image, **shape_kw))
         if neighbours:
@@ -805,6 +832,8 @@ def run_inference(dataset_name, output_dir, visualize=True, threshold=0.65, draw
     _write_csv(os.path.join(output_dir, "measurements_results.csv"), CSV_HEADER + (SHAPE_HEADER if shape_columns else []), meas_text)
     if neighbours:
         _write_csv(os.path.join(output_dir, "neighbours_results.csv"), NEIGHBOUR_HEADER, nb_text)
+    if coco_json:
+        _write_coco(os.path.join(output_dir, "coco_instances.json"), coco_images, coco_ann, thing_classes, coco_classes)
     write_class_color_legend(output_dir, thing_classes)
     return None
 
@@ -882,10 +911,7 @@ def remeasure_results(dataset_name, results_dir, output_dir, *, images=None, sca
     for (name, image), (psum, um_pix) in zip(images, _scale_bars(images, dataset_name, _dataset_config(dataset_name), output_dir,
                                                                   scale_bar_fn)):
         iset = sets[name]
-        if iset.n == 0:
-            continue
-        engine.measure(iset, um_pix=um_pix, min_area=engine.default_min_area(image.shape[0], image.shape[1]))
-        measured = np.unique(iset.rec_inst[iset.records[:, engine.REC_MEASURED] == 1.0].cpu().numpy())
+        measured = _measure_saved(iset, image, um_pix)
         if len(measured) == 0:
             continue
         index, class_idx = {}, [0] * iset.n         # (Class, Class_Name) of the old rows -> index; unmeasured instances: unused
@@ -894,11 +920,136 @@ def remeasure_results(dataset_name, results_dir, output_dir, *, images=None, sca
             if key not in class_of:
                 raise ValueError(f"remeasure_results: {key} has a measured contour but no row in {results_dir}/measurements_results.csv")
             class_idx[k] = index.setdefault(class_of[key], len(index))
-        texts.append(engine.measurements_csv_text(iset, name, psum, class_idx, list(index), _contrast(iset, image),
-                                                  engine.shape_descriptors(iset) if shape_columns else None))
-        if neighbours:
-            nb = engine.neighbours(iset, class_idx, um_pix)
-            nb_text.append(engine.neighbours_csv_text(iset, nb, name, psum, class_idx, list(index)))
+        _saved_texts(texts, nb_text, iset, name, image, psum, um_pix, class_idx, list(index), shape_columns, neighbours)
+    _write_results(output_dir, texts, nb_text, shape_columns, neighbours)
+
+
+def _measure_saved(iset, image, um_pix):
+    """engine.measure of an image's saved instances -> the ids (ascending) of those with a measured contour."""
+    if iset.n == 0:
+        return np.zeros(0, np.int64)
+    engine.measure(iset, um_pix=um_pix, min_area=engine.default_min_area(image.shape[0], image.shape[1]))
+    return np.unique(iset.rec_inst[iset.records[:, engine.REC_MEASURED] == 1.0].cpu().numpy())
+
+
+def _saved_texts(texts, nb_text, iset, name, image, psum, um_pix, class_idx, class_fields, shape_columns, neighbours):
+    """The measurements_results.csv rows (and neighbours_results.csv rows) of one image's measured saved instances."""
+    texts.append(engine.measurements_csv_text(iset, name, psum, class_idx, class_fields, _contrast(iset, image),
+                                              engine.shape_descriptors(iset) if shape_columns else None))
+    if neighbours:
+        nb = engine.neighbours(iset, class_idx, um_pix)
+        nb_text.append(engine.neighbours_csv_text(iset, nb, name, psum, class_idx, class_fields))
+
+
+def _write_results(output_dir, texts, nb_text, shape_columns, neighbours):
     _write_csv(os.path.join(output_dir, "measurements_results.csv"), CSV_HEADER + (SHAPE_HEADER if shape_columns else []), texts)
     if neighbours:
         _write_csv(os.path.join(output_dir, "neighbours_results.csv"), NEIGHBOUR_HEADER, nb_text)
+
+
+# =================================================================================================================
+# COCO instance JSON (coco_instances.json, or any COCO file with compressed-RLE masks) -> instances -> measurements_results.csv
+# =================================================================================================================
+def _coco_error(path, ann, why):
+    return ValueError(f"{path}: annotation {ann.get('id')!r}: {why}")
+
+
+def _load_coco(path, images):
+    """(file dict, {file name: InstanceSet with classes / scores}) of a COCO instance file for the (file name, image) pairs."""
+    images = list(images)
+    by_name = {}
+    for k, (name, _) in enumerate(images):
+        if name in by_name:
+            raise ValueError(f"load_coco_results: the file name {name!r} is given twice")
+        by_name[name] = k
+    with open(path, "rb") as f:
+        d = json.loads(f.read())
+    img_of, matched = {}, set()
+    for e in d.get("images", []):
+        name = e.get("file_name")
+        k = by_name.get(name)
+        if k is None:
+            raise ValueError(f"{path}: image {e.get('id')!r}: file_name {name!r} matches no image")
+        if k in matched:
+            raise ValueError(f"{path}: image {e.get('id')!r}: file_name {name!r} appears twice")
+        if e.get("id") in img_of:
+            raise ValueError(f"{path}: image id {e.get('id')!r} appears twice")
+        img_of[e.get("id")] = k
+        matched.add(k)
+    per = [[] for _ in images]                     # (counts bytes, category, score or None, annotation) per image, file order
+    for ann in d.get("annotations", []):
+        seg = ann.get("segmentation")
+        if not isinstance(seg, dict) or not isinstance(seg.get("counts"), str):
+            raise _coco_error(path, ann, "only compressed-RLE segmentations are read (not polygons or uncompressed counts lists)")
+        if ann.get("image_id") not in img_of:
+            raise _coco_error(path, ann, f"image_id {ann.get('image_id')!r} has no images entry")
+        k = img_of[ann["image_id"]]
+        H, W = (int(v) for v in images[k][1].shape[:2])
+        if list(seg.get("size", [])) != [H, W]:
+            raise _coco_error(path, ann, f"size {seg.get('size')!r} is not the image's [{H}, {W}]")
+        cat = ann.get("category_id")
+        if isinstance(cat, bool) or not isinstance(cat, int) or not 0 <= cat <= 2 ** 31 - 1:
+            raise _coco_error(path, ann, f"category_id {cat!r} is not a non-negative integer")
+        per[k].append((seg["counts"].encode("utf-8"), cat, ann.get("score"), ann))
+    by_size = {}
+    for k, (_, image) in enumerate(images):
+        by_size.setdefault(tuple(int(s) for s in image.shape[:2]), []).append(k)
+    out, bad = {}, []
+    for (H, W), ks in by_size.items():
+        items = [it for k in ks for it in per[k]]
+        raw = [it[0] for it in items]
+        off = np.concatenate([[0], np.cumsum([len(b) for b in raw])]).astype(np.int64)
+        iset, status = engine._coco_decode(b"".join(raw), off, H, W)
+        bad += [(items[j][3], int(status[j])) for j in np.nonzero(status)[0][:1]]
+        a = 0
+        for k in ks:
+            m = len(per[k])
+            s = iset if len(ks) == 1 else engine.select(iset, list(range(a, a + m)))
+            dev = s.device
+            s.classes = torch.as_tensor(np.asarray([it[1] for it in per[k]], np.int32), device=dev)
+            scores = [it[2] for it in per[k]]
+            s.scores = torch.as_tensor(np.asarray(scores, np.float32), device=dev) if all(
+                isinstance(v, (int, float)) and not isinstance(v, bool) for v in scores) else None
+            out[images[k][0]] = s
+            a += m
+    if bad:
+        ann, code = min(bad, key=lambda b: d["annotations"].index(b[0]))
+        raise engine._lib.EmiaError(f"{path}: annotation {ann.get('id')!r}: {engine.COCO_STATUS[code]}")
+    return d, out
+
+
+def load_coco_results(path, images):
+    """A COCO instance JSON file with compressed-RLE masks (coco_instances.json of run_inference, an annotation tool's export, a
+    dataset's ground truth) -> {file name: engine.InstanceSet} for the (file name, image) pairs `images` that run_inference takes.
+    Images are matched by file_name; instance k of an image is its k-th annotation in file order; an image without annotations maps
+    to an empty set.  iset.classes (int32) holds the category_id values and iset.scores (float32) the scores when every annotation
+    of the image has one.  The file is parsed with json.loads; the counts strings are decoded on the device, once per distinct frame
+    size, into the tight bbox crops rle_decode gives.  Raises ValueError for a polygon or uncompressed segmentation, a size that is
+    not the image's, an image_id without images entry, a category_id that is not a non-negative integer (each naming the
+    annotation's id), an images entry that matches no image or a file name given twice; EmiaError naming the annotation of a
+    malformed counts string."""
+    return _load_coco(path, images)[1]
+
+
+def measure_coco(path, output_dir, *, images=None, dataset_name=None, scale_bar_fn=None, shape_columns=False, neighbours=False):
+    """Measure the masks of a COCO instance JSON file (load_coco_results): writes output_dir/measurements_results.csv (and, with
+    neighbours, neighbours_results.csv) as run_inference writes them for the same masks.  Class is the category_id; Class_Name its
+    name in the file's categories (class_<id> when it has none).  Images and scale bars resolve as in remeasure_results (images= /
+    the images provider; scale_bar_fn / the scale_bar provider / the package's detector); shape_columns as in run_inference."""
+    images = _resolve_images(dataset_name, images)
+    if images is None:
+        raise FileNotFoundError(f"No images registered for dataset '{dataset_name}': call "
+                                "deepemia_b200.functions.inference.set_providers(...) (or pass images=)")
+    images = list(images)
+    d, sets = _load_coco(path, images)
+    names = {c.get("id"): c.get("name") for c in d.get("categories", [])}
+    os.makedirs(output_dir, exist_ok=True)
+    texts, nb_text = [], []
+    for (name, image), (psum, um_pix) in zip(images, _scale_bars(images, dataset_name, _dataset_config(dataset_name), output_dir,
+                                                                  scale_bar_fn)):
+        iset = sets[name]
+        if len(_measure_saved(iset, image, um_pix)) == 0:
+            continue
+        fields, class_idx = _class_table(iset.classes.cpu().numpy().tolist(), names)
+        _saved_texts(texts, nb_text, iset, name, image, psum, um_pix, class_idx, fields, shape_columns, neighbours)
+    _write_results(output_dir, texts, nb_text, shape_columns, neighbours)

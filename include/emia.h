@@ -388,6 +388,31 @@ int emia_csv_neighbour_count(const double* nbf, const int32_t* nbi, int64_t n, c
                              const int64_t* str_off, int n_str, int64_t* row_len, void* stream);
 int emia_csv_neighbour_write(const double* nbf, const int32_t* nbi, int64_t n, const int32_t* class_idx, const uint8_t* strs,
                              const int64_t* str_off, int n_str, const int64_t* row_off, uint8_t* text, void* stream);
+/* ---- COCO instance JSON with compressed RLE (csrc/emia_coco_kernels.cuh, core/emia_coco.cuh; definition in oracle/coco.py) -------
+ * emia_coco_ann_count / _write: the "annotations" entry of instance i of (run_off, runs) (emia_rle_encode's layout) in an H x W frame,
+ *   count -> exclusive scan of the n + 1 lengths (caller) -> write, byte for byte json.dumps: id first_id + i, image_id, category_id
+ *   category[i], segmentation {"size": [H, W], "counts": pycocotools' rleToString of the column-major counts}, area[i], bbox
+ *   [x_min, y_min, width, height] from bbox[i] (y_min, x_min, y_max, x_max) as floats ([0.0, 0.0, 0.0, 0.0] when area[i] == 0),
+ *   "iscrowd": 0, score[i] as a Python float; entries are followed by ", " except the last.
+ * emia_coco_counts_count: string j = data[str_off[j], str_off[j + 1]) is the counts string of an H x W mask: run_cnt[j] = its
+ *   non-empty foreground runs when well-formed (0 otherwise; caller scans the n + 1 entries into run_off), status[j] = EMIA_COCO_*.
+ * emia_coco_counts_fill: the (start, length) runs of string j at runs[2 * run_off[j] ..] (1-indexed, column-major: the layout of
+ *   emia_rle_encode, adjacent runs where a background count is 0), for emia_rle_decode_plan / emia_rle_decode. */
+#define EMIA_COCO_OK 0
+#define EMIA_COCO_BAD_CHAR 1      /* a character outside '0'..'o' */
+#define EMIA_COCO_OPEN_VALUE 2    /* the string ends inside a value */
+#define EMIA_COCO_RANGE 3         /* a count below 0 or above 2^31 - 1, or a value of more than 7 characters */
+#define EMIA_COCO_SUM 4           /* the counts do not add up to H * W */
+int emia_coco_ann_count(const int64_t* runs, const int64_t* run_off, int64_t n, const int32_t* bbox, const int32_t* area,
+                        const double* score, const int32_t* category, int H, int W, int64_t image_id, int64_t first_id,
+                        int64_t* ann_len, void* stream);
+int emia_coco_ann_write(const int64_t* runs, const int64_t* run_off, int64_t n, const int32_t* bbox, const int32_t* area,
+                        const double* score, const int32_t* category, int H, int W, int64_t image_id, int64_t first_id,
+                        const int64_t* ann_off, uint8_t* text, void* stream);
+int emia_coco_counts_count(const uint8_t* data, const int64_t* str_off, int64_t n, int H, int W, int64_t* run_cnt, int32_t* status,
+                           void* stream);
+int emia_coco_counts_fill(const uint8_t* data, const int64_t* str_off, int64_t n, int H, int W, const int64_t* run_off,
+                          int64_t* runs, void* stream);
 /* raw moments (m00, m10, m01) of every instance as exact integers: cv2.moments(mask) of src/functions/inference.py:1101-1104 */
 int emia_moments01(const uint32_t* crops, const emia_inst_meta* meta, const int64_t* crop_off, int64_t n, int64_t* out,
                    void* stream);
