@@ -105,6 +105,14 @@ _SIGNATURES = {
                                     c_void_p, c_void_p, c_void_p]),
     "emia_coco_counts_count": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "emia_coco_counts_fill": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p]),
+    "emia_cocoeval_order_workspace_bytes": (c_size_t, [c_int64]),
+    "emia_cocoeval_order": (c_int, [c_void_p] * 4 + [c_int64, c_int, c_int64] + [c_void_p] * 4 + [c_size_t, c_void_p]),
+    "emia_cocoeval_grid": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "emia_cocoeval_pair_count": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_int]
+                                 + [c_void_p] * 6 + [c_int, c_void_p, c_void_p]),
+    "emia_cocoeval_pair_fill": (c_int, [c_void_p] * 13 + [c_int64, c_int, c_int, c_int, c_int] + [c_void_p] * 15),
+    "emia_cocoeval_match": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64] + [c_void_p] * 7 + [c_int64] + [c_void_p] * 5),
+    "emia_cocoeval_accumulate": (c_int, [c_void_p] * 7 + [c_int64, c_int] + [c_void_p] * 5),
     "emia_moments01": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "emia_moments": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "emia_color_sums": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int, c_int, c_void_p, c_void_p]),

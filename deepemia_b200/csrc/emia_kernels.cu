@@ -22,6 +22,7 @@
 #include "core/emia_shape.cuh"
 #include "core/emia_neighbour.cuh"
 #include "core/emia_coco.cuh"
+#include "core/emia_cocoeval.cuh"
 
 static thread_local char g_err[512] = "";
 static int emia_fail(int code, const char* fmt, const char* detail) {
@@ -831,6 +832,7 @@ extern "C" int emia_paste_threshold_bitpack(const float* probs, const float* box
 #include "emia_rle_kernels.cuh"
 #include "emia_text_kernels.cuh"
 #include "emia_coco_kernels.cuh"
+#include "emia_cocoeval_kernels.cuh"
 #include "emia_neighbour_kernels.cuh"
 #include "emia_flow_kernels.cuh"
 #include "emia_scalebar_kernels.cuh"

@@ -1497,6 +1497,187 @@ def coco_decode(strings, H, W):
     return iset
 
 
+# COCOeval.Params for iouType="segm": the values numpy gives, passed to the kernels as they are
+COCO_IOU_THRS = np.linspace(.5, 0.95, int(np.round((0.95 - .5) / .05)) + 1, endpoint=True)
+COCO_REC_THRS = np.linspace(.0, 1.00, int(np.round((1.00 - .0) / .01)) + 1, endpoint=True)
+COCO_AREA_RNG = [[0 ** 2, 1e5 ** 2], [0 ** 2, 32 ** 2], [32 ** 2, 96 ** 2], [96 ** 2, 1e5 ** 2]]
+COCO_AREA_LBL = ["all", "small", "medium", "large"]
+
+
+def _coco_eval_params():
+    thr = [min([t, 1 - 1e-10]) for t in COCO_IOU_THRS]
+    return np.array(thr + list(COCO_REC_THRS) + [r[0] for r in COCO_AREA_RNG] + [r[1] for r in COCO_AREA_RNG] + [np.spacing(1)],
+                    np.float64)
+
+
+def check_max_dets(max_dets, who="evaluate_coco"):
+    """max_dets as an int32 array of three strictly increasing positive ints (COCOeval's maxDets); ValueError otherwise."""
+    md = tuple(max_dets) if isinstance(max_dets, (list, tuple, np.ndarray)) else ()
+    if len(md) != 3 or not all(isinstance(m, (int, np.integer)) and not isinstance(m, (bool, np.bool_)) and 0 < m <= 2 ** 31 - 1
+                               for m in md) or not md[0] < md[1] < md[2]:
+        raise ValueError(f"{who}: max_dets must be three strictly increasing positive ints, not {max_dets!r}")
+    return np.asarray([int(m) for m in md], np.int32)
+
+
+def coco_eval_order(score, category, segment, seg_off, n_categories, n_segments):
+    """(rank, corder, morder) int32 device tensors of n detections listed in (category, image, file order): stable device radix
+    sorts (emia_cocoeval_order) by score descending, then by category (corder: COCOeval.accumulate's order) and by (category,
+    image) segment (morder: evaluateImg's order; rank = the place in the segment).  Work and memory grow linearly with n."""
+    lib = _lib.load()
+    dev = score.device
+    n = int(score.numel())
+    out = [torch.empty(max(n, 1), dtype=torch.int32, device=dev) for _ in range(3)]
+    nb = int(lib.emia_cocoeval_order_workspace_bytes(n))
+    ws = torch.empty(nb, dtype=torch.uint8, device=dev)
+    _lib.check(lib.emia_cocoeval_order(_ptr(score), _ptr(category), _ptr(segment), _ptr(seg_off), n, max(int(n_categories), 1),
+                                       max(int(n_segments), 1), _ptr(out[0]), _ptr(out[1]), _ptr(out[2]), _ptr(ws), nb, _stream()),
+               "emia_cocoeval_order")
+    LAUNCHES["count"] += 2 + 5 * ((64 + 7) // 8 + (max(int(n_categories) - 1, 0).bit_length() + 7) // 8 +
+                                  (max(int(n_segments) - 1, 0).bit_length() + 7) // 8)
+    return tuple(out)
+
+
+def coco_evaluate(gt_sets, dt_sets, n_images, n_categories, max_dets=(1, 10, 100)):
+    """COCO `segm` evaluation (COCOeval.evaluate + accumulate; definition in oracle/cocoeval.py) -> (precision [10, 101, K, 4, 3],
+    recall [10, K, 4, 3]) as float64 device tensors, -1 where COCOeval leaves -1.
+
+    gt_sets[j] / dt_sets[j] hold the instances of one frame size (either may be None): dicts with "iset" (InstanceSet; instance i
+    of an image is its i-th annotation in file order) and per-instance numpy arrays "image" (position 0 .. n_images - 1 in ascending
+    image id), "category" (index 0 .. K - 1 in ascending category id; -1: not evaluated); GT also "area" (float64, the file's
+    area), "iscrowd" (bool) and "id" (int64 annotation id); DT also "score" (float64) and "area" (float64, loadRes' area).
+    One launch per stage and frame size; one host synchronisation per frame size sizes the grid's cell lists, one the pair list."""
+    lib = _lib.load()
+    dev = _need_cuda(None)
+    md = check_max_dets(max_dets, "coco_evaluate")
+    K, I = int(n_categories), int(n_images)
+    if K < 0 or I < 0:
+        raise ValueError(f"coco_evaluate: n_images {n_images!r} and n_categories {n_categories!r} must be >= 0")
+    T, R, A, M = len(COCO_IOU_THRS), len(COCO_REC_THRS), len(COCO_AREA_RNG), len(md)
+    precision = torch.full((T, R, K, A, M), -1.0, dtype=torch.float64, device=dev)
+    recall = torch.full((T, K, A, M), -1.0, dtype=torch.float64, device=dev)
+    groups = [(g, d) for g, d in zip(gt_sets, dt_sets)]
+
+    def side(j, s, fields):
+        if s is None or s["iset"] is None or s["iset"].n == 0:
+            return None
+        n = s["iset"].n
+        cols = {f: np.asarray(s[f]).reshape(-1) for f in fields}
+        assert all(len(c) == n for c in cols.values())
+        cols["grp"] = np.full(n, j, np.int64)
+        cols["loc"] = np.arange(n, dtype=np.int64)
+        return cols
+
+    def table(sides, fields):
+        parts = [p for p in sides if p is not None]
+        if not parts:
+            return {f: np.zeros(0, np.int64) for f in fields + ["image", "category", "grp", "loc"]}, np.zeros(0, np.int64)
+        cols = {f: np.concatenate([p[f] for p in parts]) for f in parts[0]}
+        keep = np.nonzero(cols["category"] >= 0)[0]
+        order = keep[np.lexsort((cols["loc"][keep], cols["image"][keep], cols["category"][keep]))]
+        return {f: v[order] for f, v in cols.items()}, order
+
+    gsides = [side(j, g, ["image", "category", "area", "iscrowd", "id"]) for j, (g, _) in enumerate(groups)]
+    dsides = [side(j, d, ["image", "category", "score", "area"]) for j, (_, d) in enumerate(groups)]
+    G, _ = table(gsides, ["area", "iscrowd", "id"])
+    D, _ = table(dsides, ["score", "area"])
+    ng, nd = len(G["loc"]), len(D["loc"])
+    gkey = G["category"].astype(np.int64) * I + G["image"]
+    dkey = D["category"].astype(np.int64) * I + D["image"]
+    seg_keys = np.unique(np.concatenate([gkey, dkey]))
+    S = len(seg_keys)
+    seg_gt_off = np.searchsorted(gkey, seg_keys).tolist() + [ng]
+    seg_dt_off = np.searchsorted(dkey, seg_keys).tolist() + [nd]
+    n_seg_gt = np.diff(seg_gt_off)
+    wseg_off = np.concatenate([[0], np.cumsum((n_seg_gt + 31) // 32)]).astype(np.int64)
+    n_words = int(wseg_off[-1])
+    cat_gt_off = np.searchsorted(G["category"], np.arange(K + 1)).astype(np.int64)
+    cat_dt_off = np.searchsorted(D["category"], np.arange(K + 1)).astype(np.int64)
+    gt_flags = (G["iscrowd"].astype(bool).astype(np.int32) | ((G["id"] == 0).astype(np.int32) << 1)).astype(np.int32)
+    dt_seg = np.searchsorted(seg_keys, dkey).astype(np.int32)
+    params = _coco_eval_params()
+
+    def dv(a, dtype):
+        return torch.as_tensor(np.ascontiguousarray(a, dtype), device=dev)
+
+    st = _stream()
+    d_score, d_cat, d_seg = dv(D["score"], np.float64), dv(D["category"], np.int32), dv(dt_seg, np.int32)
+    d_area, g_area, g_flags = dv(D["area"], np.float64), dv(G["area"], np.float64), dv(gt_flags, np.int32)
+    t_seg_dt, t_seg_gt, t_wseg = dv(seg_dt_off, np.int64), dv(seg_gt_off, np.int64), dv(wseg_off, np.int64)
+    t_cat_dt, t_cat_gt = dv(cat_dt_off, np.int64), dv(cat_gt_off, np.int64)
+    with _stage("cocoeval_order"):
+        rank, corder, morder = coco_eval_order(d_score, d_cat, d_seg, t_seg_dt, K, S)
+    # pairs, per frame size: grid of the GT boxes keyed by (segment, cell), candidate counts in match order
+    pair_cnt = torch.zeros(nd + 1, dtype=torch.int64, device=dev)
+    work = []
+    for j, (gs, ds) in enumerate(groups):
+        gp, dp = gsides[j], dsides[j]
+        if gp is None or dp is None:
+            continue
+        gi, di = gs["iset"], ds["iset"]
+        sel_g = np.nonzero(G["grp"] == j)[0]
+        sel_d = np.nonzero(D["grp"] == j)[0]
+        gseg_ids = np.unique(np.searchsorted(seg_keys, gkey[sel_g]))
+        if not len(gseg_ids) or not len(sel_d):
+            continue
+        gt_eval = np.full(gi.n, -1, np.int32)
+        gt_eval[G["loc"][sel_g]] = sel_g
+        gt_gseg = np.full(gi.n, -1, np.int32)
+        gt_gseg[G["loc"][sel_g]] = np.searchsorted(gseg_ids, np.searchsorted(seg_keys, gkey[sel_g]))
+        dt_eval = np.full(di.n, -1, np.int32)
+        dt_eval[D["loc"][sel_d]] = sel_d
+        dt_gseg = np.full(di.n, -1, np.int32)
+        s_d = dt_seg[sel_d]
+        pos = np.minimum(np.searchsorted(gseg_ids, s_d), len(gseg_ids) - 1)
+        dt_gseg[D["loc"][sel_d]] = np.where(gseg_ids[pos] == s_d, pos, -1)
+        n_gs = len(gseg_ids)
+        cs = neighbour_cell_size(gi.H, gi.W, max(1, len(sel_g) // n_gs))
+        ncells = n_gs * ((gi.W + cs - 1) // cs) * ((gi.H + cs - 1) // cs)
+        t_geval, t_ggseg, t_deval, t_dgseg = dv(gt_eval, np.int32), dv(gt_gseg, np.int32), dv(dt_eval, np.int32), dv(dt_gseg, np.int32)
+        gb, db = gi.bbox.contiguous(), di.bbox.contiguous()
+        cell_off = torch.empty(ncells + 1, dtype=torch.int64, device=dev)
+        with _stage("cocoeval_pairs"):
+            _lib.check(lib.emia_cocoeval_grid(_ptr(gb), _ptr(t_ggseg), gi.n, n_gs, gi.H, gi.W, cs, _ptr(cell_off), st), "emia_cocoeval_grid")
+            exclusive_scan_(cell_off)
+            n_ent = buffer_len(cell_off[ncells:], ncells)
+            ent = torch.empty(max(n_ent, 1), dtype=torch.int32, device=dev)
+            cursor = torch.empty(ncells, dtype=torch.int32, device=dev)
+            _lib.check(lib.emia_cocoeval_pair_count(_ptr(gb), _ptr(t_ggseg), gi.n, _ptr(db), _ptr(t_deval), _ptr(t_dgseg), di.n, n_gs, gi.H,
+                                                    gi.W, cs, _ptr(cell_off), _ptr(ent), _ptr(cursor), _ptr(rank), _ptr(d_seg),
+                                                    _ptr(t_seg_dt), int(md[-1]), _ptr(pair_cnt), st), "emia_cocoeval_pair_count")
+        LAUNCHES["count"] += 3
+        work.append((gi, di, t_geval, t_deval, t_dgseg, n_gs, cs, cell_off, ent))
+    with _stage("cocoeval_pairs"):
+        exclusive_scan_(pair_cnt)
+    P = buffer_len(pair_cnt[nd:], nd)
+    pair_g = torch.empty(max(P, 1), dtype=torch.int32, device=dev)
+    pair_d = torch.empty(max(P, 1), dtype=torch.int32, device=dev)
+    pair_f = torch.empty(max(P, 1), dtype=torch.int32, device=dev)
+    pair_iou = torch.empty(max(P, 1), dtype=torch.float64, device=dev)
+    pp, mp = params.ctypes.data, md.ctypes.data
+    for gi, di, t_geval, t_deval, t_dgseg, n_gs, cs, cell_off, ent in work:
+        with _stage("cocoeval_pairs"):
+            _lib.check(lib.emia_cocoeval_pair_fill(_ptr(gi.crops), _ptr(gi.meta), _ptr(gi.crop_off), _ptr(gi.bbox.contiguous()),
+                                                   _ptr(gi.area.contiguous()), _ptr(t_geval), _ptr(di.crops), _ptr(di.meta),
+                                                   _ptr(di.crop_off), _ptr(di.bbox.contiguous()), _ptr(di.area.contiguous()), _ptr(t_deval),
+                                                   _ptr(t_dgseg), di.n, n_gs, gi.H, gi.W, cs, _ptr(cell_off), _ptr(ent), _ptr(rank),
+                                                   _ptr(d_seg), _ptr(t_seg_dt), _ptr(g_area), _ptr(g_flags), pp, mp, _ptr(pair_cnt),
+                                                   _ptr(pair_g), _ptr(pair_d), _ptr(pair_f), _ptr(pair_iou), st), "emia_cocoeval_pair_fill")
+        LAUNCHES["count"] += 1
+    # matching per (segment, area range), then the curves per (category, area range, maxDet, threshold)
+    matched = torch.empty(max(n_words * A * T, 1), dtype=torch.int32, device=dev)
+    state = torch.empty(max(A * nd, 1), dtype=torch.int32, device=dev)
+    with _stage("cocoeval_match"):
+        _lib.check(lib.emia_cocoeval_match(_ptr(t_seg_dt), _ptr(t_seg_gt), _ptr(t_wseg), S, n_words, _ptr(morder),
+                                           _ptr(d_area), _ptr(pair_cnt), _ptr(pair_g), _ptr(pair_d), _ptr(pair_f), _ptr(pair_iou), nd,
+                                           pp, mp, _ptr(matched), _ptr(state), st), "emia_cocoeval_match")
+    with _stage("cocoeval_accumulate"):
+        _lib.check(lib.emia_cocoeval_accumulate(_ptr(corder), _ptr(rank), _ptr(state), _ptr(t_cat_dt), _ptr(t_cat_gt), _ptr(g_area),
+                                                _ptr(g_flags), nd, K, pp, mp, _ptr(precision), _ptr(recall), st),
+                   "emia_cocoeval_accumulate")
+    LAUNCHES["count"] += 2
+    return precision, recall
+
+
 def measurements_csv_text(iset, file_name, psum, class_idx, class_fields, contrast=None, shape=None):
     """The rows of measurements_results.csv for the measured records of `iset` (after measure()), in record order: byte for byte
     what csv.writer writes for the rows of inference.measure_masks, UTF-8, "\\r\\n" line ends.  Instance i gets Instance_ID

@@ -954,16 +954,18 @@ def _coco_error(path, ann, why):
     return ValueError(f"{path}: annotation {ann.get('id')!r}: {why}")
 
 
-def _load_coco(path, images):
-    """(file dict, {file name: InstanceSet with classes / scores}) of a COCO instance file for the (file name, image) pairs."""
-    images = list(images)
+def _decode_coco(path, names, sizes, d=None):
+    """(file dict, per-image [(counts bytes, category, score or None, annotation)] in file order, [((H, W), image positions,
+    InstanceSet of their annotations in that order)] with one decode per distinct frame size) of a COCO instance file, for the
+    images `names` of frame sizes `sizes`.  d: the file, already parsed."""
     by_name = {}
-    for k, (name, _) in enumerate(images):
+    for k, name in enumerate(names):
         if name in by_name:
             raise ValueError(f"load_coco_results: the file name {name!r} is given twice")
         by_name[name] = k
-    with open(path, "rb") as f:
-        d = json.loads(f.read())
+    if d is None:
+        with open(path, "rb") as f:
+            d = json.loads(f.read())
     img_of, matched = {}, set()
     for e in d.get("images", []):
         name = e.get("file_name")
@@ -976,7 +978,7 @@ def _load_coco(path, images):
             raise ValueError(f"{path}: image id {e.get('id')!r} appears twice")
         img_of[e.get("id")] = k
         matched.add(k)
-    per = [[] for _ in images]                     # (counts bytes, category, score or None, annotation) per image, file order
+    per = [[] for _ in names]                      # (counts bytes, category, score or None, annotation) per image, file order
     for ann in d.get("annotations", []):
         seg = ann.get("segmentation")
         if not isinstance(seg, dict) or not isinstance(seg.get("counts"), str):
@@ -984,7 +986,7 @@ def _load_coco(path, images):
         if ann.get("image_id") not in img_of:
             raise _coco_error(path, ann, f"image_id {ann.get('image_id')!r} has no images entry")
         k = img_of[ann["image_id"]]
-        H, W = (int(v) for v in images[k][1].shape[:2])
+        H, W = sizes[k]
         if list(seg.get("size", [])) != [H, W]:
             raise _coco_error(path, ann, f"size {seg.get('size')!r} is not the image's [{H}, {W}]")
         cat = ann.get("category_id")
@@ -992,15 +994,28 @@ def _load_coco(path, images):
             raise _coco_error(path, ann, f"category_id {cat!r} is not a non-negative integer")
         per[k].append((seg["counts"].encode("utf-8"), cat, ann.get("score"), ann))
     by_size = {}
-    for k, (_, image) in enumerate(images):
-        by_size.setdefault(tuple(int(s) for s in image.shape[:2]), []).append(k)
-    out, bad = {}, []
+    for k, hw in enumerate(sizes):
+        by_size.setdefault(tuple(hw), []).append(k)
+    groups, bad = [], []
     for (H, W), ks in by_size.items():
         items = [it for k in ks for it in per[k]]
         raw = [it[0] for it in items]
         off = np.concatenate([[0], np.cumsum([len(b) for b in raw])]).astype(np.int64)
         iset, status = engine._coco_decode(b"".join(raw), off, H, W)
         bad += [(items[j][3], int(status[j])) for j in np.nonzero(status)[0][:1]]
+        groups.append(((H, W), ks, iset))
+    if bad:
+        ann, code = min(bad, key=lambda b: d["annotations"].index(b[0]))
+        raise engine._lib.EmiaError(f"{path}: annotation {ann.get('id')!r}: {engine.COCO_STATUS[code]}")
+    return d, per, groups
+
+
+def _load_coco(path, images):
+    """(file dict, {file name: InstanceSet with classes / scores}) of a COCO instance file for the (file name, image) pairs."""
+    images = list(images)
+    d, per, groups = _decode_coco(path, [name for name, _ in images], [tuple(int(v) for v in im.shape[:2]) for _, im in images])
+    out = {}
+    for _, ks, iset in groups:
         a = 0
         for k in ks:
             m = len(per[k])
@@ -1012,9 +1027,6 @@ def _load_coco(path, images):
                 isinstance(v, (int, float)) and not isinstance(v, bool) for v in scores) else None
             out[images[k][0]] = s
             a += m
-    if bad:
-        ann, code = min(bad, key=lambda b: d["annotations"].index(b[0]))
-        raise engine._lib.EmiaError(f"{path}: annotation {ann.get('id')!r}: {engine.COCO_STATUS[code]}")
     return d, out
 
 
@@ -1053,3 +1065,118 @@ def measure_coco(path, output_dir, *, images=None, dataset_name=None, scale_bar_
         fields, class_idx = _class_table(iset.classes.cpu().numpy().tolist(), names)
         _saved_texts(texts, nb_text, iset, name, image, psum, um_pix, class_idx, fields, shape_columns, neighbours)
     _write_results(output_dir, texts, nb_text, shape_columns, neighbours)
+
+
+# =================================================================================================================
+# COCO segm evaluation of a detections file against a ground-truth file (definition: oracle/cocoeval.py)
+# =================================================================================================================
+COCO_EVAL_HEADER = ["Metric", "Category", "IoU", "Area", "MaxDets", "Value"]
+# (AP or AR, IoU threshold or None for .50:.95, area range, index into max_dets) of COCOeval.summarize's 12 segm stats
+COCO_STAT_ROWS = [(1, None, "all", 2), (1, .5, "all", 2), (1, .75, "all", 2), (1, None, "small", 2), (1, None, "medium", 2),
+                  (1, None, "large", 2), (0, None, "all", 0), (0, None, "all", 1), (0, None, "all", 2), (0, None, "small", 2),
+                  (0, None, "medium", 2), (0, None, "large", 2)]
+
+
+def _coco_mean(s):
+    return float(np.mean(s[s > -1])) if len(s[s > -1]) else -1.0
+
+
+def _coco_summarize(precision, recall, max_dets):
+    """COCOeval.summarize on the host arrays: the 12 stats and the per-category AP (IoU .50:.95, area all, maxDets[2])."""
+    stats = []
+    for ap, thr, area, m in COCO_STAT_ROWS:
+        aind = [i for i, lbl in enumerate(engine.COCO_AREA_LBL) if lbl == area]
+        s = precision if ap else recall
+        if thr is not None:
+            s = s[np.where(thr == engine.COCO_IOU_THRS)[0]]
+        s = s[:, :, :, aind, [m]] if ap else s[:, :, aind, [m]]
+        stats.append(_coco_mean(s))
+    return stats, [_coco_mean(precision[:, :, k, 0, 2]) for k in range(precision.shape[2])]
+
+
+def _coco_number(v):
+    return isinstance(v, (int, float)) and not isinstance(v, bool) and not (isinstance(v, float) and v != v)
+
+
+def evaluate_coco(gt_path, dt_path, output_dir=None, *, max_dets=(1, 10, 100), match_categories="id"):
+    """COCO `segm` evaluation of the detections file dt_path (coco_instances.json of run_inference, or any COCO instance JSON with
+    compressed-RLE masks and scores) against the ground truth gt_path: pycocotools' COCOeval (iouType "segm") with maxDets
+    max_dets, on the device.  Returns {"stats": the 12 numbers of COCOeval.summarize, "per_category": {name: AP}, "precision"
+    [10, 101, K, 4, 3], "recall" [10, K, 4, 3]} (numpy float64, -1 where COCOeval leaves -1); with output_dir also writes
+    coco_eval_results.csv.  The default max_dets are pycocotools' and keep only the 100 best detections of an image: a dense
+    micrograph needs larger values, e.g. (100, 1000, 30000).  The frame sizes come from the GT file's images; no pixel data is read.
+
+    Images are matched by file_name; categories are the GT file's, and match_categories="name" maps a DT category_id to the GT
+    category of the same name (run_inference writes 0-based thing_classes ids, annotation tools usually start at 1).  Raises
+    ValueError, naming the file and the annotation or image, for max_dets that are not three strictly increasing positive ints, a
+    detection without a numeric score, a DT image whose file_name has no GT image, a GT category name given twice under "name",
+    and the load_coco_results errors."""
+    md = tuple(int(m) for m in engine.check_max_dets(max_dets))
+    if match_categories not in ("id", "name"):
+        raise ValueError(f"evaluate_coco: match_categories must be 'id' or 'name', not {match_categories!r}")
+    with open(gt_path, "rb") as f:
+        gt = json.loads(f.read())
+    with open(dt_path, "rb") as f:
+        dt = json.loads(f.read())
+    gimgs = sorted(gt.get("images", []), key=lambda e: e.get("id"))
+    names = [e.get("file_name") for e in gimgs]
+    seen = set()
+    for e in gimgs:
+        if e.get("file_name") in seen:
+            raise ValueError(f"{gt_path}: image {e.get('id')!r}: file_name {e.get('file_name')!r} appears twice")
+        seen.add(e.get("file_name"))
+    sizes = [(int(e["height"]), int(e["width"])) for e in gimgs]
+    cat_ids = sorted(c["id"] for c in gt.get("categories", []))
+    kidx = {c: k for k, c in enumerate(cat_ids)}
+    if match_categories == "name":
+        by_name = {}
+        for c in gt.get("categories", []):
+            if c.get("name") in by_name:
+                raise ValueError(f"{gt_path}: category {c.get('id')!r}: name {c.get('name')!r} is given twice")
+            by_name[c.get("name")] = c["id"]
+        dmap = {c.get("id"): kidx[by_name[c.get("name")]] for c in dt.get("categories", []) if c.get("name") in by_name}
+    else:
+        dmap = kidx
+    dt_anns = dt.get("annotations", [])
+    for ann in dt_anns:
+        if not _coco_number(ann.get("score")):
+            raise _coco_error(dt_path, ann, f"score {ann.get('score')!r} is not a number")
+    for e in dt.get("images", []):
+        if e.get("file_name") not in seen:
+            raise ValueError(f"{dt_path}: image {e.get('id')!r}: file_name {e.get('file_name')!r} has no GT image")
+    bbox_area = bool(dt_anns) and bool(dt_anns[0].get("bbox"))      # loadRes' bbox branch: area = w * h of each bbox
+    _, gper, ggroups = _decode_coco(gt_path, names, sizes, d=gt)
+    _, dper, dgroups = _decode_coco(dt_path, names, sizes, d=dt)
+    gt_sets, dt_sets = [], []
+    for (_, ks, gi), (_, _, di) in zip(ggroups, dgroups):
+        g_items = [(k, it) for k in ks for it in gper[k]]
+        d_items = [(k, it) for k in ks for it in dper[k]]
+        g_pop = gi.area.cpu().numpy() if g_items else np.zeros(0)
+        d_pop = di.area.cpu().numpy() if d_items else np.zeros(0)
+        gt_sets.append({"iset": gi, "image": np.array([k for k, _ in g_items], np.int64),
+                        "category": np.array([kidx.get(it[1], -1) for _, it in g_items], np.int64),
+                        "area": np.array([float(it[3]["area"]) if "area" in it[3] else float(g_pop[j])
+                                          for j, (_, it) in enumerate(g_items)], np.float64),
+                        "iscrowd": np.array([bool(it[3].get("iscrowd", 0)) for _, it in g_items], bool),
+                        "id": np.array([int(it[3].get("id", -1)) for _, it in g_items], np.int64)})
+        dt_sets.append({"iset": di, "image": np.array([k for k, _ in d_items], np.int64),
+                        "category": np.array([dmap.get(it[1], -1) for _, it in d_items], np.int64),
+                        "score": np.array([float(it[2]) for _, it in d_items], np.float64),
+                        "area": np.array([float(it[3]["bbox"][2] * it[3]["bbox"][3]) if bbox_area else float(d_pop[j])
+                                          for j, (_, it) in enumerate(d_items)], np.float64)})
+    precision, recall = engine.coco_evaluate(gt_sets, dt_sets, len(names), len(cat_ids), md)
+    precision, recall = precision.cpu().numpy(), recall.cpu().numpy()
+    stats, per_cat = _coco_summarize(precision, recall, md)
+    cnames = {c["id"]: c.get("name") for c in gt.get("categories", [])}
+    cat_names = [cnames[c] for c in cat_ids]
+    if output_dir is not None:
+        os.makedirs(output_dir, exist_ok=True)
+        with open(os.path.join(output_dir, "coco_eval_results.csv"), "w", newline="", encoding="utf-8") as f:
+            w = csv.writer(f)
+            w.writerow(COCO_EVAL_HEADER)
+            iou = lambda t: "0.50:0.95" if t is None else f"{t:.2f}"      # noqa: E731
+            for (ap, t, area, m), v in zip(COCO_STAT_ROWS, stats):
+                w.writerow(["AP" if ap else "AR", "all", iou(t), area, md[m], repr(float(v))])
+            for name, v in zip(cat_names, per_cat):
+                w.writerow(["AP", name, iou(None), "all", md[2], repr(float(v))])
+    return {"stats": stats, "per_category": dict(zip(cat_names, per_cat)), "precision": precision, "recall": recall}

@@ -247,3 +247,4 @@ def scalebar_strips(seed, B, rh=92, W=1024, x0=512):
                      int(rng.integers(120, 256)), int(rng.integers(1, 3)))
         out[b] = g[:, :, None]
     return out
+

@@ -413,6 +413,50 @@ int emia_coco_counts_count(const uint8_t* data, const int64_t* str_off, int64_t 
                            void* stream);
 int emia_coco_counts_fill(const uint8_t* data, const int64_t* str_off, int64_t n, int H, int W, const int64_t* run_off,
                           int64_t* runs, void* stream);
+/* ---- COCO segm evaluation (csrc/emia_cocoeval_kernels.cuh, core/emia_cocoeval.cuh; definition in oracle/cocoeval.py) -----------
+ * The evaluated detections (DT list, n_dt) and GTs (GT list) are sorted by (category, image, file order); cat_*_off[K + 1] and
+ * seg_*_off[S + 1] bound the categories and the (category, image) segments in each list; dt_seg / img / cat are per DT list entry.
+ * params_host: EMIA_CE_PARAMS doubles, min(iouThrs[t], 1 - 1e-10) x 10, recThrs x 101, the area ranges' lower bounds x 4 and upper
+ * bounds x 4, np.spacing(1); max_dets_host: the three maxDets.  gt_flags: bit 0 iscrowd, bit 1 the GT's id is 0.
+ * emia_cocoeval_order: stable radix sorts (O(n) per 8-bit pass) of the DT list: corder[cat_off[k] + p] = the DT at place p of
+ *   category k by (score desc, image, file order); morder[seg_off[s] + r] = the DT of rank r of segment s by (score desc, file
+ *   order) ("match position"); rank[i] = that place r of DT i.  workspace: emia_cocoeval_order_workspace_bytes(n_dt) bytes.
+ * emia_cocoeval_grid (per frame size): cell_cnt[(gseg * gy + y) * gx + x] = GT boxes (gt_gseg[i] >= 0: a grid segment) covering the
+ *   cell (cell_cnt has n_seg * gx * gy + 1 entries; caller scans it into cell_off).
+ * emia_cocoeval_pair_count: fills the cell lists (ent, cursor: n_seg * gx * gy ints of scratch) and writes, for every local DT j with
+ *   dt_eval[j] >= 0 and rank < max_det, pair_cnt[match position] = GTs of its grid segment whose box meets its box (caller zeroes
+ *   pair_cnt[n_dt + 1] before the first frame size and scans it into pair_off after the last).
+ * emia_cocoeval_pair_fill: those pairs at pair_off[match position]: GT list index, DT list index, flags (gt_flags | _ignore of area
+ *   range a at bit 4 + a) and the IoU of maskApi.c rleIou.
+ * emia_cocoeval_match: per segment and area range the greedy matching of evaluateImg at the 10 thresholds; state[a * n_dt + i] = tp
+ *   bits 0..9 and fp bits 10..19 of DT i (matched: n_words * 40 words of scratch, wseg_off[s] = the segment's first bitmap word).
+ * emia_cocoeval_accumulate: precision [10, 101, n_cat, 4, 3] and recall [10, n_cat, 4, 3] (float64, caller fills them with -1) as
+ *   COCOeval.accumulate. */
+size_t emia_cocoeval_order_workspace_bytes(int64_t n_dt);
+int emia_cocoeval_order(const double* score, const int32_t* cat, const int32_t* dt_seg, const int64_t* seg_off, int64_t n_dt,
+                        int32_t n_cat, int64_t n_seg, int32_t* rank, int32_t* corder, int32_t* morder, void* workspace,
+                        size_t workspace_bytes, void* stream);
+int emia_cocoeval_grid(const int32_t* gt_bbox, const int32_t* gt_gseg, int64_t n_gt, int32_t n_seg, int32_t H, int32_t W,
+                       int32_t cell_size, int64_t* cell_cnt, void* stream);
+int emia_cocoeval_pair_count(const int32_t* gt_bbox, const int32_t* gt_gseg, int64_t n_gt, const int32_t* dt_bbox, const int32_t* dt_eval,
+                             const int32_t* dt_gseg, int64_t n_dt, int32_t n_seg, int32_t H, int32_t W, int32_t cell_size,
+                             const int64_t* cell_off, int32_t* ent, int32_t* cursor, const int32_t* rank, const int32_t* dt_seg,
+                             const int64_t* seg_dt_off, int32_t max_det, int64_t* pair_cnt, void* stream);
+int emia_cocoeval_pair_fill(const uint32_t* gt_crops, const emia_inst_meta* gt_meta, const int64_t* gt_crop_off, const int32_t* gt_bbox,
+                            const int32_t* gt_area, const int32_t* gt_eval, const uint32_t* dt_crops, const emia_inst_meta* dt_meta,
+                            const int64_t* dt_crop_off, const int32_t* dt_bbox, const int32_t* dt_area, const int32_t* dt_eval,
+                            const int32_t* dt_gseg, int64_t n_dt, int32_t n_seg, int32_t H, int32_t W, int32_t cell_size,
+                            const int64_t* cell_off, const int32_t* ent, const int32_t* rank, const int32_t* dt_seg,
+                            const int64_t* seg_dt_off, const double* gt_area_eval, const int32_t* gt_flags, const double* params_host,
+                            const int32_t* max_dets_host, const int64_t* pair_off, int32_t* pair_g, int32_t* pair_d, int32_t* pair_f,
+                            double* pair_iou, void* stream);
+int emia_cocoeval_match(const int64_t* seg_dt_off, const int64_t* seg_gt_off, const int64_t* wseg_off, int64_t n_seg, int64_t n_words,
+                        const int32_t* morder, const double* dt_area, const int64_t* pair_off, const int32_t* pair_g, const int32_t* pair_d,
+                        const int32_t* pair_f, const double* pair_iou, int64_t n_dt, const double* params_host,
+                        const int32_t* max_dets_host, uint32_t* matched, uint32_t* state, void* stream);
+int emia_cocoeval_accumulate(const int32_t* corder, const int32_t* rank, const uint32_t* state, const int64_t* cat_dt_off,
+                             const int64_t* cat_gt_off, const double* gt_area, const int32_t* gt_flags, int64_t n_dt, int32_t n_cat,
+                             const double* params_host, const int32_t* max_dets_host, double* precision, double* recall, void* stream);
 /* raw moments (m00, m10, m01) of every instance as exact integers: cv2.moments(mask) of src/functions/inference.py:1101-1104 */
 int emia_moments01(const uint32_t* crops, const emia_inst_meta* meta, const int64_t* crop_off, int64_t n, int64_t* out,
                    void* stream);
